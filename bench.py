@@ -11,6 +11,8 @@ One "step" = one pass of the hot path over one batch of B frame pairs per GPU, a
           D2H of the results inside the timed region.
 The reference arm (--impl reference) times the CPU restatement of the reference (oracle/, kind "port": the reference itself
 needs OpenCV/Eigen/Sophus/Ceres and cannot be built here) on all host threads.
+--dump-outputs DIR writes what the timed path returned in its last step for rank 0's batch (poses, tracked counts, refined patch positions and
+flags, float32 / float64 .npy) for comparing two builds on the same seeded inputs.
 No pair shards across GPUs: N > 1 = N independent replicas of the batch (weak scaling), no collective on the data path.
 Extra keys on the same line: `refine_chain` = the step with the reference's own refinement chain (reprojection -> closest observation ->
 affine -> warp -> Align2D on the device) instead of host patches; `strong_scaling` = BASELINE configs[4] as written: ONE batch of 4096
@@ -217,6 +219,25 @@ def measured_traffic(kernel, pairs):
     return None if not t else float(t["bytes_per_pair"]) * pairs
 
 
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(d, poses, n_tracked, px, conv):
+    """--dump-outputs: what the timed path returned for its last step, one float array per output as DIR/<name>.npy, so that two
+    builds can be compared output for output on the same seeded inputs. Above DUMP_LIMIT bytes a fixed seeded sample of the pairs is
+    written; pair_index.npy names the pairs either way."""
+    n = len(poses)
+    per_pair = 8 * (1 + 7 + 1 + px[0].size) + 4 * conv[0].size
+    idx = np.arange(n)
+    if n * per_pair > DUMP_LIMIT - 4096:                       # 4 KB for the .npy headers
+        idx = np.sort(np.random.default_rng(0).choice(n, (DUMP_LIMIT - 4096) // per_pair, replace=False))
+    os.makedirs(d, exist_ok=True)
+    out = {"pair_index": idx.astype(np.float64), "poses": poses[idx], "n_tracked": n_tracked[idx].astype(np.float64),
+           "patch_px": px[idx], "patch_converged": conv[idx].astype(np.float32)}
+    for name, a in out.items():
+        np.save(os.path.join(d, name + ".npy"), np.ascontiguousarray(a))
+
+
 def dist_setup(n_gpus):
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -289,6 +310,8 @@ def run_ours(args):
     tw1 = time.perf_counter()
     launches = ctx.launch_count() - l0
     barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *ctx.batch_fetch())
     t = torch.tensor([dev_ms], dtype=torch.float64, device="cuda")
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -875,8 +898,10 @@ def run_reference(args):
         O.pair_batch(*a)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        O.pair_batch(*a)
+        res = O.pair_batch(*a)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, *res)
     value = sample * args.steps / dt
     line = {"impl": "reference", "metric": METRIC.replace("640x480", "%dx%d" % (cam["width"], cam["height"])), "value": value, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps, "warmup": max(args.warmup, 1),
             "ms_per_step": dt * 1e3 / args.steps, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f64",
@@ -903,7 +928,10 @@ def main():
     ap.add_argument("--no-strong", action="store_true", help="skip the strong-scaling extra")
     ap.add_argument("--cam", default="kinect", choices=["kinect", "euroc"],
                     help="kinect = 640x480 (the metric's configuration, default); euroc = 752x480, BASELINE configs[4]'s sweep geometry")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the timed path's outputs of its last step (rank 0) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -16,16 +16,16 @@ _REF = os.path.join(_HERE, "_ref", "libfast_ref.so")
 
 
 def build(force=False):
-    """Compile the oracle (and oracle/_ref when /root/reference is mounted). Building is not using."""
+    """Compile the oracle (and oracle/_ref where refpin.REFERENCE holds a checkout of the reference). Building is not using."""
     src = os.path.join(_HERE, "dsdtm_oracle.cpp")
     stale = (not os.path.exists(_LIB)) or os.path.getmtime(_LIB) < max(
         os.path.getmtime(src), os.path.getmtime(os.path.join(_HERE, "dsdtm_oracle.h")))
     if force or stale:
         subprocess.check_call(["make", "-C", _HERE, "_build/liboracle.so"], stdout=subprocess.DEVNULL)
-    if os.path.isdir("/root/reference/Thirdparty/fast/src") and (force or not os.path.exists(_REF)):
-        subprocess.check_call(["make", "-C", _HERE, "ref"], stdout=subprocess.DEVNULL)
-    # the reference's own hot-path translation units against the stand-in headers of tests/ref_shim (oracle/refpin.py)
     from . import refpin
+    if refpin.REFERENCE and os.path.isdir(os.path.join(refpin.REFERENCE, "Thirdparty", "fast", "src")) and (force or not os.path.exists(_REF)):
+        subprocess.check_call(["make", "-C", _HERE, "ref", "REF=" + refpin.REFERENCE], stdout=subprocess.DEVNULL)
+    # the reference's own hot-path translation units against the stand-in headers of tests/ref_shim (oracle/refpin.py)
     refpin.build(force)
 
 

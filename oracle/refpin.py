@@ -1,5 +1,5 @@
 """TEST INFRASTRUCTURE -- ctypes loader for oracle/_ref/libdsdtm_ref.so: the reference's OWN hot-path translation units
-(/root/reference/src/{Sprase_ImageAlign,Feature_alignment,Feature_detection,Camera,Frame,MapPoint,Keyframe,Map,Config}.cpp and
+(<reference>/src/{Sprase_ImageAlign,Feature_alignment,Feature_detection,Camera,Frame,MapPoint,Keyframe,Map,Config}.cpp and
 Thirdparty/fast), compiled unmodified against the stand-in third-party headers of tests/ref_shim by `make -C oracle ref_dsdtm`,
 driven through oracle/ref_dsdtm_wrap.cpp.
 
@@ -7,6 +7,7 @@ Only tests/ (and the golden generator tests/golden/make_golden_refpin.py) import
 oracle/dsdtm_oracle.cpp to the reference's source for the floating-point rows of SURVEY.md 8(a).
 """
 import ctypes as C
+import json
 import os
 import subprocess
 import tempfile
@@ -15,7 +16,21 @@ import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 _LIBS = {False: os.path.join(_HERE, "_ref", "libdsdtm_ref.so"), True: os.path.join(_HERE, "_ref", "libdsdtm_ref_tree.so")}
-_REFROOT = "/root/reference"
+
+
+def _reference_root():
+    """A checkout of the original DSDTM sources (github.com/gaochq/DSDTM): DSDTM_REFERENCE, else the location BASELINE.json
+    records as reference_path. Without a checkout there the pin tests skip."""
+    if os.environ.get("DSDTM_REFERENCE"):
+        return os.environ["DSDTM_REFERENCE"]
+    try:
+        with open(os.path.join(os.path.dirname(_HERE), "BASELINE.json")) as f:
+            return json.load(f).get("reference_path") or ""
+    except (OSError, ValueError):
+        return ""
+
+
+REFERENCE = _reference_root()
 
 
 def available(tree=False):
@@ -23,9 +38,9 @@ def available(tree=False):
 
 
 def build(force=False):
-    """Only possible where the reference tree is mounted (the build container)."""
-    if os.path.isdir(os.path.join(_REFROOT, "src")) and (force or not (available(False) and available(True))):
-        subprocess.check_call(["make", "-C", _HERE, "ref_dsdtm"], stdout=subprocess.DEVNULL)
+    """Only possible where REFERENCE holds a checkout of the reference."""
+    if REFERENCE and os.path.isdir(os.path.join(REFERENCE, "src")) and (force or not (available(False) and available(True))):
+        subprocess.check_call(["make", "-C", _HERE, "ref_dsdtm", "REF=" + REFERENCE], stdout=subprocess.DEVNULL)
 
 
 def _p(a):
@@ -60,7 +75,7 @@ class Ref:
 
     def __init__(self, cam, tree=False, **params):
         if not available(tree):
-            raise RuntimeError("oracle/_ref/libdsdtm_ref.so is not built (needs /root/reference: make -C oracle ref_dsdtm)")
+            raise RuntimeError("oracle/_ref/libdsdtm_ref.so is not built (needs the reference sources at %s: make -C oracle ref_dsdtm)" % (REFERENCE or "DSDTM_REFERENCE"))
         # the library keeps its objects (Config singleton, camera, frames, map) in globals: every Ref gets a private copy of the
         # shared object so that two parameter sets can be alive at once
         import shutil

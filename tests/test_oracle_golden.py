@@ -1,5 +1,5 @@
 """CPU suite: the oracle against the golden vectors (cv2 4.13, the reference's FAST library, the 167-corner KAT) and,
-when it was built in this container, against oracle/_ref (the reference's own FAST sources)."""
+where a checkout of the reference is present, against oracle/_ref (the reference's own FAST sources)."""
 import numpy as np
 import pytest
 
@@ -44,7 +44,7 @@ def test_fast_detect_score_nonmax_equal_reference_lists(golden, barrier):
         assert len(xy) == 3787 and len(keep) == 843      # SURVEY App. C probe 2
 
 
-@pytest.mark.skipif(not O.have_ref(), reason="oracle/_ref (reference FAST sources) not built here")
+@pytest.mark.skipif(not O.have_ref(), reason="oracle/_ref/libfast_ref.so needs the reference sources at BASELINE.json's reference_path (or DSDTM_REFERENCE)")
 def test_fast_closed_form_equals_reference_library_on_adversarial_images():
     rng = np.random.default_rng(5)
     for t in range(24):

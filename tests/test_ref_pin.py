@@ -1,6 +1,6 @@
 """Pins oracle/dsdtm_oracle.cpp to the reference's OWN source for the floating-point rows of SURVEY.md 8(a) (a5-a16, f-1, f-3).
 
-oracle/_ref/libdsdtm_ref.so = /root/reference/src/{Sprase_ImageAlign,Feature_alignment,Feature_detection,Camera,Frame,MapPoint,
+oracle/_ref/libdsdtm_ref.so = <reference>/src/{Sprase_ImageAlign,Feature_alignment,Feature_detection,Camera,Frame,MapPoint,
 Keyframe,Map,Config}.cpp + Thirdparty/fast, compiled UNMODIFIED (recipe: oracle/Makefile, target ref_dsdtm) against the stand-in
 third-party headers of tests/ref_shim. Every test below feeds the reference's classes and the oracle the same inputs.
 
@@ -10,8 +10,8 @@ What "equal" means here:
 * what happens inside Eigen / Sophus calls (LDLT, SE3::exp, quaternion products, norms) is the stand-in's restatement; the default
   build associates reductions left to right like the oracle, and the `_tree` build (Eigen's fixed-size unroller order) is checked to
   move results only in the last bits -- i.e. the comparison does not hinge on that unpinnable choice.
-These tests need the library built from /root/reference (this container); the values they establish travel to the GPU box as
-tests/golden/refpin.npz (see test_ref_golden.py)."""
+These tests need the library built from a checkout of the reference (at BASELINE.json's reference_path, or DSDTM_REFERENCE) and skip without it; part of the
+values they establish travel as tests/golden/refpin.npz (see test_ref_golden.py)."""
 import numpy as np
 import pytest
 
@@ -22,7 +22,7 @@ from oracle import refpin as RP
 from oracle_seq import CELL, LEVELS, OMap, OracleFrame, _oracle_search_multi, _oracle_sparse_align, _trajectory
 
 RP.build()
-pytestmark = pytest.mark.skipif(not RP.available(), reason="oracle/_ref/libdsdtm_ref.so needs /root/reference (make -C oracle ref_dsdtm)")
+pytestmark = pytest.mark.skipif(not RP.available(), reason="oracle/_ref/libdsdtm_ref.so needs the reference sources at %s (or DSDTM_REFERENCE)" % RP.REFERENCE)
 
 CFGS = [(4, 0, 30), (5, 0, 8), (5, 2, 8), (3, 1, 4)]        # BASELINE configs[0] ctor, production ctor, truncated variants
 
