@@ -35,6 +35,12 @@ BA_SUMMARY_DT = np.dtype([("iterations", "<i4"), ("termination", "<i4"), ("n_suc
 assert BA_OBS_DT.itemsize == 56 and BA_SUMMARY_DT.itemsize == 32
 BA_FUNCTION_TOL, BA_PARAMETER_TOL, BA_GRADIENT_TOL, BA_NO_CONVERGENCE, BA_FAILURE, BA_MIN_RADIUS, BA_NO_RESIDUALS = range(7)
 BA_MAX_OBS = 4096
+MATCH_DT = np.dtype([("point", "<i4"), ("px", "<f4", 2), ("level", "<i4")])
+assert MATCH_DT.itemsize == 16
+TRACK_MAX_MATCHES = 200
+# dsdtm_batch_run flags: 1 = rebuild the cur pyramids, 2 = the refinement chain (batch_stage_map), 4 (with 2) = SearchLocalPoints'
+# selection + PoseOptimization behind it (batch_stage_track): flags 7 ends in the tracked pose of every pair
+RUN_PYRAMID, RUN_CHAIN, RUN_TRACK = 1, 2, 4
 
 
 class Cam(C.Structure):
@@ -78,6 +84,7 @@ SYMBOLS = [
     "dsdtm_local_map_align_batch", "dsdtm_depth_upload", "dsdtm_depth_convert_f32", "dsdtm_keyframe_lift",
     "dsdtm_frame_upload_pyramid_host", "dsdtm_frames_upload_clahe_pyramid", "dsdtm_track_frame",
     "dsdtm_pose_optimize", "dsdtm_pose_optimize_batch", "dsdtm_map_table_upload", "dsdtm_close_keyframes", "dsdtm_probe_fp64", "dsdtm_frame_upload_pyramid_async", "dsdtm_track_frame_store", "dsdtm_store_set_points", "dsdtm_store_update_points", "dsdtm_store_append_keyframe", "dsdtm_store_set_keyframe", "dsdtm_store_clear", "dsdtm_store_track", "dsdtm_frame_upload_level", "dsdtm_batch_stage_map", "dsdtm_batch_fetch_map", "dsdtm_track_batch_e2e",
+    "dsdtm_batch_stage_track", "dsdtm_batch_fetch_track",
 ]
 
 
@@ -426,6 +433,21 @@ class Context:
         out = np.zeros((self._n, self._map_ppp), REPROJ_DT)
         self._ck(self.L.dsdtm_batch_fetch_map(self.hp, _p(out)))
         return out
+
+    def batch_stage_track(self, found=None, max_iters=100):
+        """after batch_stage_map: found = (n_pairs, points_per_pair) MapPoint::mnFound counts (None = all 1), max_iters = PoseOptimization's
+        cap; batch_run(7) then ends in the tracked poses"""
+        f = None if found is None else np.ascontiguousarray(found, np.int32).reshape(self._n, self._map_ppp)
+        self._ck(self.L.dsdtm_batch_stage_track(self.hp, _p(f), int(max_iters)))
+
+    def batch_fetch_track(self):
+        """-> (poses c2w after PoseOptimization (n, 7), n_matches (n,), matches (n, 200) MATCH_DT, res_norm (n, 200), summaries (n,)
+        BA_SUMMARY_DT); rows past n_matches[i] are zero"""
+        n, K = self._n, TRACK_MAX_MATCHES
+        poses = np.empty((n, 7)); nm = np.empty(n, np.int32); m = np.empty((n, K), MATCH_DT); res = np.empty((n, K))
+        summ = np.empty(n, BA_SUMMARY_DT)
+        self._ck(self.L.dsdtm_batch_fetch_track(self.hp, _p(poses), _p(nm), _p(m), _p(res), _p(summ)))
+        return poses, nm, m, res, summ
 
     def track_batch_e2e(self, cur_imgs, ref_slots, cur_slots, feats, feat_stride, n_feats, ref_centers, poses_ref, poses_in, max_level, min_level,
                         max_iters, points_per_pair, max_search_level, align_iters, out):

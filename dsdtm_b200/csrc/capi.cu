@@ -302,7 +302,7 @@ void dsdtm_destroy(dsdtm_ctx* c)
     if (!c) return;
     cudaSetDevice(c->device);
     if (c->stream) cudaStreamSynchronize(c->stream);
-    for (int k = 0; k < 4; ++k) if (c->batch.graph[k]) cudaGraphExecDestroy(c->batch.graph[k]);
+    for (int k = 0; k < 8; ++k) if (c->batch.graph[k]) cudaGraphExecDestroy(c->batch.graph[k]);
     void* bufs[] = { c->frames_d, c->cells_d, c->occupied_d, c->scoremap_d, c->fast_tiles_d, c->ref_slots_d, c->cur_slots_d,
                      c->feats_d, c->n_feats_d, c->centers_d, c->poses_in_d, c->poses_out_d, c->n_tracked_d, c->log_d, c->n_log_d,
                      c->patches_d, c->patch_px_d, c->patch_px_in_d, c->patch_level_d, c->patch_slot_d, c->patch_conv_d, c->wa_A_d, c->wa_px_d, c->wa_meta_d, c->sa_ws_d, c->cand_d,
@@ -310,7 +310,8 @@ void dsdtm_destroy(dsdtm_ctx* c)
                      c->depth_d, c->depth_f32_d, c->lift_px_d, c->lift_initial_d, c->lift_out_d, c->clahe_src_d, c->clahe_lut_d,
                      c->po_obs_d, c->po_res_d, c->po_nobs_d, c->po_pose_in_d, c->po_pose_out_d, c->po_sum_d,
                      c->mt_kfs_d, c->mt_pts_d, c->mt_vis_d, c->mt_dist_d,
-                     c->st_kfs_d, c->st_feats_d, c->st_pts_d, c->st_claim_d, c->st_vis_d, c->st_dist_d, c->st_sel_d, c->st_out_d };
+                     c->st_kfs_d, c->st_feats_d, c->st_pts_d, c->st_claim_d, c->st_vis_d, c->st_dist_d, c->st_sel_d, c->st_out_d,
+                     c->trk_found_d, c->trk_match_d, c->trk_obs_d, c->trk_nobs_d, c->trk_pose_in_d, c->trk_pose_out_d, c->trk_res_d, c->trk_sum_d };
     for (void* p : bufs) if (p) cudaFree(p);
     if (c->pinned) cudaFreeHost(c->pinned);
     if (c->stage_pin) cudaFreeHost(c->stage_pin);
@@ -368,25 +369,25 @@ int dsdtm_set_option(dsdtm_ctx* c, const char* key, int value)
     if (std::strcmp(key, "sa_warps_per_pair") == 0) {
         if (value != 0 && value != 1 && value != 2 && value != 3 && value != 4 && value != 5 && value != 6 && value != 10) return fail(c, DSDTM_E_ARG, "sa_warps_per_pair must be 0, 1, 2, 3, 4, 5, 6 or 10");
         c->sa_wpp_override = value;
-        for (int k = 0; k < 4; ++k) if (c->batch.graph[k]) { cudaGraphExecDestroy(c->batch.graph[k]); c->batch.graph[k] = nullptr; }
+        for (int k = 0; k < 8; ++k) if (c->batch.graph[k]) { cudaGraphExecDestroy(c->batch.graph[k]); c->batch.graph[k] = nullptr; }
         return 0;
     }
     if (std::strcmp(key, "sa_variant") == 0) {
         if (value != 0 && value != 1) return fail(c, DSDTM_E_ARG, "sa_variant must be 0 (shared-memory recompute) or 1 (L2 workspace)");
         c->sa_variant = value;
-        for (int k = 0; k < 4; ++k) if (c->batch.graph[k]) { cudaGraphExecDestroy(c->batch.graph[k]); c->batch.graph[k] = nullptr; }
+        for (int k = 0; k < 8; ++k) if (c->batch.graph[k]) { cudaGraphExecDestroy(c->batch.graph[k]); c->batch.graph[k] = nullptr; }
         return 0;
     }
     if (std::strcmp(key, "step_chunks") == 0) {
         if (value < 1 || value > kMaxStepStreams) return fail(c, DSDTM_E_ARG, "step_chunks must be 1..8");
         c->step_chunks = value;
-        for (int k = 0; k < 4; ++k) if (c->batch.graph[k]) { cudaGraphExecDestroy(c->batch.graph[k]); c->batch.graph[k] = nullptr; }
+        for (int k = 0; k < 8; ++k) if (c->batch.graph[k]) { cudaGraphExecDestroy(c->batch.graph[k]); c->batch.graph[k] = nullptr; }
         return 0;
     }
     if (std::strcmp(key, "pyramid_kernel") == 0) {
         if (value != 0 && value != 1 && value != 2) return fail(c, DSDTM_E_ARG, "pyramid_kernel must be 0 (auto: bulk-staged where eligible), 1 (tile) or 2 (register strip)");
         c->pyr_kernel = value;
-        for (int k = 0; k < 4; ++k) if (c->batch.graph[k]) { cudaGraphExecDestroy(c->batch.graph[k]); c->batch.graph[k] = nullptr; }
+        for (int k = 0; k < 8; ++k) if (c->batch.graph[k]) { cudaGraphExecDestroy(c->batch.graph[k]); c->batch.graph[k] = nullptr; }
         return 0;
     }
     if (std::strcmp(key, "pose_opt_solo_max") == 0) {
@@ -1498,7 +1499,7 @@ int dsdtm_batch_stage(dsdtm_ctx* c, int n_pairs, const int* ref_slots, const int
     auto& b = c->batch;
     b.staged = true; b.n_pairs = n_pairs; b.feat_stride = feat_stride; b.max_level = max_level; b.min_level = min_level;
     b.max_iters = max_iters; b.patches_per_pair = ppp; b.align_iters = align_iters;
-    b.map_staged = false;
+    b.map_staged = false; b.track_staged = false;
     return 0;
 }
 
@@ -1513,7 +1514,52 @@ int dsdtm_batch_stage_map(dsdtm_ctx* c, const double* poses_ref_c2w, int points_
     DSDTM_CUDA(c, cudaMemcpyAsync(c->poses_ref_d, poses_ref_c2w, (size_t)b.n_pairs * 7 * sizeof(double), cudaMemcpyHostToDevice, c->stream));
     DSDTM_CUDA(c, cudaStreamSynchronize(c->stream));
     b.map_staged = true; b.map_ppp = points_per_pair; b.max_search_level = max_search_level; b.map_align_iters = align_iters;
-    for (int k = 0; k < 4; ++k) if (b.graph[k]) { cudaGraphExecDestroy(b.graph[k]); b.graph[k] = nullptr; }
+    b.track_staged = false;
+    for (int k = 0; k < 8; ++k) if (b.graph[k]) { cudaGraphExecDestroy(b.graph[k]); b.graph[k] = nullptr; }
+    return 0;
+}
+
+int dsdtm_batch_stage_track(dsdtm_ctx* c, const int32_t* found, int max_iters)
+{
+    if (!c) return DSDTM_E_ARG;
+    auto& b = c->batch;
+    if (!b.staged || !b.map_staged) return fail(c, DSDTM_E_STATE, "dsdtm_batch_stage_track: call dsdtm_batch_stage_map first");
+    if (max_iters < 0) return fail(c, DSDTM_E_ARG, "negative max_iters");
+    if (c->prm.cell_size > track_select_max_radius()) return fail(c, DSDTM_E_ARG, "dsdtm_batch_stage_track: cell_size above the selection's circle bound");
+    if (c->n_cells >= (1 << 22)) return fail(c, DSDTM_E_ARG, "dsdtm_batch_stage_track: too many grid cells");
+    const size_t B = c->prm.max_batch, K = DSDTM_TRACK_MAX_MATCHES;
+    if (!c->trk_found_d) {
+        // once per context at max_batch size: a captured step keeps pointing at these buffers
+        if (dalloc(c, &c->trk_found_d, B * std::max(c->prm.max_patches, 1)) || dalloc(c, &c->trk_match_d, B * K) || dalloc(c, &c->trk_obs_d, B * K) ||
+            dalloc(c, &c->trk_nobs_d, B) || dalloc(c, &c->trk_pose_in_d, B * 7) || dalloc(c, &c->trk_pose_out_d, B * 7) ||
+            dalloc(c, &c->trk_res_d, B * K) || dalloc(c, &c->trk_sum_d, B))
+            return DSDTM_E_NOMEM;
+    }
+    cudaStream_t s = c->stream;
+    const size_t n = (size_t)b.n_pairs * b.map_ppp;
+    std::vector<int32_t> ones;
+    if (!found) { ones.assign(n, 1); found = ones.data(); }                 // MapPoint::mnFound starts at 1
+    DSDTM_CUDA(c, cudaMemcpyAsync(c->trk_found_d, found, n * sizeof(int32_t), cudaMemcpyHostToDevice, s));
+    // rows past a pair's match count are never written by the step: defined (zero) bytes for the fetch
+    DSDTM_CUDA(c, cudaMemsetAsync(c->trk_match_d, 0, B * K * sizeof(dsdtm_match), s));
+    DSDTM_CUDA(c, cudaMemsetAsync(c->trk_res_d, 0, B * K * sizeof(double), s));
+    DSDTM_CUDA(c, cudaStreamSynchronize(s));
+    b.track_staged = true; b.track_iters = max_iters;
+    for (int k = 0; k < 8; ++k) if (b.graph[k]) { cudaGraphExecDestroy(b.graph[k]); b.graph[k] = nullptr; }
+    return 0;
+}
+
+// SearchLocalPoints' selection + PoseOptimization behind the chain (dsdtm_batch_run bit 2), on the buffers of dsdtm_batch_stage_track
+static int enqueue_track(dsdtm_ctx* c, cudaStream_t s, bool timed)
+{
+    auto& b = c->batch;
+    if (timed) stage_begin(c, DSDTM_STAGE_LOCAL_MAP);
+    DSDTM_CUDA(c, launch_track_select(c, b.n_pairs, b.feat_stride, b.map_ppp, s));
+    if (timed) stage_end(c, 1);
+    const PoseOptIo io = { c->trk_obs_d, c->trk_nobs_d, c->trk_pose_in_d, c->trk_pose_out_d, c->trk_res_d, c->trk_sum_d };
+    if (timed) stage_begin(c, DSDTM_STAGE_POSE_OPT);
+    DSDTM_CUDA(c, launch_pose_opt_io(c, io, b.n_pairs, DSDTM_TRACK_MAX_MATCHES, std::min(DSDTM_TRACK_MAX_MATCHES, b.map_ppp), b.track_iters, s));
+    if (timed) stage_end(c, 1);
     return 0;
 }
 
@@ -1556,6 +1602,10 @@ static int enqueue_step(dsdtm_ctx* c, int flags, cudaStream_t s, bool timed)
             DSDTM_CUDA(c, launch_align2d(c, b.n_pairs * b.map_ppp, b.map_align_iters, s));
             DSDTM_CUDA(c, launch_local_map_finalize(c, b.n_pairs * b.map_ppp, s, c->pair_reproj_d, 0));
             if (timed) stage_end(c, 2);
+            if (flags & 4) {
+                int r = enqueue_track(c, s, timed);
+                if (r) return r;
+            }
         } else if (b.patches_per_pair > 0) {
             if (timed) stage_begin(c, DSDTM_STAGE_ALIGN2D);
             DSDTM_CUDA(c, launch_align2d(c, b.n_pairs * b.patches_per_pair, b.align_iters, s));
@@ -1590,7 +1640,9 @@ int dsdtm_batch_run(dsdtm_ctx* c, int flags)
     auto& b = c->batch;
     if (!b.staged) return fail(c, DSDTM_E_STATE, "dsdtm_batch_run: no staged batch");
     if ((flags & 2) && !b.map_staged) return fail(c, DSDTM_E_STATE, "dsdtm_batch_run: flags bit 1 needs dsdtm_batch_stage_map");
-    const int gi = flags & 3;
+    if ((flags & 4) && !(flags & 2)) return fail(c, DSDTM_E_STATE, "dsdtm_batch_run: flags bit 2 needs bit 1 (the refinement chain)");
+    if ((flags & 4) && !b.track_staged) return fail(c, DSDTM_E_STATE, "dsdtm_batch_run: flags bit 2 needs dsdtm_batch_stage_track");
+    const int gi = flags & 7;
     DSDTM_CUDA(c, cudaEventRecord(c->ev_a, c->stream));
     if (c->profiling) {
         // per-stage events cannot be recorded inside a captured graph: launch directly
@@ -1618,7 +1670,7 @@ int dsdtm_batch_run(dsdtm_ctx* c, int flags)
         DSDTM_CUDA(c, cudaGraphLaunch(b.graph[gi], c->stream));
         {
             const int chunks = (c->step_chunks <= 1 || b.n_pairs < 4 * c->sm_count) ? 1 : std::min(c->step_chunks, kMaxStepStreams);
-            if (flags & 2) c->launches += ((flags & 1) ? c->geo.levels - 1 : 0) + 1 + 5;
+            if (flags & 2) c->launches += ((flags & 1) ? c->geo.levels - 1 : 0) + 1 + 5 + ((flags & 4) ? 2 : 0);
             else c->launches += ((flags & 1) ? c->geo.levels - 1 : 0) + (long long)chunks * (1 + (b.patches_per_pair > 0 ? 1 : 0));
         }
     }
@@ -1650,6 +1702,25 @@ int dsdtm_batch_fetch_map(dsdtm_ctx* c, dsdtm_reproj* reproj_out)
     if (!b.staged || !b.map_staged) return fail(c, DSDTM_E_STATE, "dsdtm_batch_fetch_map: no staged map batch");
     DSDTM_CUDA(c, cudaMemcpyAsync(reproj_out, c->pair_reproj_d, (size_t)b.n_pairs * b.map_ppp * sizeof(dsdtm_reproj), cudaMemcpyDeviceToHost, c->stream));
     DSDTM_CUDA(c, cudaStreamSynchronize(c->stream));
+    return 0;
+}
+
+int dsdtm_batch_fetch_track(dsdtm_ctx* c, double* poses_c2w_out, int32_t* n_matches, dsdtm_match* matches, double* res_norm,
+                            dsdtm_ba_summary* summaries)
+{
+    if (!c) return DSDTM_E_ARG;
+    auto& b = c->batch;
+    if (!b.staged || !b.map_staged || !b.track_staged) return fail(c, DSDTM_E_STATE, "dsdtm_batch_fetch_track: no staged track batch");
+    cudaStream_t s = c->stream;
+    const size_t n = (size_t)b.n_pairs, K = DSDTM_TRACK_MAX_MATCHES;
+    if (poses_c2w_out) DSDTM_CUDA(c, cudaMemcpyAsync(poses_c2w_out, c->trk_pose_out_d, n * 7 * sizeof(double), cudaMemcpyDeviceToHost, s));
+    if (n_matches) DSDTM_CUDA(c, cudaMemcpyAsync(n_matches, c->trk_nobs_d, n * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+    if (matches) DSDTM_CUDA(c, cudaMemcpyAsync(matches, c->trk_match_d, n * K * sizeof(dsdtm_match), cudaMemcpyDeviceToHost, s));
+    if (res_norm) DSDTM_CUDA(c, cudaMemcpyAsync(res_norm, c->trk_res_d, n * K * sizeof(double), cudaMemcpyDeviceToHost, s));
+    if (summaries) DSDTM_CUDA(c, cudaMemcpyAsync(summaries, c->trk_sum_d, n * sizeof(dsdtm_ba_summary), cudaMemcpyDeviceToHost, s));
+    DSDTM_CUDA(c, cudaStreamSynchronize(s));
+    float ms = 0.f;
+    if (cudaEventElapsedTime(&ms, c->ev_a, c->ev_b) == cudaSuccess) c->last_run_ms = ms;
     return 0;
 }
 

@@ -135,6 +135,16 @@ struct dsdtm_ctx {
     double* po_pose_out_d = nullptr;     size_t po_pose_out_cap = 0;
     dsdtm_ba_summary* po_sum_d = nullptr; size_t po_sum_cap = 0;
     int po_solo_max = -1;                        // frames up to which a CTA of eight warps owns a frame (-1: the SM count); 0 = always one warp per frame
+    // selection + pose optimization behind the batched chain (dsdtm_batch_stage_track): allocated once at max_batch size, owned by the
+    // captured step (dsdtm_pose_optimize_batch's po_* buffers may be reallocated between two replays)
+    int* trk_found_d = nullptr;                  // max_batch * max_patches found counts
+    dsdtm_match* trk_match_d = nullptr;          // max_batch * DSDTM_TRACK_MAX_MATCHES
+    dsdtm_ba_obs* trk_obs_d = nullptr;           // max_batch * DSDTM_TRACK_MAX_MATCHES
+    int* trk_nobs_d = nullptr;                   // max_batch: matches per pair
+    double* trk_pose_in_d = nullptr;             // max_batch * 7: cur.Get_Pose() after Run
+    double* trk_pose_out_d = nullptr;            // max_batch * 7: after PoseOptimization
+    double* trk_res_d = nullptr;                 // max_batch * DSDTM_TRACK_MAX_MATCHES
+    dsdtm_ba_summary* trk_sum_d = nullptr;       // max_batch
 
     // pinned host staging for small synchronous calls
     uint8_t* pinned = nullptr;
@@ -149,8 +159,10 @@ struct dsdtm_ctx {
         int patches_per_pair = 0, align_iters = 0;
         bool map_staged = false;                           // dsdtm_batch_stage_map: the refinement chain's inputs are on the device
         int map_ppp = 0, max_search_level = 0, map_align_iters = 0;
-        cudaGraphExec_t graph[4] = { nullptr, nullptr, nullptr, nullptr };   // [flags & 3]
-        int graph_key[4][8];
+        bool track_staged = false;                         // dsdtm_batch_stage_track: selection + pose optimization buffers are ready
+        int track_iters = 0;
+        cudaGraphExec_t graph[8] = {};                     // [flags & 7]
+        int graph_key[8][8];
     } batch;
 };
 
@@ -217,6 +229,15 @@ cudaError_t launch_close_keyframes(dsdtm_ctx* c, const double pose_cur[7], int n
 cudaError_t pose_opt_init(dsdtm_ctx* c);
 cudaError_t launch_pose_opt(dsdtm_ctx* c, int n_frames, int obs_stride, int max_obs, int max_iters, bool want_res, bool want_sum,
                             cudaStream_t s);
+// the same solve on explicit device buffers (res / sum may be null)
+struct PoseOptIo {
+    const dsdtm_ba_obs* obs; const int* n_obs; const double* pose_in;
+    double* pose_out; double* res; dsdtm_ba_summary* sum;
+};
+cudaError_t launch_pose_opt_io(dsdtm_ctx* c, const PoseOptIo& io, int n_frames, int obs_stride, int max_obs, int max_iters, cudaStream_t s);
+// SearchLocalPoints' selection over the batched chain's records + the PoseOptimization inputs of every pair (select.cu)
+cudaError_t launch_track_select(dsdtm_ctx* c, int n_pairs, int feat_stride, int ppp, cudaStream_t s);
+int track_select_max_radius();                 // largest Camera.CellSize the selection's circle table holds
 int sparse_align_smem_bytes(int nf_pad);
 size_t sparse_align_ws_doubles(int max_feats);
 cudaError_t sparse_align_init(dsdtm_ctx* c);

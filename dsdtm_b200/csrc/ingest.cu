@@ -96,11 +96,7 @@ __global__ void __launch_bounds__(128) keyframe_lift_kernel(const LiftArgs a)
     const float ux = __double2float_rn(__dadd_rn(__dmul_rn(fx, x), cx)), uy = __double2float_rn(__dadd_rn(__dmul_rn(fy, y), cy));
     o.px[0] = ux; o.px[1] = uy;
     // ---- mNormal = Pixel2Camera(px, 1.0).normalize()  (float evaluation, ref: src/Camera.cpp:173-178, src/Frame.cpp:146-147)
-    {
-        const double n0 = (double)__fdiv_rn(__fmul_rn(1.0f, __fsub_rn(ux, a.cx)), a.fx), n1 = (double)__fdiv_rn(__fmul_rn(1.0f, __fsub_rn(uy, a.cy)), a.fy), n2 = 1.0;
-        const double nn = sqrt(__dadd_rn(__dadd_rn(__dmul_rn(n0, n0), __dmul_rn(n1, n1)), __dmul_rn(n2, n2)));
-        o.normal[0] = __ddiv_rn(n0, nn); o.normal[1] = __ddiv_rn(n1, nn); o.normal[2] = __ddiv_rn(n2, nn);
-    }
+    feature_normal_exact(ux, uy, a.fx, a.fy, a.cx, a.cy, o.normal);
     o.status = DSDTM_LIFT_NO_DEPTH; o.depth = -1.0f;
     if (a.depth) {
         // ---- Get_FeatureDetph (ref: src/Frame.cpp:200-224)

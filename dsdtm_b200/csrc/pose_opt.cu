@@ -58,26 +58,32 @@ cudaError_t pose_opt_init(dsdtm_ctx*)
     return cudaFuncSetAttribute(pose_opt_solo_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kPoseOptSmemLimit);
 }
 
-// max_obs = the largest n_obs of the batch (sizes the shared-memory slice of a frame: 48 bytes per observation)
-cudaError_t launch_pose_opt(dsdtm_ctx* c, int n_frames, int obs_stride, int max_obs, int max_iters, bool want_res, bool want_sum,
-                            cudaStream_t s)
+// max_obs = an upper bound of the batch's n_obs (sizes the shared-memory slice of a frame: 48 bytes per observation; the slice is
+// laid out by the frame's own n_obs, so the bound never changes a result)
+cudaError_t launch_pose_opt_io(dsdtm_ctx* c, const PoseOptIo& io, int n_frames, int obs_stride, int max_obs, int max_iters, cudaStream_t s)
 {
     const int soa_stride = 6 * ((max_obs + 1) & ~1);
     const size_t per_frame = (size_t)soa_stride * sizeof(double);
-    double* rn = want_res ? c->po_res_d : nullptr;
-    dsdtm_ba_summary* sm = want_sum ? c->po_sum_d : nullptr;
     const int solo_max = c->po_solo_max >= 0 ? c->po_solo_max : c->sm_count;   // one solo CTA per SM: 64 frames 108 us; two per SM (296 frames) 189 us vs 167 us for the sweep kernel
     if (n_frames <= solo_max) {
-        pose_opt_solo_kernel<<<n_frames, kSoloWarps * 32, per_frame, s>>>(c->po_obs_d, obs_stride, c->po_nobs_d, c->po_pose_in_d, max_iters,
-                                                                        c->po_pose_out_d, rn, sm);
+        pose_opt_solo_kernel<<<n_frames, kSoloWarps * 32, per_frame, s>>>(io.obs, obs_stride, io.n_obs, io.pose_in, max_iters, io.pose_out,
+                                                                        io.res, io.sum);
     } else {
         int wpc = kSweepWarps;                     // frames per CTA, while their slices fit
         while (wpc > 1 && wpc * per_frame > (size_t)kPoseOptSmemLimit) wpc >>= 1;
-        pose_opt_sweep_kernel<<<(n_frames + wpc - 1) / wpc, wpc * 32, wpc * per_frame, s>>>(n_frames, c->po_obs_d, obs_stride, c->po_nobs_d,
-                                                                                         c->po_pose_in_d, max_iters, c->po_pose_out_d, rn, sm, soa_stride);
+        pose_opt_sweep_kernel<<<(n_frames + wpc - 1) / wpc, wpc * 32, wpc * per_frame, s>>>(n_frames, io.obs, obs_stride, io.n_obs,
+                                                                                         io.pose_in, max_iters, io.pose_out, io.res, io.sum, soa_stride);
     }
     c->launches++;
     return cudaGetLastError();
+}
+
+cudaError_t launch_pose_opt(dsdtm_ctx* c, int n_frames, int obs_stride, int max_obs, int max_iters, bool want_res, bool want_sum,
+                            cudaStream_t s)
+{
+    const PoseOptIo io = { c->po_obs_d, c->po_nobs_d, c->po_pose_in_d, c->po_pose_out_d, want_res ? c->po_res_d : nullptr,
+                           want_sum ? c->po_sum_d : nullptr };
+    return launch_pose_opt_io(c, io, n_frames, obs_stride, max_obs, max_iters, s);
 }
 
 }  // namespace dsdtm

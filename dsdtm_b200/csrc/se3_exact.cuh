@@ -42,4 +42,13 @@ __device__ __forceinline__ void se3_mul_exact(const double* A, const double* B, 
     o[4] = t0; o[5] = t1; o[6] = t2;
 }
 
+// Feature::mNormal = Pixel2Camera(px, 1.0).normalize(): float evaluation of the camera ray, widened, then normalised in fp64
+// (ref: src/Camera.cpp:173-178, src/Frame.cpp:83-92,146-147; Q8)
+__device__ __forceinline__ void feature_normal_exact(float ux, float uy, float fx, float fy, float cx, float cy, double* o)
+{
+    const double n0 = (double)__fdiv_rn(__fmul_rn(1.0f, __fsub_rn(ux, cx)), fx), n1 = (double)__fdiv_rn(__fmul_rn(1.0f, __fsub_rn(uy, cy)), fy), n2 = 1.0;
+    const double nn = sqrt(__dadd_rn(__dadd_rn(__dmul_rn(n0, n0), __dmul_rn(n1, n1)), __dmul_rn(n2, n2)));
+    o[0] = __ddiv_rn(n0, nn); o[1] = __ddiv_rn(n1, nn); o[2] = __ddiv_rn(n2, nn);
+}
+
 }  // namespace dsdtm

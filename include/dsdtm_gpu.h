@@ -447,7 +447,8 @@ int dsdtm_track_frame_store(dsdtm_ctx* ctx, const dsdtm_track_store_in* in, dsdt
 /* One "step" over n_pairs independent frame pairs: [pyramid(cur)] -> sparse align -> Align2D of the pair's patches
  * against its cur frame. Inputs are staged once (H2D), run() only launches kernels on HBM-resident data (CUDA-graph
  * replayed), fetch() copies results back. patches: n_pairs * patches_per_pair entries, patch_level < 0 = unused.
- * flags bit0: rebuild the cur pyramids from their level 0 inside run(). */
+ * flags bit0: rebuild the cur pyramids from their level 0 inside run(); bit1: the refinement chain (dsdtm_batch_stage_map);
+ * bit2 (with bit1): selection + pose optimization behind it (dsdtm_batch_stage_track). */
 int dsdtm_batch_stage(dsdtm_ctx* ctx, int n_pairs, const int* ref_slots, const int* cur_slots,
                       const dsdtm_ref_feat* feats, int feat_stride, const int* n_feats, const double* ref_centers,
                       const double* poses_in, int max_level, int min_level, int max_iters,
@@ -461,9 +462,37 @@ int dsdtm_batch_run(dsdtm_ctx* ctx, int flags);
  * dsdtm_batch_run(flags | 2) runs pyramid -> sparse alignment -> pose composition + reprojection + closest observation + gates ->
  * SolveAffineMatrix / GetBestSearchLevel -> WarpAffine -> Align2DGaussNewton for every candidate, all on the device, and
  * fetch_map returns n_pairs x points_per_pair records (obs = feature index; cell, flags, level, refined px as in
- * dsdtm_local_map_align_batch). The greedy per-cell selection of SearchLocalPoints stays with the caller. */
+ * dsdtm_local_map_align_batch). The greedy per-cell selection of SearchLocalPoints stays with the caller unless flags bit 2 runs it
+ * on the device (dsdtm_batch_stage_track below). */
 int dsdtm_batch_stage_map(dsdtm_ctx* ctx, const double* poses_ref_c2w, int points_per_pair, int max_search_level, int align_iters);
 int dsdtm_batch_fetch_map(dsdtm_ctx* ctx, dsdtm_reproj* reproj_out /* n_pairs x points_per_pair */);
+/* The rest of Tracking::TrackWithLocalMap behind the chain (ref: src/Tracking.cpp:219-236): SearchLocalPoints' selection
+ * (ref: src/Feature_alignment.cpp:71-121) and Optimizer::PoseOptimization (ref: src/Optimizer.cpp:20-101) on the device, so that
+ * dsdtm_batch_run(flags | 2 | 4) ends in the tracked pose of every pair. Selection over a pair's records: cells in index order;
+ * a cell's candidates (feature index order = the ReprojectPoint order) stably sorted by found count, descending; a candidate is
+ * skipped when the mask at cvRound((float)px_proj) is painted, when OBS_OK | REF_OK is incomplete, when level < 0 or when it did
+ * not converge; the first other candidate is the cell's match (Feature(px as Point2f, level), ref: :100-113) and paints a filled
+ * circle of radius Camera.CellSize at cvRound of that px; 200 matches (the reference's literal, :75) end the search. The mask
+ * starts all free (a new Frame). Then one dsdtm_ba_obs per match in match order (normal = Frame::Add_Feature's bearing of the
+ * float px, point_w = the staged feature's point, the match level) and PoseOptimization from cur.Get_Pose() after Run
+ * (T_c2r * T_ref, ref: src/Sprase_ImageAlign.cpp:57), with the solver of dsdtm_pose_optimize_batch for the same n_pairs. */
+typedef struct {
+    int32_t point;          /* feature index of the pair's staged dsdtm_ref_feat records (its map point) */
+    float   px[2];          /* Feature::mpx of the new feature: Point2f of the refined position, level 0 */
+    int32_t level;          /* Feature::mlevel: the search level */
+} dsdtm_match;              /* 16 bytes */
+#define DSDTM_TRACK_MAX_MATCHES 200
+/* after dsdtm_batch_stage_map: found = n_pairs x points_per_pair MapPoint::mnFound counts (NULL = all 1, the value a new map point
+ * starts with), max_iters = PoseOptimization's iteration cap (100 in the reference). Allocates the buffers of the selection and
+ * the solve, which the replayed step owns. Calling dsdtm_batch_stage or dsdtm_batch_stage_map again drops this staging. */
+int dsdtm_batch_stage_track(dsdtm_ctx* ctx, const int32_t* found, int max_iters);
+/* after dsdtm_batch_run(flags | 2 | 4): poses_c2w_out = n_pairs x 7, the argument of Frame::Set_Pose after PoseOptimization;
+ * n_matches = n_pairs; matches = n_pairs x DSDTM_TRACK_MAX_MATCHES (mvFeatures order, the first n_matches[i] valid);
+ * res_norm = n_pairs x DSDTM_TRACK_MAX_MATCHES, GetReprojectReidual() at the final pose per match (ref: src/Optimizer.cpp:298-318):
+ * the caller compares it with LocalBAthreshhold / Camera.f to call MapPoint::EraseFound (ref: :81-94) and keeps the found counts
+ * itself; summaries = n_pairs. Every pointer may be NULL. */
+int dsdtm_batch_fetch_track(dsdtm_ctx* ctx, double* poses_c2w_out, int32_t* n_matches, dsdtm_match* matches, double* res_norm,
+                            dsdtm_ba_summary* summaries);
 int dsdtm_batch_fetch(dsdtm_ctx* ctx, double* poses_out, int* n_tracked, double* patch_px_out, uint8_t* patch_conv);
 /* end-to-end step with HOST buffers: uploads the n_pairs cur images (dense, pinned recommended) into their cur slots,
  * stages the per-pair inputs, runs, and fetches -- copies overlapped with compute in chunks on internal streams. */
