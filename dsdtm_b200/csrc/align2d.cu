@@ -1,13 +1,13 @@
-// align2d.cu -- kernel (d): batched 2-D inverse-compositional patch alignment, one WARP per 8x8 feature patch,
+// align2d.cu -- kernel (d): batched 2-D inverse-compositional patch alignment, an 8-lane group per 8x8 feature patch,
 // and the affine patch warp that feeds it.
 //
 // align2d_kernel replaces Feature_Alignment::Align2DGaussNewton (ref: src/Feature_alignment.cpp:318-417), fp32 like the
 // reference: H = sum J J^T over the 8x8 interior of the 10x10 bordered patch (exact in fp32: quarter-integers < 2^22),
 // Hinv by the 3x3 cofactor formula (Eigen Matrix3f::inverse), then <= max_iters iterations of bilinear sampling,
 // Jres accumulation and the (u, v, mean) update; converged iff du^2 + dv^2 < 0.03^2.
-// One half-warp per patch: lane l owns 4 pixels; the three Jres sums are reduced with a 16-lane xor-shuffle butterfly (bitwise
-// identical in every lane of the half => uniform control flow per patch). The reference sums the 64 terms sequentially in fp32, the butterfly
-// is a tree: documented tolerance 1e-3 px on the refined position.
+// Eight lanes per patch: lane (g, m) owns 8 pixels; the three Jres sums are reduced with an xor-shuffle tree (bitwise identical in
+// every lane of the group => uniform control flow per patch). The reference sums the 64 terms sequentially in fp32, the tree
+// differs: documented tolerance 1e-3 px on the refined position.
 // Q4 (ref: :367-368 uses '>' where SVO uses '>='): with u_r == cols-4 or v_r == rows-4 the reference reads one byte past
 // the row / image. We reproduce the linear addressing (next row's first pixel) and read bytes past the end of the level
 // image as 0, identically in the oracle.
@@ -35,68 +35,79 @@ struct A2dArgs {
     dsdtm_store_cand* store_out;   // optional: fold (px * 2^level, level, converged) into the map-store records (ref: :154-156)
 };
 
-constexpr int A2D_WARPS = 8;          // 8 warps = 16 patches per CTA
+constexpr int A2D_WARPS = 8;          // 8 warps = 32 patches per CTA
+constexpr int A2D_PPW = 4;            // patches per warp: 8 lanes per patch
 
-// sum over the 16 lanes of a half-warp (xor butterfly with offsets < 16 never crosses the half)
-__device__ __forceinline__ float hsum(float v)
-{
-#pragma unroll
-    for (int o = 8; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    return v;
-}
-__device__ __forceinline__ int hsum_i(int v)
-{
-#pragma unroll
-    for (int o = 8; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-    return v;
-}
-
-// v2: one HALF-warp per patch (16 lanes x 4 pixels). The per-patch scalar work (weights, 3x3 update, control) is shared by
-// two patches per warp instruction and the butterflies are 4 levels deep instead of 5: ~35 % fewer instructions per patch
-// than the warp-per-patch v1, which was issue-bound (71 % issue slots busy, profiles/r1_pyramid_fast_align2d.md).
-// v3: a lane owns four CONSECUTIVE rows of one column, so its 4 x (2 x 2) bilinear taps are a 5 x 2 block: 10 byte loads and
-// conversions per iteration instead of 16, one inside/edge branch per iteration instead of four; registers capped at 48
-// (5 CTAs per SM). 0.756 -> 0.632 ms per 1.23 M patches.
+// v4: an 8-lane group per patch, four patches per warp. The per-patch scalar work (bilinear weights, Hinv * J, the update, the
+// convergence test, loop control) is shared by four patches per warp instruction instead of two. Lane (g, m) = (l8 >> 2, l8 & 3)
+// owns columns 2m, 2m + 1 and rows 4g .. 4g + 3 of the 8x8 interior; its taps are a 5 x 3 block (15 byte loads for 8 pixels), and
+// both columns share one set of weights, so the per-pixel arithmetic runs as paired fp32 (FMUL2 / FADD2) on float2 (x = column 2m,
+// y = column 2m + 1).
+// Bit-equal to v3 (one half-warp per patch, lane = one column x four rows, xor butterfly 8, 4, 2, 1): every column is still summed
+// sequentially over its four rows, and the tree below adds the same operands at every level -- xor 4 (row groups, v3's xor 8),
+// xor 2 (columns c ^ 4, v3's xor 4), xor 1 (columns c ^ 2, v3's xor 2), then the two columns of a lane (v3's xor 1). IEEE addition
+// is commutative, so both lanes of a pair hold the same value and control flow stays uniform per patch.
+// No multiply-add is contracted: ptxas fuses FMUL2 -> FADD2 into FFMA2 even with the _rn intrinsics, so every product -> sum edge
+// has exactly one paired side (tests/test_align2d_sass.py checks the SASS).
+// Iterations on the bench batch are 2 or 3 for 99.8 % of the patches (profiles/r4_a2d_iter_hist.json): waiting for the slowest of
+// four patches costs 7 % more lane-iterations than the slowest of two, far less than the amortised scalar work saves.
 #ifndef DSDTM_A2D_MINB
-#define DSDTM_A2D_MINB 5      // 48 registers: 0.632 ms per 1.23 M patches (1 -> 74 regs 0.809, 6 -> 40 regs 0.633, 8 -> 32 regs 0.739)
+#define DSDTM_A2D_MINB 3      // 80 registers, no spills (2 -> 101 registers; 4 -> 64 registers, 36 B spilled); per-cap times not measured
 #endif
+// reduce the three Jres sums of a patch (see above); on return every lane of the group holds the same three values
+__device__ __forceinline__ float a2d_sum(float2 s, int g)
+{
+    s = __fadd2_rn(s, make_float2(__shfl_xor_sync(0xffffffffu, s.x, 4), __shfl_xor_sync(0xffffffffu, s.y, 4)));
+    float v = g ? s.y : s.x;                              // column 2m + g: v3's xor 4 and xor 2 partners own the same parity
+    v = __fadd_rn(v, __shfl_xor_sync(0xffffffffu, v, 2));
+    v = __fadd_rn(v, __shfl_xor_sync(0xffffffffu, v, 1));
+    return __fadd_rn(v, __shfl_xor_sync(0xffffffffu, v, 4));   // even + odd columns (v3's xor 1)
+}
+__device__ __forceinline__ int a2d_sum_i(int v)
+{
+#pragma unroll
+    for (int o = 4; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    return v;
+}
+__device__ __forceinline__ float2 f2(float a) { return make_float2(a, a); }
+
 __global__ void __launch_bounds__(A2D_WARPS * 32, DSDTM_A2D_MINB) align2d_kernel(const A2dArgs a)
 {
-    __shared__ __align__(16) uint8_t s_patch[A2D_WARPS * 2][104];
-    const int half = threadIdx.x >> 4, l16 = threadIdx.x & 15;
+    __shared__ __align__(16) uint8_t s_patch[A2D_WARPS * A2D_PPW][104];
+    const int grp = threadIdx.x >> 3, l8 = threadIdx.x & 7, g = l8 >> 2, m = l8 & 3;
     const int n_eff = a.n_dev ? min(a.n, *a.n_dev) : a.n;
     const int last = a.patch0 + n_eff - 1;
-    const int iraw = a.patch0 + blockIdx.x * (A2D_WARPS * 2) + half;
-    if (iraw - (half & 1) > last) return;                 // whole warp out of range (both halves)
+    const int iraw = a.patch0 + blockIdx.x * (A2D_WARPS * A2D_PPW) + grp;
+    if (iraw - (grp & (A2D_PPW - 1)) > last) return;      // whole warp out of range
     const bool exists = iraw <= last;
-    const int i = exists ? iraw : last;                   // a missing odd half shadows the last patch and never writes
+    const int i = exists ? iraw : last;                   // a missing group shadows the last patch and never writes
     const int L = a.patch_level[i];
     bool active = exists && L >= 0;
-    if (exists && L < 0 && l16 == 0) { a.conv[i] = 0; a.px[2 * i] = a.px_in[2 * i]; a.px[2 * i + 1] = a.px_in[2 * i + 1]; }
+    if (exists && L < 0 && l8 == 0) { a.conv[i] = 0; a.px[2 * i] = a.px_in[2 * i]; a.px[2 * i + 1] = a.px_in[2 * i + 1]; }
     const int Lc = L < 0 ? 0 : L;
 
     // stage the 10x10 bordered patch (100 bytes = 25 words; patch10 rows are 4-byte aligned because 100 % 4 == 0)
-    for (int q = l16; q < 25; q += 16)
-        reinterpret_cast<uint32_t*>(s_patch[half])[q] = __ldg(reinterpret_cast<const uint32_t*>(a.patch10 + (size_t)i * 100) + q);
+    for (int q = l8; q < 25; q += 8)
+        reinterpret_cast<uint32_t*>(s_patch[grp])[q] = __ldg(reinterpret_cast<const uint32_t*>(a.patch10 + (size_t)i * 100) + q);
     __syncwarp();
 
-    // lane owns column pc = l16 & 7 and the four CONSECUTIVE rows 4 * (l16 >> 3) + k (k = 0..3) of the 8x8 interior: its
-    // bilinear taps are a 5 x 2 block of the current image (10 byte loads per iteration instead of 16)
-    const int pc = l16 & 7, pr0 = (l16 >> 3) * 4;
-    float rdx[4], rdy[4], rref[4];
+    // negated gradients and reference (exact): s - ref == s + (-ref) and j - res * d == j + res * (-d) bit for bit
+    float2 ndx[4], ndy[4], nref[4];
     int i00 = 0, i01 = 0, i02 = 0, i11 = 0, i12 = 0;      // sums of the integer pixel differences (2*dx, 2*dy)
 #pragma unroll
     for (int k = 0; k < 4; ++k) {
-        const uint8_t* it = s_patch[half] + (pr0 + k + 1) * 10 + 1 + pc;
-        const int ddx = (int)it[1] - (int)it[-1], ddy = (int)it[10] - (int)it[-10];
-        rdx[k] = 0.5f * (float)ddx;                        // ref: :336 (exact half-integers)
-        rdy[k] = 0.5f * (float)ddy;                        // ref: :337
-        rref[k] = (float)it[0];
-        i00 += ddx * ddx; i01 += ddx * ddy; i02 += ddx; i11 += ddy * ddy; i12 += ddy;
+        const uint8_t* it = s_patch[grp] + (4 * g + k + 1) * 10 + 1 + 2 * m;
+        const int dx0 = (int)it[1] - (int)it[-1], dy0 = (int)it[10] - (int)it[-10];
+        const int dx1 = (int)it[2] - (int)it[0], dy1 = (int)it[11] - (int)it[-9];
+        ndx[k] = make_float2(-0.5f * (float)dx0, -0.5f * (float)dx1);        // ref: :336 (exact half-integers)
+        ndy[k] = make_float2(-0.5f * (float)dy0, -0.5f * (float)dy1);        // ref: :337
+        nref[k] = make_float2(-(float)it[0], -(float)it[1]);
+        i00 += dx0 * dx0 + dx1 * dx1; i01 += dx0 * dy0 + dx1 * dy1; i02 += dx0 + dx1;
+        i11 += dy0 * dy0 + dy1 * dy1; i12 += dy0 + dy1;
     }
     // H = sum J J^T with J = (dx, dy, 1): every entry is an integer / 4 (or / 2) below 2^22, exact in fp32 in any order
-    const float h00 = 0.25f * (float)hsum_i(i00), h01 = 0.25f * (float)hsum_i(i01), h02 = 0.5f * (float)hsum_i(i02);
-    const float h11 = 0.25f * (float)hsum_i(i11), h12 = 0.5f * (float)hsum_i(i12);
+    const float h00 = 0.25f * (float)a2d_sum_i(i00), h01 = 0.25f * (float)a2d_sum_i(i01), h02 = 0.5f * (float)a2d_sum_i(i02);
+    const float h11 = 0.25f * (float)a2d_sum_i(i11), h12 = 0.5f * (float)a2d_sum_i(i12);
     const float h22 = 64.0f;
     // Eigen 3x3 inverse: cofactor(i,j) = m(i1,j1) m(i2,j2) - m(i1,j2) m(i2,j1); det = sum_i cof(i,0) m(i,0)
     float Hinv[9];
@@ -107,7 +118,12 @@ __global__ void __launch_bounds__(A2D_WARPS * 32, DSDTM_A2D_MINB) align2d_kernel
                             __fmul_rn(M(((i) + 1) % 3, ((j) + 2) % 3), M(((i) + 2) % 3, ((j) + 1) % 3)))
         const float c00 = COF(0, 0), c10 = COF(1, 0), c20 = COF(2, 0);
         const float det = __fadd_rn(__fadd_rn(__fmul_rn(c00, M(0, 0)), __fmul_rn(c10, M(1, 0))), __fmul_rn(c20, M(2, 0)));
-        const float invdet = __fdiv_rn(1.0f, det);
+        // 1 / det rounded to fp64 and then to fp32 equals the fp32 quotient (double rounding is innocuous for a division when
+        // 53 >= 2 * 24 + 2). __fdiv_rn's refinement would put FFMAs into the kernel's SASS; in inline PTX the compiler cannot
+        // narrow the fp64 division back to it.
+        double rdet;
+        asm("div.rn.f64 %0, %1, %2;" : "=d"(rdet) : "d"(1.0), "d"((double)det));
+        const float invdet = (float)rdet;
         Hinv[0] = __fmul_rn(c00, invdet); Hinv[1] = __fmul_rn(c10, invdet); Hinv[2] = __fmul_rn(c20, invdet);
         Hinv[3] = __fmul_rn(COF(0, 1), invdet); Hinv[4] = __fmul_rn(COF(1, 1), invdet); Hinv[5] = __fmul_rn(COF(2, 1), invdet);
         Hinv[6] = __fmul_rn(COF(0, 2), invdet); Hinv[7] = __fmul_rn(COF(1, 2), invdet); Hinv[8] = __fmul_rn(COF(2, 2), invdet);
@@ -127,52 +143,59 @@ __global__ void __launch_bounds__(A2D_WARPS * 32, DSDTM_A2D_MINB) align2d_kernel
         const float uf = floorf(u), vf = floorf(v);
         // ref: :367-369 (Q4 '>'); written on floats so that NaN / huge values break like the reference
         if (active && !(uf >= 4.f && vf >= 4.f && uf <= (float)(cols - 4) && vf <= (float)(rows - 4))) active = false;
-        if (!__any_sync(0xffffffffu, active)) break;       // both patches of the warp are done
-        // a finished half keeps executing the (warp-wide) shuffles on clamped coordinates and discards the result
+        if (!__any_sync(0xffffffffu, active)) break;       // all four patches of the warp are done
+        // a finished group keeps executing the (warp-wide) shuffles on clamped coordinates and discards the result
         const int u_r = active ? (int)uf : 4, v_r = active ? (int)vf : 4;
         const float sx = active ? u - uf : 0.f, sy = active ? v - vf : 0.f;
         const float wTL = (float)((1.0 - (double)sx) * (1.0 - (double)sy));   // ref: :373 (double arithmetic, narrowed)
         const float wTR = __fmul_rn(sx, 1.0f - sy);                          // ref: :374 (float arithmetic)
         const float wBL = (float)((1.0 - (double)sx) * (double)sy);          // ref: :375
         const float wBR = __fmul_rn(sx, sy);                                 // ref: :376
-        float j0 = 0.f, j1 = 0.f, j2 = 0.f;
-        const unsigned o0 = (unsigned)(v_r + pr0 - 4) * (unsigned)cols + (unsigned)(u_r - 4 + pc);
+        const unsigned o0 = (unsigned)(v_r + 4 * g - 4) * (unsigned)cols + (unsigned)(u_r - 4 + 2 * m);
         // the whole 9x9 window lies inside the level image unless the Q4 edge case is hit (u_r == cols-4 or v_r == rows-4)
         const bool inside = (u_r + 4 < cols) && (v_r + 4 < rows);
-        float pl[5], pr[5];                                 // left / right tap of rows pr0 .. pr0 + 4
+        float2 tl[5], tr[5];                                // taps (2m, 2m+1) and (2m+1, 2m+2) of rows 4g .. 4g + 4
         if (inside) {
 #pragma unroll
             for (int k = 0; k < 5; ++k) {
                 const unsigned o = o0 + (unsigned)k * (unsigned)cols;
-                pl[k] = (float)__ldg(img + o); pr[k] = (float)__ldg(img + o + 1);
+                const float p0 = (float)__ldg(img + o), p1 = (float)__ldg(img + o + 1), p2 = (float)__ldg(img + o + 2);
+                tl[k] = make_float2(p0, p1); tr[k] = make_float2(p1, p2);
             }
         } else {                                            // ref: linear addressing, zeros past the end of the level image (Q4)
 #pragma unroll
             for (int k = 0; k < 5; ++k) {
                 const unsigned o = o0 + (unsigned)k * (unsigned)cols;
-                pl[k] = (float)(o < img_bytes ? __ldg(img + o) : 0);
-                pr[k] = (float)(o + 1 < img_bytes ? __ldg(img + o + 1) : 0);
+                const float p0 = (float)(o < img_bytes ? __ldg(img + o) : 0);
+                const float p1 = (float)(o + 1 < img_bytes ? __ldg(img + o + 1) : 0);
+                const float p2 = (float)(o + 2 < img_bytes ? __ldg(img + o + 2) : 0);
+                tl[k] = make_float2(p0, p1); tr[k] = make_float2(p1, p2);
             }
         }
+        // paired products feed scalar sums (bilinear sample); scalar products feed paired sums (Jres): never both paired
+        float2 j0 = f2(0.f), j1 = f2(0.f), j2 = f2(0.f);
 #pragma unroll
         for (int k = 0; k < 4; ++k) {
-            const float s = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(wTL, pl[k]), __fmul_rn(wTR, pr[k])), __fmul_rn(wBL, pl[k + 1])), __fmul_rn(wBR, pr[k + 1]));   // ref: :386
-            const float res = __fadd_rn(__fsub_rn(s, rref[k]), mean_diff);                                                                              // ref: :387
-            j0 = __fsub_rn(j0, __fmul_rn(res, rdx[k]));
-            j1 = __fsub_rn(j1, __fmul_rn(res, rdy[k]));
-            j2 = __fsub_rn(j2, res);
+            const float2 a0 = __fmul2_rn(f2(wTL), tl[k]), a1 = __fmul2_rn(f2(wTR), tr[k]);
+            const float2 a2 = __fmul2_rn(f2(wBL), tl[k + 1]), a3 = __fmul2_rn(f2(wBR), tr[k + 1]);
+            const float2 s = make_float2(__fadd_rn(__fadd_rn(__fadd_rn(a0.x, a1.x), a2.x), a3.x),
+                                         __fadd_rn(__fadd_rn(__fadd_rn(a0.y, a1.y), a2.y), a3.y));          // ref: :386
+            const float2 res = __fadd2_rn(__fadd2_rn(s, nref[k]), f2(mean_diff));                          // ref: :387
+            j0 = __fadd2_rn(j0, make_float2(__fmul_rn(res.x, ndx[k].x), __fmul_rn(res.y, ndx[k].y)));
+            j1 = __fadd2_rn(j1, make_float2(__fmul_rn(res.x, ndy[k].x), __fmul_rn(res.y, ndy[k].y)));
+            j2 = make_float2(__fsub_rn(j2.x, res.x), __fsub_rn(j2.y, res.y));
         }
-        j0 = hsum(j0); j1 = hsum(j1); j2 = hsum(j2);
+        const float J0 = a2d_sum(j0, g), J1 = a2d_sum(j1, g), J2 = a2d_sum(j2, g);
         // ref: :395 tUpdate = Hinv * Jres (row-wise, left to right)
-        const float d0 = __fadd_rn(__fadd_rn(__fmul_rn(Hinv[0], j0), __fmul_rn(Hinv[1], j1)), __fmul_rn(Hinv[2], j2));
-        const float d1 = __fadd_rn(__fadd_rn(__fmul_rn(Hinv[3], j0), __fmul_rn(Hinv[4], j1)), __fmul_rn(Hinv[5], j2));
-        const float d2 = __fadd_rn(__fadd_rn(__fmul_rn(Hinv[6], j0), __fmul_rn(Hinv[7], j1)), __fmul_rn(Hinv[8], j2));
+        const float d0 = __fadd_rn(__fadd_rn(__fmul_rn(Hinv[0], J0), __fmul_rn(Hinv[1], J1)), __fmul_rn(Hinv[2], J2));
+        const float d1 = __fadd_rn(__fadd_rn(__fmul_rn(Hinv[3], J0), __fmul_rn(Hinv[4], J1)), __fmul_rn(Hinv[5], J2));
+        const float d2 = __fadd_rn(__fadd_rn(__fmul_rn(Hinv[6], J0), __fmul_rn(Hinv[7], J1)), __fmul_rn(Hinv[8], J2));
         if (active) {
             u = __fadd_rn(u, d0); v = __fadd_rn(v, d1); mean_diff = __fadd_rn(mean_diff, d2);
             if (__fadd_rn(__fmul_rn(d0, d0), __fmul_rn(d1, d1)) < min_update_squared) { converged = true; active = false; }   // ref: :400
         }
     }
-    if (exists && L >= 0 && l16 == 0) {
+    if (exists && L >= 0 && l8 == 0) {
         a.px[2 * i] = (double)u; a.px[2 * i + 1] = (double)v;     // ref: :414
         a.conv[i] = converged ? 1 : 0;
         if (a.store_out) {
@@ -311,7 +334,7 @@ cudaError_t launch_align2d(dsdtm_ctx* c, int n_patches, int max_iters, cudaStrea
     a.frames = c->frames_d; a.frame_stride = c->geo.frame_stride; a.geo = c->geo;
     a.patch_slot = c->patch_slot_d; a.patch_level = c->patch_level_d; a.patch10 = c->patches_d;
     a.px_in = c->patch_px_in_d; a.px = c->patch_px_d; a.conv = c->patch_conv_d; a.n = n_patches; a.max_iters = max_iters; a.patch0 = patch0;
-    align2d_kernel<<<(n_patches + 2 * A2D_WARPS - 1) / (2 * A2D_WARPS), A2D_WARPS * 32, 0, s>>>(a);
+    align2d_kernel<<<(n_patches + A2D_PPW * A2D_WARPS - 1) / (A2D_PPW * A2D_WARPS), A2D_WARPS * 32, 0, s>>>(a);
     c->launches++;
     return cudaGetLastError();
 }
