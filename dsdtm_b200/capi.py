@@ -38,6 +38,8 @@ BA_MAX_OBS = 4096
 MATCH_DT = np.dtype([("point", "<i4"), ("px", "<f4", 2), ("level", "<i4")])
 assert MATCH_DT.itemsize == 16
 TRACK_MAX_MATCHES = 200
+CIRCLE_DT = np.dtype([("px", "<f4", 2), ("radius", "<i4"), ("reserved", "<i4")])
+assert CIRCLE_DT.itemsize == 16
 # dsdtm_batch_run flags: 1 = rebuild the cur pyramids, 2 = the refinement chain (batch_stage_map), 4 (with 2) = SearchLocalPoints'
 # selection + PoseOptimization behind it (batch_stage_track): flags 7 ends in the tracked pose of every pair
 RUN_PYRAMID, RUN_CHAIN, RUN_TRACK = 1, 2, 4
@@ -84,7 +86,7 @@ SYMBOLS = [
     "dsdtm_local_map_align_batch", "dsdtm_depth_upload", "dsdtm_depth_convert_f32", "dsdtm_keyframe_lift",
     "dsdtm_frame_upload_pyramid_host", "dsdtm_frames_upload_clahe_pyramid", "dsdtm_track_frame",
     "dsdtm_pose_optimize", "dsdtm_pose_optimize_batch", "dsdtm_map_table_upload", "dsdtm_close_keyframes", "dsdtm_probe_fp64", "dsdtm_frame_upload_pyramid_async", "dsdtm_track_frame_store", "dsdtm_store_set_points", "dsdtm_store_update_points", "dsdtm_store_append_keyframe", "dsdtm_store_set_keyframe", "dsdtm_store_clear", "dsdtm_store_track", "dsdtm_frame_upload_level", "dsdtm_batch_stage_map", "dsdtm_batch_fetch_map", "dsdtm_track_batch_e2e",
-    "dsdtm_batch_stage_track", "dsdtm_batch_fetch_track",
+    "dsdtm_batch_stage_track", "dsdtm_batch_fetch_track", "dsdtm_detect", "dsdtm_detect_batch",
 ]
 
 
@@ -264,6 +266,39 @@ class Context:
         occ = np.ascontiguousarray(occupied, np.uint8) if occupied is not None else None
         self._ck(self.L.dsdtm_fast_cells_batch(self.hp, int(slot), int(n), int(barrier), C.c_float(seed_score), _p(occ), _p(cells)))
         return cells if n == 1 else cells.reshape(n, self.n_cells)
+
+    def detect(self, slot, threshold=5.0, occupied=None, mask=None, circles=None, max_new=300, n=1):
+        """Feature_detector::detect for the n slots slot..slot+n-1 (dsdtm_detect for n == 1, dsdtm_detect_batch otherwise).
+        occupied: (n, n_cells) or None; mask: (n, h, w) uint8 or None; circles: one CIRCLE_DT array per frame (a list) or, for
+        n == 1, one array; max_new: an int or one per frame. Returns (list of CORNER_DT arrays in Add_Feature order, exact-path
+        flags (n,) bool)."""
+        mn = np.broadcast_to(np.asarray(max_new, np.int32), (n,)).copy()
+        occ = None if occupied is None else np.ascontiguousarray(occupied, np.uint8).reshape(n, self.n_cells)
+        msk = None if mask is None else np.ascontiguousarray(mask, np.uint8).reshape(n, self.height, self.width)
+        if circles is not None and n == 1 and not isinstance(circles, (list, tuple)):
+            circles = [circles]
+        exact = np.zeros(n, np.uint8)
+        if n == 1:
+            c = None if circles is None else np.ascontiguousarray(circles[0], CIRCLE_DT)
+            out = np.zeros(max(int(mn[0]), 1), CORNER_DT)
+            n_out = C.c_int(0)
+            self._ck(self.L.dsdtm_detect(self.hp, int(slot), C.c_float(threshold), _p(occ), _p(msk), _p(c), 0 if c is None else len(c),
+                                         int(mn[0]), _p(out), C.byref(n_out), _p(exact)))
+            return [out[:n_out.value].copy()], exact.astype(bool)
+        stride = max(int(mn.max()), 1)
+        out = np.zeros((n, stride), CORNER_DT)
+        n_out = np.zeros(n, np.int32)
+        circ = nc = None
+        cs = 0
+        if circles is not None:
+            nc = np.array([len(c) for c in circles], np.int32)
+            cs = max(int(nc.max()), 1)
+            circ = np.zeros((n, cs), CIRCLE_DT)
+            for i, c in enumerate(circles):
+                circ[i, :len(c)] = c
+        self._ck(self.L.dsdtm_detect_batch(self.hp, int(slot), int(n), C.c_float(threshold), _p(occ), _p(msk), _p(circ), cs, _p(nc),
+                                           _p(mn), stride, _p(out), _p(n_out), _p(exact)))
+        return [out[i, :n_out[i]].copy() for i in range(n)], exact.astype(bool)
 
     def fast_score_map(self, slot, level, barrier=20):
         s = np.empty((self.hs[level], self.ws[level]), np.uint8)

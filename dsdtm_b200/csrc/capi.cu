@@ -311,7 +311,8 @@ void dsdtm_destroy(dsdtm_ctx* c)
                      c->po_obs_d, c->po_res_d, c->po_nobs_d, c->po_pose_in_d, c->po_pose_out_d, c->po_sum_d,
                      c->mt_kfs_d, c->mt_pts_d, c->mt_vis_d, c->mt_dist_d,
                      c->st_kfs_d, c->st_feats_d, c->st_pts_d, c->st_claim_d, c->st_vis_d, c->st_dist_d, c->st_sel_d, c->st_out_d,
-                     c->trk_found_d, c->trk_match_d, c->trk_obs_d, c->trk_nobs_d, c->trk_pose_in_d, c->trk_pose_out_d, c->trk_res_d, c->trk_sum_d };
+                     c->trk_found_d, c->trk_match_d, c->trk_obs_d, c->trk_nobs_d, c->trk_pose_in_d, c->trk_pose_out_d, c->trk_res_d, c->trk_sum_d,
+                     c->det_mask_d, c->det_buf_d };
     for (void* p : bufs) if (p) cudaFree(p);
     if (c->pinned) cudaFreeHost(c->pinned);
     if (c->stage_pin) cudaFreeHost(c->stage_pin);
@@ -570,6 +571,119 @@ int dsdtm_fast_score_map(dsdtm_ctx* c, int slot, int level, int barrier, uint8_t
     DSDTM_CUDA(c, cudaMemcpyAsync(score, c->scoremap_d, n, cudaMemcpyDeviceToHost, c->stream));
     DSDTM_CUDA(c, cudaMemcpyAsync(nonmax, c->scoremap_d + n0, n, cudaMemcpyDeviceToHost, c->stream));
     DSDTM_CUDA(c, cudaStreamSynchronize(c->stream));
+    return 0;
+}
+
+// ------------------------------------------------------------------------------------------------ detect (FAST + sort + mask-circle selection)
+static int check_detect(dsdtm_ctx* c, int first_slot, int n, float thr, const dsdtm_circle* circles, int circle_stride, const int* n_circles,
+                        const int* max_new, int out_stride, const dsdtm_corner* out, const int* n_out)
+{
+    if (!out || !n_out || !max_new || n < 0 || out_stride < 0 || !(thr >= 0.f)) return fail(c, DSDTM_E_ARG, "bad detect argument");
+    if (check_slot(c, first_slot, n)) return DSDTM_E_ARG;
+    if (n > c->prm.max_batch) return fail(c, DSDTM_E_ARG, "n > max_batch");
+    int max_smem = 0;
+    DSDTM_CUDA(c, cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, c->device));
+    if (!detect_select_fits(c, (size_t)max_smem))
+        return fail(c, DSDTM_E_ARG, "detect: frame geometry beyond the selection bitmap (752 x 480 pixels, CellSize <= 64)");
+    for (int i = 0; i < n; ++i)
+        if (max_new[i] > out_stride) return fail(c, DSDTM_E_ARG, "detect: max_new > out_stride");
+    if (circles) {
+        if (!n_circles || circle_stride < 0) return fail(c, DSDTM_E_ARG, "detect: circles without n_circles / circle_stride");
+        for (int i = 0; i < n; ++i) {
+            if (n_circles[i] < 0 || n_circles[i] > circle_stride) return fail(c, DSDTM_E_ARG, "detect: n_circles out of range (circle_stride)");
+            for (int q = 0; q < n_circles[i]; ++q) {
+                const int r = circles[(size_t)i * circle_stride + q].radius;
+                if (r < 0 || r > detect_select_max_radius()) return fail(c, DSDTM_E_ARG, "detect: circle radius out of range (0..64)");
+            }
+        }
+    }
+    return 0;
+}
+
+static int detect_submit(dsdtm_ctx* c, int first_slot, int n, float thr, bool use_occupied, const uint8_t* masks_d, const dsdtm_circle* circles_d,
+                         int circle_stride, const int* n_circles_d, const int* max_new_d, dsdtm_corner* out_d, int out_stride, int* n_out_d,
+                         uint8_t* exact_d)
+{
+    stage_begin(c, DSDTM_STAGE_FAST);
+    DSDTM_CUDA(c, launch_fast_cells(c, first_slot, n, 20, thr, use_occupied, c->stream));           // ref: :81-82 barrier literal 20
+    DSDTM_CUDA(c, launch_detect_select(c, n, thr, masks_d, circles_d, circle_stride, n_circles_d, max_new_d, out_d, out_stride, n_out_d,
+                                       exact_d, c->stream));
+    stage_end(c, 2);
+    return 0;
+}
+
+int dsdtm_detect_batch(dsdtm_ctx* c, int first_slot, int n, float thr, const uint8_t* occupied, const uint8_t* masks, const dsdtm_circle* circles,
+                       int circle_stride, const int* n_circles, const int* max_new, int out_stride, dsdtm_corner* out, int* n_out,
+                       uint8_t* exact_path)
+{
+    if (!c) return DSDTM_E_ARG;
+    if (int e = check_detect(c, first_slot, n, thr, circles, circle_stride, n_circles, max_new, out_stride, out, n_out)) return e;
+    if (n == 0) return 0;
+    auto pad = [](size_t b) { return (b + 15) & ~(size_t)15; };
+    const size_t cs = circles ? (size_t)circle_stride : 0;
+    // det_buf_d / pinned: max_new | n_circles | circles || n_out | exact | corners
+    const size_t o_ncirc = pad(n * sizeof(int)), o_circ = o_ncirc + pad(n * sizeof(int)), in_b = o_circ + pad(n * cs * sizeof(dsdtm_circle));
+    const size_t o_exact = in_b + pad(n * sizeof(int)), o_out = o_exact + pad(n), total = o_out + pad((size_t)n * out_stride * sizeof(dsdtm_corner));
+    const size_t frame_px = (size_t)c->geo.w[0] * c->geo.h[0];
+    if (grow(c, &c->det_buf_d, &c->det_buf_cap, total) || ensure_pinned(c, total)) return DSDTM_E_NOMEM;
+    if (masks && grow(c, &c->det_mask_d, &c->det_mask_cap, n * frame_px)) return DSDTM_E_NOMEM;
+    uint8_t* P = c->pinned;
+    std::memcpy(P, max_new, n * sizeof(int));
+    if (circles) {
+        std::memcpy(P + o_ncirc, n_circles, n * sizeof(int));
+        std::memcpy(P + o_circ, circles, n * cs * sizeof(dsdtm_circle));
+    }
+    if (occupied) DSDTM_CUDA(c, cudaMemcpyAsync(c->occupied_d, occupied, (size_t)n * c->n_cells, cudaMemcpyHostToDevice, c->stream));
+    if (masks) DSDTM_CUDA(c, cudaMemcpyAsync(c->det_mask_d, masks, n * frame_px, cudaMemcpyHostToDevice, c->stream));
+    DSDTM_CUDA(c, cudaMemcpyAsync(c->det_buf_d, P, in_b, cudaMemcpyHostToDevice, c->stream));
+    uint8_t* B = c->det_buf_d;
+    if (detect_submit(c, first_slot, n, thr, occupied != nullptr, masks ? c->det_mask_d : nullptr,
+                      circles ? reinterpret_cast<const dsdtm_circle*>(B + o_circ) : nullptr, (int)cs,
+                      circles ? reinterpret_cast<const int*>(B + o_ncirc) : nullptr, reinterpret_cast<const int*>(B), reinterpret_cast<dsdtm_corner*>(B + o_out),
+                      out_stride, reinterpret_cast<int*>(B + in_b), B + o_exact))
+        return DSDTM_E_CUDA;
+    DSDTM_CUDA(c, cudaMemcpyAsync(P + in_b, B + in_b, total - in_b, cudaMemcpyDeviceToHost, c->stream));
+    DSDTM_CUDA(c, cudaStreamSynchronize(c->stream));
+    std::memcpy(n_out, P + in_b, n * sizeof(int));
+    if (exact_path) std::memcpy(exact_path, P + o_exact, n);
+    const dsdtm_corner* R = reinterpret_cast<const dsdtm_corner*>(P + o_out);
+    for (int i = 0; i < n; ++i) std::memcpy(out + (size_t)i * out_stride, R + (size_t)i * out_stride, n_out[i] * sizeof(dsdtm_corner));
+    return 0;
+}
+
+int dsdtm_detect(dsdtm_ctx* c, int slot, float thr, const uint8_t* occupied, const uint8_t* mask, const dsdtm_circle* circles, int n_circles,
+                 int max_new, dsdtm_corner* out, int* n_out, uint8_t* exact_path)
+{
+    if (!c) return DSDTM_E_ARG;
+    if (n_circles < 0 || (n_circles > 0 && !circles)) return fail(c, DSDTM_E_ARG, "detect: n_circles < 0 or circles NULL");
+    const int nc = circles ? n_circles : 0, stride = std::max(max_new, 0);
+    if (int e = check_detect(c, slot, 1, thr, circles, nc, &nc, &max_new, stride, out, n_out)) return e;
+    const size_t frame_px = (size_t)c->geo.w[0] * c->geo.h[0];
+    const size_t in_b = (occupied ? c->n_cells : 0) + (mask ? frame_px : 0) + 2 * sizeof(int) + nc * sizeof(dsdtm_circle);
+    const size_t out_b = sizeof(int) + 1 + (size_t)stride * sizeof(dsdtm_corner);
+    Arena ar(c, in_b, out_b, 5, 3);
+    if (!ar.active)
+        return dsdtm_detect_batch(c, slot, 1, thr, occupied, mask, circles, nc, &nc, &max_new, stride, out, n_out, exact_path);
+    uint8_t* occ_d = occupied ? ar.in(occupied, c->n_cells) : nullptr;
+    const uint8_t* mask_d = mask ? ar.in(mask, frame_px) : nullptr;
+    const int* max_new_d = ar.in(&max_new, 1);
+    const int* nc_d = ar.in(&nc, 1);
+    const dsdtm_circle* circ_d = nc ? ar.in(circles, nc) : nullptr;
+    uint8_t exact = 0;
+    int* n_out_d = ar.out(n_out, 1);
+    uint8_t* exact_d = ar.out(&exact, 1);
+    dsdtm_corner* out_d = ar.out(static_cast<dsdtm_corner*>(nullptr), std::max(stride, 1));
+    DSDTM_CUDA(c, ar.upload(c->stream));
+    {
+        PtrSwap<uint8_t> sw(c->occupied_d, occ_d ? occ_d : c->occupied_d);
+        if (detect_submit(c, slot, 1, thr, occ_d != nullptr, mask_d, circ_d, nc, circ_d ? nc_d : nullptr, max_new_d, out_d, stride, n_out_d, exact_d))
+            return DSDTM_E_CUDA;
+    }
+    DSDTM_CUDA(c, ar.download(c->stream));
+    DSDTM_CUDA(c, cudaStreamSynchronize(c->stream));
+    ar.finish();
+    std::memcpy(out, ar.host_view(out_d), *n_out * sizeof(dsdtm_corner));
+    if (exact_path) *exact_path = exact;
     return 0;
 }
 

@@ -145,6 +145,9 @@ struct dsdtm_ctx {
     double* trk_pose_out_d = nullptr;            // max_batch * 7: after PoseOptimization
     double* trk_res_d = nullptr;                 // max_batch * DSDTM_TRACK_MAX_MATCHES
     dsdtm_ba_summary* trk_sum_d = nullptr;       // max_batch
+    // key-frame detection (dsdtm_detect_batch), grown on demand
+    uint8_t* det_mask_d = nullptr;       size_t det_mask_cap = 0;    // n * w*h mask images: allocated by the first call that passes masks
+    uint8_t* det_buf_d = nullptr;        size_t det_buf_cap = 0;     // small inputs (max_new, n_circles, circles) | outputs, one copy each way
 
     // pinned host staging for small synchronous calls
     uint8_t* pinned = nullptr;
@@ -238,6 +241,12 @@ cudaError_t launch_pose_opt_io(dsdtm_ctx* c, const PoseOptIo& io, int n_frames, 
 // SearchLocalPoints' selection over the batched chain's records + the PoseOptimization inputs of every pair (select.cu)
 cudaError_t launch_track_select(dsdtm_ctx* c, int n_pairs, int feat_stride, int ppp, cudaStream_t s);
 int track_select_max_radius();                 // largest Camera.CellSize the selection's circle table holds
+// Feature_detector::detect's sort + mask-circle selection over the cell keys of the last launch_fast_cells (detect_select.cu)
+cudaError_t launch_detect_select(dsdtm_ctx* c, int n, float seed, const uint8_t* masks_d, const dsdtm_circle* circles_d, int circle_stride,
+                                 const int* n_circles_d, const int* max_new_d, dsdtm_corner* out_d, int out_stride, int* n_out_d,
+                                 uint8_t* exact_d, cudaStream_t s);
+bool detect_select_fits(const dsdtm_ctx* c, size_t max_smem);
+int detect_select_max_radius();                // largest dsdtm_circle.radius (and Camera.CellSize) the span table holds
 int sparse_align_smem_bytes(int nf_pad);
 size_t sparse_align_ws_doubles(int max_feats);
 cudaError_t sparse_align_init(dsdtm_ctx* c);

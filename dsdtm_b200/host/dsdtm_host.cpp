@@ -495,40 +495,40 @@ void Feature_detector::detect(Frame* frame, const double detection_threshold, co
     if ((int)frame->mvFeatures.size() >= mMax_fts) return;
     const bool timing = getenv("DSDTM_HOST_TIMING") != nullptr;
     const auto T0 = std::chrono::steady_clock::now();
+    if (frame->mvFeatures.size() > 0) frame->Set_Mask();          // ref: :120-123
+    const auto T1 = std::chrono::steady_clock::now();
     GpuRuntime& rt = GpuRuntime::Instance();
     const int slot = rt.Resident(frame->mGpu);
     const int n = mGrid_rows * mGrid_cols;
     std::vector<uint8_t> occ(n);
     for (int i = 0; i < n; ++i) occ[i] = mvGrid_occupy[i] ? 1 : 0;
-    std::vector<dsdtm_corner> cells(n);
-    // levels loop + FAST + non-max + Shi-Tomasi + per-cell best on the device (ref: :76-109)
-    if (dsdtm_fast_cells(rt.ctx(), slot, 20, (float)detection_threshold, occ.data(), cells.data()) != 0)
-        throw std::runtime_error(std::string("dsdtm_fast_cells: ") + dsdtm_last_error(rt.ctx()));
-    const auto T1 = std::chrono::steady_clock::now();
-    Corners corners;
-    corners.reserve(n);
-    for (int i = 0; i < n; ++i) corners.emplace_back(cells[i].x, cells[i].y, cells[i].score, cells[i].level, 0.0f);
-    std::sort(corners.begin(), corners.end());                    // ref: :111 -- same (unstable) std::sort on the same comparator
-    const auto T2 = std::chrono::steady_clock::now();
-    if (frame->mvFeatures.size() > 0) frame->Set_Mask();          // ref: :120-123
-    const auto T3 = std::chrono::steady_clock::now();
-    for (size_t it = 0; it < corners.size(); ++it) {              // ref: :125-150
-        const Corner c = corners[it];
-        if (c.score > 20) {
-            const Point2f p((float)c.x, (float)c.y);
-            if (frame->mImgMask.at(cvRound(p.y), cvRound(p.x)) == 255) {
-                frame->Add_Feature(new Feature(frame, p, c.level), 0);
-                circle(frame->mImgMask, p, mCell_size, 0);
-            }
+    // mImgMask as Set_Mask and SearchLocalPoints left it (an empty Mat = nothing painted; rows are copied dense if strided)
+    const Mat8& m = frame->mImgMask;
+    std::vector<uint8_t> dense;
+    const uint8_t* mask = nullptr;
+    if (!m.empty()) {
+        mask = m.data;
+        if (m.step != m.cols) {
+            dense.resize((size_t)m.rows * m.cols);
+            for (int y = 0; y < m.rows; ++y) std::memcpy(dense.data() + (size_t)y * m.cols, m.data + (size_t)y * m.step, m.cols);
+            mask = dense.data();
         }
-        if ((int)frame->mvFeatures.size() >= mMax_fts) break;
     }
+    const int max_new = mMax_fts - (int)frame->mvFeatures.size();
+    std::vector<dsdtm_corner> sel(max_new);
+    int n_sel = 0;
+    // levels loop + FAST + non-max + Shi-Tomasi + per-cell best, the unstable std::sort and the mask-circle walk on the device (ref: :76-150)
+    if (dsdtm_detect(rt.ctx(), slot, (float)detection_threshold, occ.data(), mask, nullptr, 0, max_new, sel.data(), &n_sel, nullptr) != 0)
+        throw std::runtime_error(std::string("dsdtm_detect: ") + dsdtm_last_error(rt.ctx()));
+    const auto T2 = std::chrono::steady_clock::now();
+    for (int i = 0; i < n_sel; ++i)                               // ref: :145
+        frame->Add_Feature(new Feature(frame, Point2f((float)sel[i].x, (float)sel[i].y), sel[i].level), 0);
     ResetGrid();
     frame->mImgMask.release();                                    // ref: :152-153
     if (timing) {
-        const auto T4 = std::chrono::steady_clock::now();
+        const auto T3 = std::chrono::steady_clock::now();
         auto us = [](std::chrono::steady_clock::time_point a, std::chrono::steady_clock::time_point b) { return std::chrono::duration<double, std::micro>(b - a).count(); };
-        fprintf(stderr, "detect: fast_cells %.1f us, sort %.1f us, Set_Mask %.1f us, selection %.1f us\n", us(T0, T1), us(T1, T2), us(T2, T3), us(T3, T4));
+        fprintf(stderr, "detect: Set_Mask %.1f us, device detect %.1f us, Add_Feature %.1f us\n", us(T0, T1), us(T1, T2), us(T2, T3));
     }
 }
 

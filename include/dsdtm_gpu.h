@@ -145,7 +145,7 @@ int dsdtm_frame_download_level(dsdtm_ctx* ctx, int slot, int level, uint8_t* out
  * `barrier` (reference literal: 20) on every level, 3x3 non-max on the FAST score, Shi-Tomasi score, per-cell best
  * (strictly greater than seed_score; earliest level, then raster order, wins ties). occupied (grid_rows*grid_cols
  * bytes, may be NULL) = mvGrid_occupy. cells_out[grid_rows*grid_cols] in cell order; empty cells = {0,0,0,seed_score}.
- * Sorting and mask-circle selection (ref: :111-150) stay on the host (dsdtm_b200/host). */
+ * The sort and mask-circle selection that follow (ref: :111-150) are dsdtm_detect / dsdtm_detect_batch below. */
 int dsdtm_fast_cells(dsdtm_ctx* ctx, int slot, int barrier, float seed_score, const uint8_t* occupied,
                      dsdtm_corner* cells_out);
 /* batched over n consecutive slots; occupied (may be NULL) and cells_out are n * grid_rows*grid_cols */
@@ -156,6 +156,36 @@ int dsdtm_fast_cells_batch(dsdtm_ctx* ctx, int first_slot, int n, int barrier, f
  * score[i] = FAST score (>= barrier) if pixel i is a corner else 0; nonmax[i] = 1 if it survives 3x3 non-max. */
 int dsdtm_fast_score_map(dsdtm_ctx* ctx, int slot, int level, int barrier, uint8_t* score, uint8_t* nonmax);
 int dsdtm_grid_dims(const dsdtm_ctx* ctx, int* rows, int* cols);
+
+/* cv::circle(mask, px, radius, 0, -1): a filled circle painted into a detection mask before the selection. The centre is rounded
+ * with cvRound on the device, so callers pass Feature::mpx as it is. 0 <= radius <= 64. */
+typedef struct {
+    float   px[2];
+    int32_t radius;
+    int32_t reserved;
+} dsdtm_circle; /* 16 bytes */
+
+/* replaces all of Feature_detector::detect (ref: src/Feature_detection.cpp:69-154) for the n consecutive slots first_slot..: FAST
+ * with the reference's literal barrier 20 and the per-cell best above detection_threshold (as dsdtm_fast_cells), then the score sort
+ * and the mask-circle selection on the device (detect_select_kernel), then one copy back. Per frame i:
+ *   occupied   (n * grid_rows*grid_cols bytes, may be NULL) = mvGrid_occupy;
+ *   masks      (n * height*width bytes, may be NULL = all 255) = mImgMask after Frame::Set_Mask; a pixel is free iff it is 255;
+ *   circles    (n * circle_stride records, may be NULL) with n_circles[i] <= circle_stride: painted into the mask first;
+ *   max_new[i] = Max_fts - mvFeatures.size(); a value <= 0 selects nothing (the early return of detect);
+ *   out        (n * out_stride corners) receives n_out[i] corners in Add_Feature order; max_new[i] <= out_stride;
+ *   exact_path (n bytes, may be NULL) = 1 where two cells above 20 tied and the frame was ordered by the restatement of libstdc++'s
+ *              std::sort the reference's selection depends on, 0 where the parallel ranking was exact.
+ * The result equals the reference's std::sort + walk bit for bit, including the order of tied scores. The device mask buffer is
+ * allocated by the first call that passes masks. DSDTM_E_ARG (nothing launched) for a slot out of range, n > max_batch,
+ * max_new > out_stride, a radius out of range, NULL out / n_out / max_new, or a frame geometry beyond 752 x 480 pixels. The
+ * device time is counted under DSDTM_STAGE_FAST. */
+int dsdtm_detect_batch(dsdtm_ctx* ctx, int first_slot, int n, float detection_threshold, const uint8_t* occupied, const uint8_t* masks,
+                       const dsdtm_circle* circles, int circle_stride, const int* n_circles, const int* max_new, int out_stride,
+                       dsdtm_corner* out, int* n_out, uint8_t* exact_path);
+/* the same for one slot; inputs travel in one host-to-device copy and outputs in one copy back. circles / mask / occupied may be
+ * NULL. Returns the selected corner count in *n_out. */
+int dsdtm_detect(dsdtm_ctx* ctx, int slot, float detection_threshold, const uint8_t* occupied, const uint8_t* mask,
+                 const dsdtm_circle* circles, int n_circles, int max_new, dsdtm_corner* out, int* n_out, uint8_t* exact_path);
 
 /* ---------------------------------------------------------------- (c) sparse image alignment --------------- */
 /* replaces Sprase_ImgAlign::Run's level loop: GetJocabianMat + GaussNewtonSolver for levels max_level-1 .. min_level
