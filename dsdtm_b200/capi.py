@@ -41,8 +41,9 @@ TRACK_MAX_MATCHES = 200
 CIRCLE_DT = np.dtype([("px", "<f4", 2), ("radius", "<i4"), ("reserved", "<i4")])
 assert CIRCLE_DT.itemsize == 16
 # dsdtm_batch_run flags: 1 = rebuild the cur pyramids, 2 = the refinement chain (batch_stage_map), 4 (with 2) = SearchLocalPoints'
-# selection + PoseOptimization behind it (batch_stage_track): flags 7 ends in the tracked pose of every pair
-RUN_PYRAMID, RUN_CHAIN, RUN_TRACK = 1, 2, 4
+# selection + PoseOptimization behind it (batch_stage_track): flags 7 ends in the tracked pose of every pair; 8 (with 4) = the key frame
+# behind the tracked pose (batch_stage_keyframe): flags 15 ends in the new corners and their lifted records
+RUN_PYRAMID, RUN_CHAIN, RUN_TRACK, RUN_KEYFRAME = 1, 2, 4, 8
 
 
 class Cam(C.Structure):
@@ -87,6 +88,7 @@ SYMBOLS = [
     "dsdtm_frame_upload_pyramid_host", "dsdtm_frames_upload_clahe_pyramid", "dsdtm_track_frame",
     "dsdtm_pose_optimize", "dsdtm_pose_optimize_batch", "dsdtm_map_table_upload", "dsdtm_close_keyframes", "dsdtm_probe_fp64", "dsdtm_frame_upload_pyramid_async", "dsdtm_track_frame_store", "dsdtm_store_set_points", "dsdtm_store_update_points", "dsdtm_store_append_keyframe", "dsdtm_store_set_keyframe", "dsdtm_store_clear", "dsdtm_store_track", "dsdtm_frame_upload_level", "dsdtm_batch_stage_map", "dsdtm_batch_fetch_map", "dsdtm_track_batch_e2e",
     "dsdtm_batch_stage_track", "dsdtm_batch_fetch_track", "dsdtm_detect", "dsdtm_detect_batch",
+    "dsdtm_batch_stage_keyframe", "dsdtm_batch_fetch_keyframe",
 ]
 
 
@@ -483,6 +485,24 @@ class Context:
         summ = np.empty(n, BA_SUMMARY_DT)
         self._ck(self.L.dsdtm_batch_fetch_track(self.hp, _p(poses), _p(nm), _p(m), _p(res), _p(summ)))
         return poses, nm, m, res, summ
+
+    def batch_stage_keyframe(self, depth_slots=None, want=None, detection_threshold=5.0, min_dist=15, max_fts=300,
+                             dist=(0.0, 0.0, 0.0, 0.0, 0.0), depth_scale=5000.0):
+        """after batch_stage_track: Tracking::CraeteKeyframe behind the tracked pose. depth_slots = (n_pairs,) depth slots (-1 = no depth;
+        None = none), want = (n_pairs,) bools (None = every pair); batch_run(15) then ends in the key frames"""
+        ds = None if depth_slots is None else np.ascontiguousarray(depth_slots, np.int32).reshape(self._n)
+        wt = None if want is None else np.ascontiguousarray(want, np.uint8).reshape(self._n)
+        self._kf_max_fts = int(max_fts)
+        self._ck(self.L.dsdtm_batch_stage_keyframe(self.hp, _p(ds), _p(wt), C.c_float(detection_threshold), int(min_dist), int(max_fts),
+                                                   _p(np.ascontiguousarray(dist, np.float32)), C.c_float(depth_scale)))
+
+    def batch_fetch_keyframe(self):
+        """-> (n_new (n,), corners (n, max_fts) CORNER_DT, lifted (n, max_fts) LIFTED_DT, exact_path (n,) bool); rows past n_new[i] are
+        zero"""
+        n, F = self._n, self._kf_max_fts
+        nn = np.empty(n, np.int32); cr = np.empty((n, F), CORNER_DT); lf = np.empty((n, F), LIFTED_DT); ex = np.empty(n, np.uint8)
+        self._ck(self.L.dsdtm_batch_fetch_keyframe(self.hp, _p(nn), _p(cr), _p(lf), _p(ex)))
+        return nn, cr, lf, ex.astype(bool)
 
     def track_batch_e2e(self, cur_imgs, ref_slots, cur_slots, feats, feat_stride, n_feats, ref_centers, poses_ref, poses_in, max_level, min_level,
                         max_iters, points_per_pair, max_search_level, align_iters, out):

@@ -189,6 +189,13 @@ static void decode_cells(const dsdtm_ctx* c, const unsigned long long* keys, flo
     }
 }
 
+// every captured step of dsdtm_batch_run: after anything a graph has baked into its launch arguments changes
+static void drop_graphs(dsdtm_ctx* c)
+{
+    for (cudaGraphExec_t& g : c->batch.graph)
+        if (g) { cudaGraphExecDestroy(g); g = nullptr; }
+}
+
 static int check_slot(dsdtm_ctx* c, int slot, int n = 1)
 {
     if (slot < 0 || n < 0 || slot + n > c->prm.max_frames) return fail(c, DSDTM_E_ARG, "frame slot out of range");
@@ -302,7 +309,7 @@ void dsdtm_destroy(dsdtm_ctx* c)
     if (!c) return;
     cudaSetDevice(c->device);
     if (c->stream) cudaStreamSynchronize(c->stream);
-    for (int k = 0; k < 8; ++k) if (c->batch.graph[k]) cudaGraphExecDestroy(c->batch.graph[k]);
+    for (cudaGraphExec_t g : c->batch.graph) if (g) cudaGraphExecDestroy(g);
     void* bufs[] = { c->frames_d, c->cells_d, c->occupied_d, c->scoremap_d, c->fast_tiles_d, c->ref_slots_d, c->cur_slots_d,
                      c->feats_d, c->n_feats_d, c->centers_d, c->poses_in_d, c->poses_out_d, c->n_tracked_d, c->log_d, c->n_log_d,
                      c->patches_d, c->patch_px_d, c->patch_px_in_d, c->patch_level_d, c->patch_slot_d, c->patch_conv_d, c->wa_A_d, c->wa_px_d, c->wa_meta_d, c->sa_ws_d, c->cand_d,
@@ -312,7 +319,8 @@ void dsdtm_destroy(dsdtm_ctx* c)
                      c->mt_kfs_d, c->mt_pts_d, c->mt_vis_d, c->mt_dist_d,
                      c->st_kfs_d, c->st_feats_d, c->st_pts_d, c->st_claim_d, c->st_vis_d, c->st_dist_d, c->st_sel_d, c->st_out_d,
                      c->trk_found_d, c->trk_match_d, c->trk_obs_d, c->trk_nobs_d, c->trk_pose_in_d, c->trk_pose_out_d, c->trk_res_d, c->trk_sum_d,
-                     c->det_mask_d, c->det_buf_d };
+                     c->det_mask_d, c->det_buf_d, c->kf_circ_d, c->kf_ncirc_d, c->kf_max_new_d, c->kf_corner_d, c->kf_lifted_d, c->kf_nnew_d,
+                     c->kf_exact_d, c->kf_depth_slot_d, c->kf_want_d, c->kf_rows_d };
     for (void* p : bufs) if (p) cudaFree(p);
     if (c->pinned) cudaFreeHost(c->pinned);
     if (c->stage_pin) cudaFreeHost(c->stage_pin);
@@ -370,25 +378,25 @@ int dsdtm_set_option(dsdtm_ctx* c, const char* key, int value)
     if (std::strcmp(key, "sa_warps_per_pair") == 0) {
         if (value != 0 && value != 1 && value != 2 && value != 3 && value != 4 && value != 5 && value != 6 && value != 10) return fail(c, DSDTM_E_ARG, "sa_warps_per_pair must be 0, 1, 2, 3, 4, 5, 6 or 10");
         c->sa_wpp_override = value;
-        for (int k = 0; k < 8; ++k) if (c->batch.graph[k]) { cudaGraphExecDestroy(c->batch.graph[k]); c->batch.graph[k] = nullptr; }
+        drop_graphs(c);
         return 0;
     }
     if (std::strcmp(key, "sa_variant") == 0) {
         if (value != 0 && value != 1) return fail(c, DSDTM_E_ARG, "sa_variant must be 0 (shared-memory recompute) or 1 (L2 workspace)");
         c->sa_variant = value;
-        for (int k = 0; k < 8; ++k) if (c->batch.graph[k]) { cudaGraphExecDestroy(c->batch.graph[k]); c->batch.graph[k] = nullptr; }
+        drop_graphs(c);
         return 0;
     }
     if (std::strcmp(key, "step_chunks") == 0) {
         if (value < 1 || value > kMaxStepStreams) return fail(c, DSDTM_E_ARG, "step_chunks must be 1..8");
         c->step_chunks = value;
-        for (int k = 0; k < 8; ++k) if (c->batch.graph[k]) { cudaGraphExecDestroy(c->batch.graph[k]); c->batch.graph[k] = nullptr; }
+        drop_graphs(c);
         return 0;
     }
     if (std::strcmp(key, "pyramid_kernel") == 0) {
         if (value != 0 && value != 1 && value != 2) return fail(c, DSDTM_E_ARG, "pyramid_kernel must be 0 (auto: bulk-staged where eligible), 1 (tile) or 2 (register strip)");
         c->pyr_kernel = value;
-        for (int k = 0; k < 8; ++k) if (c->batch.graph[k]) { cudaGraphExecDestroy(c->batch.graph[k]); c->batch.graph[k] = nullptr; }
+        drop_graphs(c);
         return 0;
     }
     if (std::strcmp(key, "pose_opt_solo_max") == 0) {
@@ -1613,7 +1621,7 @@ int dsdtm_batch_stage(dsdtm_ctx* c, int n_pairs, const int* ref_slots, const int
     auto& b = c->batch;
     b.staged = true; b.n_pairs = n_pairs; b.feat_stride = feat_stride; b.max_level = max_level; b.min_level = min_level;
     b.max_iters = max_iters; b.patches_per_pair = ppp; b.align_iters = align_iters;
-    b.map_staged = false; b.track_staged = false;
+    b.map_staged = false; b.track_staged = false; b.kf_staged = false;
     return 0;
 }
 
@@ -1628,8 +1636,8 @@ int dsdtm_batch_stage_map(dsdtm_ctx* c, const double* poses_ref_c2w, int points_
     DSDTM_CUDA(c, cudaMemcpyAsync(c->poses_ref_d, poses_ref_c2w, (size_t)b.n_pairs * 7 * sizeof(double), cudaMemcpyHostToDevice, c->stream));
     DSDTM_CUDA(c, cudaStreamSynchronize(c->stream));
     b.map_staged = true; b.map_ppp = points_per_pair; b.max_search_level = max_search_level; b.map_align_iters = align_iters;
-    b.track_staged = false;
-    for (int k = 0; k < 8; ++k) if (b.graph[k]) { cudaGraphExecDestroy(b.graph[k]); b.graph[k] = nullptr; }
+    b.track_staged = false; b.kf_staged = false;
+    drop_graphs(c);
     return 0;
 }
 
@@ -1658,8 +1666,73 @@ int dsdtm_batch_stage_track(dsdtm_ctx* c, const int32_t* found, int max_iters)
     DSDTM_CUDA(c, cudaMemsetAsync(c->trk_match_d, 0, B * K * sizeof(dsdtm_match), s));
     DSDTM_CUDA(c, cudaMemsetAsync(c->trk_res_d, 0, B * K * sizeof(double), s));
     DSDTM_CUDA(c, cudaStreamSynchronize(s));
-    b.track_staged = true; b.track_iters = max_iters;
-    for (int k = 0; k < 8; ++k) if (b.graph[k]) { cudaGraphExecDestroy(b.graph[k]); b.graph[k] = nullptr; }
+    b.track_staged = true; b.track_iters = max_iters; b.kf_staged = false;
+    drop_graphs(c);
+    return 0;
+}
+
+int dsdtm_batch_stage_keyframe(dsdtm_ctx* c, const int32_t* depth_slots, const uint8_t* want, float detection_threshold, int min_dist, int max_fts,
+                               const float dist[5], float depth_scale)
+{
+    if (!c) return DSDTM_E_ARG;
+    auto& b = c->batch;
+    if (!b.staged || !b.map_staged || !b.track_staged) return fail(c, DSDTM_E_STATE, "dsdtm_batch_stage_keyframe: call dsdtm_batch_stage_track first");
+    if (!dist || !(detection_threshold >= 0.f)) return fail(c, DSDTM_E_ARG, "dsdtm_batch_stage_keyframe: dist NULL or detection_threshold < 0");
+    if (max_fts < 1 || max_fts > DSDTM_MAX_FEATS_LIMIT) return fail(c, DSDTM_E_ARG, "dsdtm_batch_stage_keyframe: max_fts must be 1..DSDTM_MAX_FEATS_LIMIT");
+    if (min_dist < 0 || min_dist > detect_select_max_radius() || c->prm.cell_size > detect_select_max_radius())
+        return fail(c, DSDTM_E_ARG, "dsdtm_batch_stage_keyframe: min_dist / cell_size out of the circle range (0..64)");
+    int max_smem = 0;
+    DSDTM_CUDA(c, cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, c->device));
+    if (!detect_select_fits(c, (size_t)max_smem))
+        return fail(c, DSDTM_E_ARG, "dsdtm_batch_stage_keyframe: frame geometry beyond the selection bitmap (752 x 480 pixels)");
+    const int n = b.n_pairs;
+    std::vector<int32_t> ds(n, -1);
+    std::vector<uint8_t> wt(n, 1);
+    bool any_depth = false;
+    for (int i = 0; i < n; ++i) {
+        if (depth_slots) ds[i] = depth_slots[i];
+        if (want) wt[i] = want[i] ? 1 : 0;
+        if (ds[i] < -1 || ds[i] >= c->depth_slots) return fail(c, DSDTM_E_ARG, "dsdtm_batch_stage_keyframe: depth slot out of range (option depth_slots)");
+        if (ds[i] >= 0 && !c->depth_d) return fail(c, DSDTM_E_ARG, "dsdtm_batch_stage_keyframe: depth slot given before any depth upload");
+        any_depth |= ds[i] >= 0;
+    }
+    if (any_depth && !(depth_scale > 0.f)) return fail(c, DSDTM_E_ARG, "dsdtm_batch_stage_keyframe: depth_scale must be > 0");
+    const size_t B = c->prm.max_batch, K = DSDTM_TRACK_MAX_MATCHES, F = DSDTM_MAX_FEATS_LIMIT;
+    if (!c->kf_circ_d) {
+        // once per context at max_batch size: a captured step keeps pointing at these buffers
+        if (dalloc(c, &c->kf_circ_d, B * 2 * K) || dalloc(c, &c->kf_ncirc_d, B) || dalloc(c, &c->kf_max_new_d, B) || dalloc(c, &c->kf_corner_d, B * F) ||
+            dalloc(c, &c->kf_lifted_d, B * F) || dalloc(c, &c->kf_nnew_d, B) || dalloc(c, &c->kf_exact_d, B) || dalloc(c, &c->kf_depth_slot_d, B) ||
+            dalloc(c, &c->kf_want_d, B) || dalloc(c, &c->kf_rows_d, B))
+            return DSDTM_E_NOMEM;
+    }
+    std::vector<int32_t> rows;
+    for (int i = 0; i < n; ++i) if (wt[i]) rows.push_back(i);
+    cudaStream_t s = c->stream;
+    DSDTM_CUDA(c, cudaMemcpyAsync(c->kf_depth_slot_d, ds.data(), n * sizeof(int32_t), cudaMemcpyHostToDevice, s));
+    DSDTM_CUDA(c, cudaMemcpyAsync(c->kf_want_d, wt.data(), n, cudaMemcpyHostToDevice, s));
+    if (!rows.empty()) DSDTM_CUDA(c, cudaMemcpyAsync(c->kf_rows_d, rows.data(), rows.size() * sizeof(int32_t), cudaMemcpyHostToDevice, s));
+    DSDTM_CUDA(c, cudaStreamSynchronize(s));
+    b.kf_staged = true; b.kf_min_dist = min_dist; b.kf_max_fts = max_fts; b.kf_thr = detection_threshold; b.kf_n_wanted = (int)rows.size();
+    for (int k = 0; k < 5; ++k) b.kf_dist[k] = dist[k];
+    b.kf_depth_scale = any_depth ? depth_scale : 1.0f;
+    drop_graphs(c);
+    return 0;
+}
+
+// Tracking::CraeteKeyframe behind the tracked pose (dsdtm_batch_run bit 3): occupancy + circles -> FAST on the cur slots -> the sort and
+// mask-circle selection -> the lift of the new corners, on the buffers of dsdtm_batch_stage_keyframe
+static int enqueue_keyframe(dsdtm_ctx* c, cudaStream_t s, bool timed)
+{
+    auto& b = c->batch;
+    if (timed) stage_begin(c, DSDTM_STAGE_FAST);
+    DSDTM_CUDA(c, launch_keyframe_seed(c, b.n_pairs, b.kf_min_dist, b.kf_max_fts, s));
+    DSDTM_CUDA(c, launch_fast_cells_slots(c, c->cur_slots_d, c->kf_rows_d, b.kf_n_wanted, b.kf_thr, s));
+    DSDTM_CUDA(c, launch_detect_select(c, b.n_pairs, b.kf_thr, nullptr, c->kf_circ_d, 2 * DSDTM_TRACK_MAX_MATCHES, c->kf_ncirc_d, c->kf_max_new_d,
+                                       c->kf_corner_d, b.kf_max_fts, c->kf_nnew_d, c->kf_exact_d, s));
+    if (timed) stage_end(c, b.kf_n_wanted ? 3 : 2);
+    if (timed) stage_begin(c, DSDTM_STAGE_INGEST);
+    DSDTM_CUDA(c, launch_keyframe_lift_batch(c, b.n_pairs, b.kf_max_fts, b.kf_dist, b.kf_depth_scale, s));
+    if (timed) stage_end(c, 1);
     return 0;
 }
 
@@ -1720,6 +1793,10 @@ static int enqueue_step(dsdtm_ctx* c, int flags, cudaStream_t s, bool timed)
                 int r = enqueue_track(c, s, timed);
                 if (r) return r;
             }
+            if (flags & 8) {
+                int r = enqueue_keyframe(c, s, timed);
+                if (r) return r;
+            }
         } else if (b.patches_per_pair > 0) {
             if (timed) stage_begin(c, DSDTM_STAGE_ALIGN2D);
             DSDTM_CUDA(c, launch_align2d(c, b.n_pairs * b.patches_per_pair, b.align_iters, s));
@@ -1756,7 +1833,9 @@ int dsdtm_batch_run(dsdtm_ctx* c, int flags)
     if ((flags & 2) && !b.map_staged) return fail(c, DSDTM_E_STATE, "dsdtm_batch_run: flags bit 1 needs dsdtm_batch_stage_map");
     if ((flags & 4) && !(flags & 2)) return fail(c, DSDTM_E_STATE, "dsdtm_batch_run: flags bit 2 needs bit 1 (the refinement chain)");
     if ((flags & 4) && !b.track_staged) return fail(c, DSDTM_E_STATE, "dsdtm_batch_run: flags bit 2 needs dsdtm_batch_stage_track");
-    const int gi = flags & 7;
+    if ((flags & 8) && !(flags & 4)) return fail(c, DSDTM_E_STATE, "dsdtm_batch_run: flags bit 3 needs bit 2 (the tracked pose)");
+    if ((flags & 8) && !b.kf_staged) return fail(c, DSDTM_E_STATE, "dsdtm_batch_run: flags bit 3 needs dsdtm_batch_stage_keyframe");
+    const int gi = flags & 15;
     DSDTM_CUDA(c, cudaEventRecord(c->ev_a, c->stream));
     if (c->profiling) {
         // per-stage events cannot be recorded inside a captured graph: launch directly
@@ -1784,7 +1863,7 @@ int dsdtm_batch_run(dsdtm_ctx* c, int flags)
         DSDTM_CUDA(c, cudaGraphLaunch(b.graph[gi], c->stream));
         {
             const int chunks = (c->step_chunks <= 1 || b.n_pairs < 4 * c->sm_count) ? 1 : std::min(c->step_chunks, kMaxStepStreams);
-            if (flags & 2) c->launches += ((flags & 1) ? c->geo.levels - 1 : 0) + 1 + 5 + ((flags & 4) ? 2 : 0);
+            if (flags & 2) c->launches += ((flags & 1) ? c->geo.levels - 1 : 0) + 1 + 5 + ((flags & 4) ? 2 : 0) + ((flags & 8) ? (b.kf_n_wanted ? 4 : 3) : 0);
             else c->launches += ((flags & 1) ? c->geo.levels - 1 : 0) + (long long)chunks * (1 + (b.patches_per_pair > 0 ? 1 : 0));
         }
     }
@@ -1833,6 +1912,31 @@ int dsdtm_batch_fetch_track(dsdtm_ctx* c, double* poses_c2w_out, int32_t* n_matc
     if (res_norm) DSDTM_CUDA(c, cudaMemcpyAsync(res_norm, c->trk_res_d, n * K * sizeof(double), cudaMemcpyDeviceToHost, s));
     if (summaries) DSDTM_CUDA(c, cudaMemcpyAsync(summaries, c->trk_sum_d, n * sizeof(dsdtm_ba_summary), cudaMemcpyDeviceToHost, s));
     DSDTM_CUDA(c, cudaStreamSynchronize(s));
+    float ms = 0.f;
+    if (cudaEventElapsedTime(&ms, c->ev_a, c->ev_b) == cudaSuccess) c->last_run_ms = ms;
+    return 0;
+}
+
+int dsdtm_batch_fetch_keyframe(dsdtm_ctx* c, int32_t* n_new, dsdtm_corner* corners, dsdtm_lifted* lifted, uint8_t* exact_path)
+{
+    if (!c) return DSDTM_E_ARG;
+    auto& b = c->batch;
+    if (!b.staged || !b.map_staged || !b.track_staged || !b.kf_staged) return fail(c, DSDTM_E_STATE, "dsdtm_batch_fetch_keyframe: no staged key-frame batch");
+    cudaStream_t s = c->stream;
+    const size_t n = (size_t)b.n_pairs, F = (size_t)b.kf_max_fts;
+    std::vector<int32_t> nn(n);
+    DSDTM_CUDA(c, cudaMemcpyAsync(nn.data(), c->kf_nnew_d, n * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+    if (corners) DSDTM_CUDA(c, cudaMemcpyAsync(corners, c->kf_corner_d, n * F * sizeof(dsdtm_corner), cudaMemcpyDeviceToHost, s));
+    if (lifted) DSDTM_CUDA(c, cudaMemcpyAsync(lifted, c->kf_lifted_d, n * F * sizeof(dsdtm_lifted), cudaMemcpyDeviceToHost, s));
+    if (exact_path) DSDTM_CUDA(c, cudaMemcpyAsync(exact_path, c->kf_exact_d, n, cudaMemcpyDeviceToHost, s));
+    DSDTM_CUDA(c, cudaStreamSynchronize(s));
+    // the step writes rows < n_new[i] only: what lies past them is left from earlier replays and is cleared here
+    for (size_t i = 0; i < n; ++i) {
+        const size_t k = (size_t)std::max(nn[i], 0);
+        if (corners) std::memset(corners + i * F + k, 0, (F - k) * sizeof(dsdtm_corner));
+        if (lifted) std::memset(lifted + i * F + k, 0, (F - k) * sizeof(dsdtm_lifted));
+    }
+    if (n_new) std::memcpy(n_new, nn.data(), n * sizeof(int32_t));
     float ms = 0.f;
     if (cudaEventElapsedTime(&ms, c->ev_a, c->ev_b) == cudaSuccess) c->last_run_ms = ms;
     return 0;

@@ -145,6 +145,19 @@ struct dsdtm_ctx {
     double* trk_pose_out_d = nullptr;            // max_batch * 7: after PoseOptimization
     double* trk_res_d = nullptr;                 // max_batch * DSDTM_TRACK_MAX_MATCHES
     dsdtm_ba_summary* trk_sum_d = nullptr;       // max_batch
+    // the key frame behind the tracked pose (dsdtm_batch_stage_keyframe): allocated once per context at max_batch size, like trk_*, because
+    // the replayed step points at them (det_buf_d / det_mask_d are regrown by dsdtm_detect_batch); cells_d / occupied_d are shared and
+    // rewritten by every replay
+    dsdtm_circle* kf_circ_d = nullptr;           // max_batch * 2 * DSDTM_TRACK_MAX_MATCHES: CellSize and Min_dist circles per match
+    int* kf_ncirc_d = nullptr;                   // max_batch
+    int* kf_max_new_d = nullptr;                 // max_batch: Max_fts - n_matches, 0 when not wanted
+    dsdtm_corner* kf_corner_d = nullptr;         // max_batch * DSDTM_MAX_FEATS_LIMIT (row stride: the staged max_fts)
+    dsdtm_lifted* kf_lifted_d = nullptr;         // same indexing
+    int* kf_nnew_d = nullptr;                    // max_batch
+    uint8_t* kf_exact_d = nullptr;               // max_batch
+    int* kf_depth_slot_d = nullptr;              // max_batch, -1 = no depth
+    uint8_t* kf_want_d = nullptr;                // max_batch
+    int* kf_rows_d = nullptr;                    // max_batch: the wanted pairs in index order (the rows of the FAST grid)
     // key-frame detection (dsdtm_detect_batch), grown on demand
     uint8_t* det_mask_d = nullptr;       size_t det_mask_cap = 0;    // n * w*h mask images: allocated by the first call that passes masks
     uint8_t* det_buf_d = nullptr;        size_t det_buf_cap = 0;     // small inputs (max_new, n_circles, circles) | outputs, one copy each way
@@ -164,8 +177,11 @@ struct dsdtm_ctx {
         int map_ppp = 0, max_search_level = 0, map_align_iters = 0;
         bool track_staged = false;                         // dsdtm_batch_stage_track: selection + pose optimization buffers are ready
         int track_iters = 0;
-        cudaGraphExec_t graph[8] = {};                     // [flags & 7]
-        int graph_key[8][8];
+        bool kf_staged = false;                            // dsdtm_batch_stage_keyframe: the key-frame half is ready
+        int kf_min_dist = 0, kf_max_fts = 0, kf_n_wanted = 0;
+        float kf_thr = 0.f, kf_dist[5] = {}, kf_depth_scale = 1.f;
+        cudaGraphExec_t graph[16] = {};                    // [flags & 15]
+        int graph_key[16][8];
     } batch;
 };
 
@@ -246,6 +262,11 @@ cudaError_t launch_detect_select(dsdtm_ctx* c, int n, float seed, const uint8_t*
                                  const int* n_circles_d, const int* max_new_d, dsdtm_corner* out_d, int out_stride, int* n_out_d,
                                  uint8_t* exact_d, cudaStream_t s);
 bool detect_select_fits(const dsdtm_ctx* c, size_t max_smem);
+// the key frame behind the batched chain (keyframe.cu, fast.cu): occupancy + circles + max_new per pair, FAST on the cur slots of the
+// wanted pairs (rows_d: their indices; n = 0 launches nothing), and the lift of the new corners
+cudaError_t launch_keyframe_seed(dsdtm_ctx* c, int n_pairs, int min_dist, int max_fts, cudaStream_t s);
+cudaError_t launch_fast_cells_slots(dsdtm_ctx* c, const int* slots_d, const int* rows_d, int n, float seed_score, cudaStream_t s);
+cudaError_t launch_keyframe_lift_batch(dsdtm_ctx* c, int n_pairs, int stride, const float dist[5], float depth_scale, cudaStream_t s);
 int detect_select_max_radius();                // largest dsdtm_circle.radius (and Camera.CellSize) the span table holds
 int sparse_align_smem_bytes(int nf_pad);
 size_t sparse_align_ws_doubles(int max_feats);

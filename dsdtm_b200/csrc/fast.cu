@@ -68,6 +68,8 @@ __device__ __forceinline__ int max_arc_min10(const int (&v)[16])
 
 struct FastArgs {
     uint8_t* frames; unsigned frame_stride; int first_slot;
+    const int* slots;                    // frame f reads slot slots[f], or first_slot + f when null
+    const int* rows;                     // grid row y runs frame rows[y], or frame y when null
     const int* tiles; int n_tiles; LevelGeom geo;
     int barrier; float seed_score;
     const uint8_t* occupied;             // n * n_cells or null
@@ -121,8 +123,9 @@ __global__ void __launch_bounds__(32 * WARPS) fast_kernel(const FastArgs a)
     const int t = a.tiles[tile];
     const int L = t >> 24, tyi = (t >> 12) & 0xFFF, txi = t & 0xFFF;
     const int w = a.geo.w[L], h = a.geo.h[L];
-    const int frame = blockIdx.y;
-    const uint8_t* __restrict__ img = a.frames + (size_t)(a.first_slot + frame) * a.frame_stride + a.geo.off[L];
+    const int frame = a.rows ? a.rows[blockIdx.y] : (int)blockIdx.y;
+    const int slot = a.slots ? a.slots[frame] : a.first_slot + frame;
+    const uint8_t* __restrict__ img = a.frames + (size_t)slot * a.frame_stride + a.geo.off[L];
     const int x0 = txi * FT_W, y0 = tyi * FT_H;
 
     // ---- stage the halo tile: rows y0-5 .. y0+20, cols [xa, xa+48) with xa = (x0-5) & ~7 (zero outside the image)
@@ -250,6 +253,7 @@ FastArgs make_args(dsdtm_ctx* c, int first_slot)
 {
     FastArgs a;
     a.frames = c->frames_d; a.frame_stride = c->geo.frame_stride; a.first_slot = first_slot;
+    a.slots = nullptr; a.rows = nullptr;
     a.tiles = c->fast_tiles_d; a.n_tiles = c->n_fast_tiles; a.geo = c->geo;
     a.barrier = 20; a.seed_score = 0;
     a.occupied = nullptr; a.cells = c->cells_d; a.n_cells = c->n_cells; a.grid_cols = c->grid_cols; a.cell_size = c->prm.cell_size;
@@ -284,6 +288,22 @@ cudaError_t launch_fast_cells(dsdtm_ctx* c, int first_slot, int n, int barrier, 
     FastArgs a = make_args(c, first_slot);
     a.barrier = barrier; a.seed_score = seed_score;
     a.occupied = use_occupied ? c->occupied_d : nullptr;
+    dim3 grid((c->n_fast_tiles + WARPS - 1) / WARPS, n);
+    fast_kernel<<<grid, 32 * WARPS, 0, s>>>(a);
+    c->launches++;
+    return cudaGetLastError();
+}
+
+// the batched chain's key-frame detection: the n frames rows_d[0..n) (the wanted pairs), frame f on slot slots_d[f]; no memset of the cell
+// keys (keyframe_seed_kernel zeroes the rows of the wanted frames inside the same step). Unwanted pairs get no CTA at all: an early return
+// per CTA for every pair cost 0.48 ms per 4096 kinect pairs on a B200 at 1000 W (DESIGN §3i).
+cudaError_t launch_fast_cells_slots(dsdtm_ctx* c, const int* slots_d, const int* rows_d, int n, float seed_score, cudaStream_t s)
+{
+    if (n == 0) return cudaSuccess;
+    FastArgs a = make_args(c, 0);
+    a.slots = slots_d; a.rows = rows_d;
+    a.seed_score = seed_score;                   // barrier: the reference's literal 20 (ref: src/Feature_detection.cpp:81-82)
+    a.occupied = c->occupied_d;
     dim3 grid((c->n_fast_tiles + WARPS - 1) / WARPS, n);
     fast_kernel<<<grid, 32 * WARPS, 0, s>>>(a);
     c->launches++;

@@ -478,7 +478,8 @@ int dsdtm_track_frame_store(dsdtm_ctx* ctx, const dsdtm_track_store_in* in, dsdt
  * against its cur frame. Inputs are staged once (H2D), run() only launches kernels on HBM-resident data (CUDA-graph
  * replayed), fetch() copies results back. patches: n_pairs * patches_per_pair entries, patch_level < 0 = unused.
  * flags bit0: rebuild the cur pyramids from their level 0 inside run(); bit1: the refinement chain (dsdtm_batch_stage_map);
- * bit2 (with bit1): selection + pose optimization behind it (dsdtm_batch_stage_track). */
+ * bit2 (with bit1): selection + pose optimization behind it (dsdtm_batch_stage_track); bit3 (with bit2): the key frame behind the
+ * tracked pose (dsdtm_batch_stage_keyframe). */
 int dsdtm_batch_stage(dsdtm_ctx* ctx, int n_pairs, const int* ref_slots, const int* cur_slots,
                       const dsdtm_ref_feat* feats, int feat_stride, const int* n_feats, const double* ref_centers,
                       const double* poses_in, int max_level, int min_level, int max_iters,
@@ -523,6 +524,29 @@ int dsdtm_batch_stage_track(dsdtm_ctx* ctx, const int32_t* found, int max_iters)
  * itself; summaries = n_pairs. Every pointer may be NULL. */
 int dsdtm_batch_fetch_track(dsdtm_ctx* ctx, double* poses_c2w_out, int32_t* n_matches, dsdtm_match* matches, double* res_norm,
                             dsdtm_ba_summary* summaries);
+/* Tracking::CraeteKeyframe behind the tracked pose (ref: src/Tracking.cpp:412-464), so that dsdtm_batch_run(flags | 2 | 4 | 8) ends in the
+ * key frame the tracker would create from every wanted pair's cur frame. Per pair, after PoseOptimization:
+ *   occupancy : Set_ExistingFeatures of the matches (ref: src/Feature_detection.cpp:43-50): cell int(px.y / (float)CellSize) * grid_cols
+ *               + int(px.x / (float)CellSize); a cell index outside the grid is skipped (the reference's operator[] is undefined there);
+ *   mask      : filled circles at cvRound of every match's px, radius Camera.CellSize (SearchLocalPoints, ref: src/Feature_alignment.cpp:
+ *               100-113) and radius min_dist = Camera.Min_dist (Frame::Set_Mask, ref: src/Frame.cpp:286-298); no dynamic mask;
+ *   detect    : Feature_detector::detect on the pair's cur slot as dsdtm_detect_batch (literal barrier 20, cells above
+ *               detection_threshold, the literal std::sort order of tied scores) with max_new = max_fts - n_matches (<= 0: nothing);
+ *   lift      : per new corner Frame::UndistortFeatures with dist = {k1,k2,p1,p2,k3}, the bearing, Get_FeatureDetph on depth slot
+ *               depth_slots[i] (-1: none, DSDTM_LIFT_NO_DEPTH; raw depth / depth_scale) and UnProject with the pose after
+ *               PoseOptimization, as dsdtm_keyframe_lift; the matches are mbInitial (SetPose) and are not lifted.
+ * The key frame's mvFeatures are the matches of dsdtm_batch_fetch_track followed by the new corners; a new MapPoint belongs to every
+ * corner whose record is DSDTM_LIFT_OK. NeedKeyframe stays with the caller: want (n_pairs bytes, NULL = all) selects the pairs; FAST
+ * runs on the wanted pairs only, the others get no corners and cost one early exit per CTA of the other three kernels. Requires dsdtm_batch_stage_track (DSDTM_E_STATE otherwise); DSDTM_E_ARG,
+ * with nothing enqueued, for a depth slot >= option depth_slots or < -1, a depth slot before the depth pool exists (dsdtm_depth_upload),
+ * max_fts outside 1..DSDTM_MAX_FEATS_LIMIT, min_dist or cell_size above 64, or a frame geometry dsdtm_detect_batch rejects. Calling
+ * dsdtm_batch_stage, _stage_map or _stage_track again drops this staging. Device time: detection under DSDTM_STAGE_FAST, the lift
+ * under DSDTM_STAGE_INGEST. */
+int dsdtm_batch_stage_keyframe(dsdtm_ctx* ctx, const int32_t* depth_slots /* n_pairs or NULL */, const uint8_t* want /* n_pairs or NULL */,
+                               float detection_threshold, int min_dist, int max_fts, const float dist[5], float depth_scale);
+/* after dsdtm_batch_run(flags | 8): n_new = n_pairs corner counts; corners and lifted = n_pairs x max_fts (Add_Feature order, rows past
+ * n_new[i] zero); exact_path = n_pairs flags as in dsdtm_detect_batch. Every pointer may be NULL. */
+int dsdtm_batch_fetch_keyframe(dsdtm_ctx* ctx, int32_t* n_new, dsdtm_corner* corners, dsdtm_lifted* lifted, uint8_t* exact_path);
 int dsdtm_batch_fetch(dsdtm_ctx* ctx, double* poses_out, int* n_tracked, double* patch_px_out, uint8_t* patch_conv);
 /* end-to-end step with HOST buffers: uploads the n_pairs cur images (dense, pinned recommended) into their cur slots,
  * stages the per-pair inputs, runs, and fetches -- copies overlapped with compute in chunks on internal streams. */
