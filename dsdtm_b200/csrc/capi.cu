@@ -202,6 +202,14 @@ static int check_slot(dsdtm_ctx* c, int slot, int n = 1)
     return 0;
 }
 
+// the pyramid, FAST, CLAHE and key-frame lift kernels take the frame / pair index from gridDim.y or gridDim.z (at most 65535);
+// checked before anything is enqueued, so that a refused call leaves no partial work behind
+static int check_grid_frames(dsdtm_ctx* c, int n)
+{
+    if (n > DSDTM_MAX_BATCH_FRAMES) return fail(c, DSDTM_E_ARG, "more than DSDTM_MAX_BATCH_FRAMES frames or pairs in one batched call");
+    return 0;
+}
+
 }  // namespace dsdtm
 
 using namespace dsdtm;
@@ -402,6 +410,7 @@ int dsdtm_set_option(dsdtm_ctx* c, const char* key, int value)
     if (std::strcmp(key, "pose_opt_solo_max") == 0) {
         if (value < -1) return fail(c, DSDTM_E_ARG, "pose_opt_solo_max must be -1 (default: the SM count), 0 (always one warp per frame) or a frame count");
         c->po_solo_max = value;
+        drop_graphs(c);                          // a captured dsdtm_batch_run step has its PoseOptimization kernel baked in
         return 0;
     }
     if (std::strcmp(key, "depth_slots") == 0) {
@@ -453,7 +462,7 @@ int dsdtm_frame_upload_pyramid(dsdtm_ctx* c, int slot, const uint8_t* img, int s
                                     cudaMemcpyHostToDevice, c->stream));
     stage_begin(c, DSDTM_STAGE_PYRAMID);
     DSDTM_CUDA(c, launch_pyramid(c, slot, 1, c->stream));
-    stage_end(c, g.levels - 1);
+    stage_end(c, pyramid_launches(c));
     DSDTM_CUDA(c, cudaStreamSynchronize(c->stream));
     return 0;
 }
@@ -468,7 +477,7 @@ int dsdtm_frame_upload_pyramid_async(dsdtm_ctx* c, int slot, const uint8_t* img,
                                     cudaMemcpyHostToDevice, c->stream));
     stage_begin(c, DSDTM_STAGE_PYRAMID);
     DSDTM_CUDA(c, launch_pyramid(c, slot, 1, c->stream));
-    stage_end(c, g.levels - 1);
+    stage_end(c, pyramid_launches(c));
     return 0;
 }
 
@@ -483,7 +492,7 @@ int dsdtm_frame_upload_pyramid_host(dsdtm_ctx* c, int slot, const uint8_t* img, 
     DSDTM_CUDA(c, cudaMemcpy2DAsync(c->frames_d + (size_t)slot * g.frame_stride, g.w[0], img, stride, g.w[0], g.h[0], cudaMemcpyHostToDevice, s));
     stage_begin(c, DSDTM_STAGE_PYRAMID);
     DSDTM_CUDA(c, launch_pyramid(c, slot, 1, s));
-    stage_end(c, g.levels - 1);
+    stage_end(c, pyramid_launches(c));
     const size_t tail = levels_out ? (size_t)g.off[g.levels - 1] + (size_t)g.w[g.levels - 1] * g.h[g.levels - 1] - g.off[1] : 0;
     Stager st(c, tail);
     if (levels_out)
@@ -496,7 +505,7 @@ int dsdtm_frame_upload_pyramid_host(dsdtm_ctx* c, int slot, const uint8_t* img, 
 int dsdtm_frames_upload_pyramid(dsdtm_ctx* c, int first_slot, int n, const uint8_t* imgs)
 {
     if (!c || !imgs) return DSDTM_E_ARG;
-    if (check_slot(c, first_slot, n)) return DSDTM_E_ARG;
+    if (check_slot(c, first_slot, n) || check_grid_frames(c, n)) return DSDTM_E_ARG;
     const LevelGeom& g = c->geo;
     const size_t img_bytes = (size_t)g.w[0] * g.h[0];
     // one strided copy: n rows of img_bytes into slots frame_stride apart
@@ -504,7 +513,7 @@ int dsdtm_frames_upload_pyramid(dsdtm_ctx* c, int first_slot, int n, const uint8
                                     cudaMemcpyHostToDevice, c->stream));
     stage_begin(c, DSDTM_STAGE_PYRAMID);
     DSDTM_CUDA(c, launch_pyramid(c, first_slot, n, c->stream));
-    stage_end(c, g.levels - 1);
+    stage_end(c, pyramid_launches(c));
     DSDTM_CUDA(c, cudaStreamSynchronize(c->stream));
     return 0;
 }
@@ -512,10 +521,10 @@ int dsdtm_frames_upload_pyramid(dsdtm_ctx* c, int first_slot, int n, const uint8
 int dsdtm_frames_build_pyramid(dsdtm_ctx* c, int first_slot, int n)
 {
     if (!c) return DSDTM_E_ARG;
-    if (check_slot(c, first_slot, n)) return DSDTM_E_ARG;
+    if (check_slot(c, first_slot, n) || check_grid_frames(c, n)) return DSDTM_E_ARG;
     stage_begin(c, DSDTM_STAGE_PYRAMID);
     DSDTM_CUDA(c, launch_pyramid(c, first_slot, n, c->stream));
-    stage_end(c, c->geo.levels - 1);
+    stage_end(c, pyramid_launches(c));
     return 0;
 }
 
@@ -547,7 +556,7 @@ int dsdtm_fast_cells_batch(dsdtm_ctx* c, int first_slot, int n, int barrier, flo
                            dsdtm_corner* cells_out)
 {
     if (!c || !cells_out || barrier < 1 || barrier > 254 || !(seed_score >= 0.f)) return c ? fail(c, DSDTM_E_ARG, "bad fast_cells argument") : DSDTM_E_ARG;
-    if (check_slot(c, first_slot, n)) return DSDTM_E_ARG;
+    if (check_slot(c, first_slot, n) || check_grid_frames(c, n)) return DSDTM_E_ARG;
     if (n > c->prm.max_batch) return fail(c, DSDTM_E_ARG, "n > max_batch");
     const size_t nc = (size_t)n * c->n_cells;
     if (occupied) DSDTM_CUDA(c, cudaMemcpyAsync(c->occupied_d, occupied, nc, cudaMemcpyHostToDevice, c->stream));
@@ -587,7 +596,7 @@ static int check_detect(dsdtm_ctx* c, int first_slot, int n, float thr, const ds
                         const int* max_new, int out_stride, const dsdtm_corner* out, const int* n_out)
 {
     if (!out || !n_out || !max_new || n < 0 || out_stride < 0 || !(thr >= 0.f)) return fail(c, DSDTM_E_ARG, "bad detect argument");
-    if (check_slot(c, first_slot, n)) return DSDTM_E_ARG;
+    if (check_slot(c, first_slot, n) || check_grid_frames(c, n)) return DSDTM_E_ARG;
     if (n > c->prm.max_batch) return fail(c, DSDTM_E_ARG, "n > max_batch");
     int max_smem = 0;
     DSDTM_CUDA(c, cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, c->device));
@@ -1059,7 +1068,7 @@ int dsdtm_track_frame(dsdtm_ctx* c, const dsdtm_track_in* in, dsdtm_track_out* o
     DSDTM_CUDA(c, ar.upload(s));
     stage_begin(c, DSDTM_STAGE_PYRAMID);
     DSDTM_CUDA(c, launch_pyramid(c, in->cur_slot, 1, s));
-    stage_end(c, g.levels - 1);
+    stage_end(c, pyramid_launches(c));
     stage_begin(c, DSDTM_STAGE_SPARSE_ALIGN);
     DSDTM_CUDA(c, launch_sparse_align(c, 1, nf, in->max_level, in->min_level, in->max_iters, false, s));
     stage_end(c, 1);
@@ -1560,7 +1569,7 @@ int dsdtm_frames_upload_clahe_pyramid(dsdtm_ctx* c, int first_slot, int n, const
 {
     if (!c || !imgs || n < 0) return DSDTM_E_ARG;
     if (n == 0) return 0;
-    if (check_slot(c, first_slot, n)) return DSDTM_E_ARG;
+    if (check_slot(c, first_slot, n) || check_grid_frames(c, n)) return DSDTM_E_ARG;
     const LevelGeom& g = c->geo;
     const int w = g.w[0], h = g.h[0];
     if (tiles_x < 1 || tiles_y < 1 || tiles_x > clahe_max_tiles_x() || w % tiles_x || h % tiles_y)
@@ -1575,7 +1584,7 @@ int dsdtm_frames_upload_clahe_pyramid(dsdtm_ctx* c, int first_slot, int n, const
     stage_end(c, 2);
     stage_begin(c, DSDTM_STAGE_PYRAMID);
     DSDTM_CUDA(c, launch_pyramid(c, first_slot, n, s));
-    stage_end(c, g.levels - 1);
+    stage_end(c, pyramid_launches(c));
     if (level0_out)
         DSDTM_CUDA(c, cudaMemcpy2DAsync(level0_out, px, c->frames_d + (size_t)first_slot * g.frame_stride + g.off[0], g.frame_stride, px, n,
                                         cudaMemcpyDeviceToHost, s));
@@ -1606,7 +1615,8 @@ int dsdtm_batch_stage(dsdtm_ctx* c, int n_pairs, const int* ref_slots, const int
                       const uint8_t* patches10, const double* patch_px, const int* patch_level, int ppp, int align_iters)
 {
     if (!c || !ref_slots || !cur_slots || !feats || !n_feats || !ref_centers || !poses_in) return DSDTM_E_ARG;
-    if (check_pairs(c, n_pairs, ref_slots, cur_slots, feat_stride, n_feats, max_level, min_level, max_iters)) return DSDTM_E_ARG;
+    if (check_grid_frames(c, n_pairs) || check_pairs(c, n_pairs, ref_slots, cur_slots, feat_stride, n_feats, max_level, min_level, max_iters))
+        return DSDTM_E_ARG;
     if (ppp < 0 || ppp > c->prm.max_patches || align_iters < 0) return fail(c, DSDTM_E_ARG, "patches_per_pair > max_patches");
     if (ppp > 0 && (!patches10 || !patch_px || !patch_level)) return fail(c, DSDTM_E_ARG, "null patch arrays");
     cudaStream_t s = c->stream;
@@ -1771,7 +1781,7 @@ static int enqueue_step(dsdtm_ctx* c, int flags, cudaStream_t s, bool timed)
         if (flags & 1) {
             if (timed) stage_begin(c, DSDTM_STAGE_PYRAMID);
             DSDTM_CUDA(c, launch_pyramid_slots(c, c->cur_slots_d, b.n_pairs, s));
-            if (timed) stage_end(c, c->geo.levels - 1);
+            if (timed) stage_end(c, pyramid_launches(c));
         }
         if (timed) stage_begin(c, DSDTM_STAGE_SPARSE_ALIGN);
         DSDTM_CUDA(c, launch_sparse_align(c, b.n_pairs, b.feat_stride, b.max_level, b.min_level, b.max_iters, false, s));
@@ -1862,9 +1872,11 @@ int dsdtm_batch_run(dsdtm_ctx* c, int flags)
         }
         DSDTM_CUDA(c, cudaGraphLaunch(b.graph[gi], c->stream));
         {
+            // what enqueue_step launched when the graph was captured (the capture's own tally was rolled back)
             const int chunks = (c->step_chunks <= 1 || b.n_pairs < 4 * c->sm_count) ? 1 : std::min(c->step_chunks, kMaxStepStreams);
-            if (flags & 2) c->launches += ((flags & 1) ? c->geo.levels - 1 : 0) + 1 + 5 + ((flags & 4) ? 2 : 0) + ((flags & 8) ? (b.kf_n_wanted ? 4 : 3) : 0);
-            else c->launches += ((flags & 1) ? c->geo.levels - 1 : 0) + (long long)chunks * (1 + (b.patches_per_pair > 0 ? 1 : 0));
+            const int pyr = (flags & 1) ? pyramid_launches(c) : 0;
+            if (flags & 2) c->launches += pyr + 1 + 5 + ((flags & 4) ? 2 : 0) + ((flags & 8) ? (b.kf_n_wanted ? 4 : 3) : 0);
+            else c->launches += pyr + (long long)chunks * (1 + (b.patches_per_pair > 0 ? 1 : 0));
         }
     }
     DSDTM_CUDA(c, cudaEventRecord(c->ev_b, c->stream));
@@ -1973,7 +1985,8 @@ static int pair_batch_e2e_impl(dsdtm_ctx* c, int n_pairs, const uint8_t* cur_img
                          int* n_tracked, double* patch_px_out, uint8_t* patch_conv, const E2eChain* chain)
 {
     if (!c || !cur_imgs || !ref_slots || !cur_slots || !feats || !n_feats || !ref_centers || !poses_in || !poses_out || !n_tracked) return DSDTM_E_ARG;
-    if (check_pairs(c, n_pairs, ref_slots, cur_slots, feat_stride, n_feats, max_level, min_level, max_iters)) return DSDTM_E_ARG;
+    if (check_grid_frames(c, n_pairs) || check_pairs(c, n_pairs, ref_slots, cur_slots, feat_stride, n_feats, max_level, min_level, max_iters))
+        return DSDTM_E_ARG;
     if (ppp < 0 || ppp > c->prm.max_patches || align_iters < 0) return fail(c, DSDTM_E_ARG, "patches_per_pair > max_patches");
     if (ppp > 0 && (!patches10 || !patch_px || !patch_level || !patch_px_out || !patch_conv)) return fail(c, DSDTM_E_ARG, "null patch arrays");
     c->batch.staged = false;

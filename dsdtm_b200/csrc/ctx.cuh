@@ -213,6 +213,8 @@ int  stage_collect(dsdtm_ctx* c);
 cudaError_t pyramid_init(dsdtm_ctx* c);
 cudaError_t launch_pyramid(dsdtm_ctx* c, int first_slot, int n, cudaStream_t s);
 cudaError_t launch_pyramid_slots(dsdtm_ctx* c, const int* slots_d, int n, cudaStream_t s);
+// kernel launches of one launch_pyramid / launch_pyramid_slots call (at most levels - 1: small levels may share one launch)
+int pyramid_launches(dsdtm_ctx* c);
 cudaError_t launch_fast_cells(dsdtm_ctx* c, int first_slot, int n, int barrier, float seed_score, bool use_occupied,
                               cudaStream_t s);
 cudaError_t launch_fast_score_map(dsdtm_ctx* c, int slot, int level, int barrier, cudaStream_t s);

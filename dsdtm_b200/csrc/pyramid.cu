@@ -431,12 +431,15 @@ int plan_small_chain(const LevelGeom& g, int first, SmallChain& ch, size_t& smem
     return ch.n;
 }
 
-cudaError_t launch_levels(dsdtm_ctx* c, int first_slot, const int* slots_d, int n, cudaStream_t s)
+// the pyramid of n frames: one launch per level, except that one pyrdown_small_kernel launch builds a chain of small levels.
+// With launch == false nothing is launched and only the count is returned (the launch tally of a replayed step, the profiler's).
+int plan_levels(dsdtm_ctx* c, int first_slot, const int* slots_d, int n, cudaStream_t s, bool launch)
 {
     const LevelGeom& g = c->geo;
     SmallChain chain;
     size_t chain_smem = 0;
-    for (int l = 1; l < g.levels; ++l) {
+    int launches = 0;
+    for (int l = 1; l < g.levels; ++l, ++launches) {
         const int w = g.w[l - 1], h = g.h[l - 1], dw = g.w[l], dh = g.h[l];
         if ((w & 7) == 0 && (dw & 3) == 0 && h >= 3 && 2 * dw == w && (dw >> 2) <= 1024 && (size_t)(2 * BRPT + 3) * w + 2 * BULK_PAD + 16 <= 48 * 1024 && c->pyr_kernel == 0) {
             const int xq = dw >> 2;
@@ -447,22 +450,25 @@ cudaError_t launch_levels(dsdtm_ctx* c, int first_slot, const int* slots_d, int 
             const int tile_rows = strips * BRPT;
             const size_t smem = (size_t)(2 * tile_rows + 3) * w + 2 * BULK_PAD + 16;   // + the round-up of the copy to 16 bytes
             dim3 grid((dh + tile_rows - 1) / tile_rows, n);
-            pyrdown_bulk_kernel<<<grid, xq * strips, smem, s>>>(c->frames_d, g.frame_stride, first_slot, slots_d, g.off[l - 1], g.off[l], w, h, dw, dh, tile_rows);
+            if (launch) pyrdown_bulk_kernel<<<grid, xq * strips, smem, s>>>(c->frames_d, g.frame_stride, first_slot, slots_d, g.off[l - 1], g.off[l], w, h, dw, dh, tile_rows);
         } else if (c->pyr_kernel == 0 && plan_small_chain(g, l, chain, chain_smem) > 0) {
-            pyrdown_small_kernel<<<n, SMALL_THREADS, chain_smem, s>>>(c->frames_d, g.frame_stride, first_slot, slots_d, chain);
-            c->launches++;
+            if (launch) pyrdown_small_kernel<<<n, SMALL_THREADS, chain_smem, s>>>(c->frames_d, g.frame_stride, first_slot, slots_d, chain);
             l += chain.n - 1;                     // the chain produced levels l .. l + n - 1
-            continue;
         } else if ((w & 7) == 0 && (dw & 3) == 0 && h >= 3 && 2 * dw == w && c->pyr_kernel != 1) {
             const int n_items = (dw >> 2) * ((dh + RPT - 1) / RPT);
             dim3 grid((n_items + 127) / 128, n);
-            pyrdown_strip_kernel<<<grid, 128, 0, s>>>(c->frames_d, g.frame_stride, first_slot, slots_d, g.off[l - 1], g.off[l], w, h, dw, dh, n_items);
+            if (launch) pyrdown_strip_kernel<<<grid, 128, 0, s>>>(c->frames_d, g.frame_stride, first_slot, slots_d, g.off[l - 1], g.off[l], w, h, dw, dh, n_items);
         } else {
             dim3 grid((dw + TW - 1) / TW, (dh + TH - 1) / TH, n);
-            pyrdown_tile_kernel<<<grid, 256, 0, s>>>(c->frames_d, g.frame_stride, first_slot, slots_d, g.off[l - 1], g.off[l], w, h, dw, dh);
+            if (launch) pyrdown_tile_kernel<<<grid, 256, 0, s>>>(c->frames_d, g.frame_stride, first_slot, slots_d, g.off[l - 1], g.off[l], w, h, dw, dh);
         }
-        c->launches++;
     }
+    return launches;
+}
+
+cudaError_t launch_levels(dsdtm_ctx* c, int first_slot, const int* slots_d, int n, cudaStream_t s)
+{
+    c->launches += plan_levels(c, first_slot, slots_d, n, s, true);
     return cudaGetLastError();
 }
 
@@ -471,5 +477,6 @@ cudaError_t launch_levels(dsdtm_ctx* c, int first_slot, const int* slots_d, int 
 cudaError_t pyramid_init(dsdtm_ctx*) { return cudaFuncSetAttribute(pyrdown_small_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMALL_SMEM_LIMIT); }
 cudaError_t launch_pyramid(dsdtm_ctx* c, int first_slot, int n, cudaStream_t s) { return launch_levels(c, first_slot, nullptr, n, s); }
 cudaError_t launch_pyramid_slots(dsdtm_ctx* c, const int* slots_d, int n, cudaStream_t s) { return launch_levels(c, 0, slots_d, n, s); }
+int pyramid_launches(dsdtm_ctx* c) { return plan_levels(c, 0, nullptr, 0, nullptr, false); }
 
 }  // namespace dsdtm

@@ -26,6 +26,9 @@ extern "C" {
 #define DSDTM_ABI_VERSION 1
 #define DSDTM_MAX_LEVELS 8
 #define DSDTM_MAX_FEATS_LIMIT 512 /* hard upper bound for dsdtm_params.max_feats */
+/* frames or frame pairs one batched call takes at most, whatever max_batch is: the pyramid, FAST, CLAHE and key-frame lift kernels
+ * index the frame with gridDim.y / gridDim.z, which CUDA caps at 65535. A larger n is DSDTM_E_ARG with nothing enqueued. */
+#define DSDTM_MAX_BATCH_FRAMES 65535
 
 enum {
     DSDTM_OK = 0,
@@ -51,7 +54,8 @@ typedef struct {
     int max_feats;   /* capacity: reference features per frame pair handed to sparse alignment (<= 512) */
     int max_patches; /* capacity: Align2D patches per frame */
     int max_frames;  /* frame slots in the device pool (each holds one full pyramid) */
-    int max_batch;   /* capacity: frame pairs per batched call */
+    int max_batch;   /* capacity: frame pairs per batched call. Not capped: it also sizes the patch capacity max_batch * max_patches,
+                      * but a batched call of frames or pairs takes at most DSDTM_MAX_BATCH_FRAMES of them */
 } dsdtm_params;
 
 /* One reference feature as Sprase_ImgAlign::GetJocabianMat reads it (ref: src/Sprase_ImageAlign.cpp:84-103) */
@@ -129,9 +133,10 @@ int dsdtm_frame_upload_pyramid_host(dsdtm_ctx* ctx, int slot, const uint8_t* img
  * returns once the image has left the caller's buffer; a page-locked `img` must stay unmodified until the next synchronising call
  * (dsdtm_sync or any call that returns results). Errors of the queued work surface at that call. */
 int dsdtm_frame_upload_pyramid_async(dsdtm_ctx* ctx, int slot, const uint8_t* img, int stride);
-/* batched: n dense (stride == width) images into slots first_slot .. first_slot+n-1 */
+/* batched: n dense (stride == width) images into slots first_slot .. first_slot+n-1; n <= DSDTM_MAX_BATCH_FRAMES */
 int dsdtm_frames_upload_pyramid(dsdtm_ctx* ctx, int first_slot, int n, const uint8_t* imgs);
-/* device-resident variant: level 0 of the n slots is already in HBM (e.g. written by a previous upload); rebuild levels */
+/* device-resident variant: level 0 of the n slots is already in HBM (e.g. written by a previous upload); rebuild levels.
+ * n <= DSDTM_MAX_BATCH_FRAMES */
 int dsdtm_frames_build_pyramid(dsdtm_ctx* ctx, int first_slot, int n);
 /* parity helper: copy one level of a slot back (dense w*h bytes) */
 /* Raw upload of ONE level image (w_level x h_level) into a slot, no pyramid: for callers that hold an image that is not a level-0
@@ -148,7 +153,8 @@ int dsdtm_frame_download_level(dsdtm_ctx* ctx, int slot, int level, uint8_t* out
  * The sort and mask-circle selection that follow (ref: :111-150) are dsdtm_detect / dsdtm_detect_batch below. */
 int dsdtm_fast_cells(dsdtm_ctx* ctx, int slot, int barrier, float seed_score, const uint8_t* occupied,
                      dsdtm_corner* cells_out);
-/* batched over n consecutive slots; occupied (may be NULL) and cells_out are n * grid_rows*grid_cols */
+/* batched over n consecutive slots (n <= max_batch and <= DSDTM_MAX_BATCH_FRAMES); occupied (may be NULL) and cells_out are
+ * n * grid_rows*grid_cols */
 int dsdtm_fast_cells_batch(dsdtm_ctx* ctx, int first_slot, int n, int barrier, float seed_score,
                            const uint8_t* occupied, dsdtm_corner* cells_out);
 /* parity helper replacing fast_corner_detect_10[_sse2] + fast_corner_score_10 + fast_nonmax_3x3
@@ -176,7 +182,8 @@ typedef struct {
  *   exact_path (n bytes, may be NULL) = 1 where two cells above 20 tied and the frame was ordered by the restatement of libstdc++'s
  *              std::sort the reference's selection depends on, 0 where the parallel ranking was exact.
  * The result equals the reference's std::sort + walk bit for bit, including the order of tied scores. The device mask buffer is
- * allocated by the first call that passes masks. DSDTM_E_ARG (nothing launched) for a slot out of range, n > max_batch,
+ * allocated by the first call that passes masks. DSDTM_E_ARG (nothing launched) for a slot out of range, n > max_batch or
+ * DSDTM_MAX_BATCH_FRAMES,
  * max_new > out_stride, a radius out of range, NULL out / n_out / max_new, or a frame geometry beyond 752 x 480 pixels. The
  * device time is counted under DSDTM_STAGE_FAST. */
 int dsdtm_detect_batch(dsdtm_ctx* ctx, int first_slot, int n, float detection_threshold, const uint8_t* occupied, const uint8_t* masks,
@@ -308,8 +315,8 @@ int dsdtm_keyframe_lift(dsdtm_ctx* ctx, int depth_slot, const double pose_c2w[7]
  * of the Frame constructor (ref: Test/test_Feature_detection.cpp:85-86, Test/test_Euroc.cpp:64, Test/test_Optimizer.cpp:75,
  * all with (3.0, 8x8)) -- fused with Frame::ComputeImagePyramid: the n dense raw images are equalised into level 0 of slots
  * first_slot.. and their pyramids are built. Bit-exact against OpenCV. The image size must be divisible by the tile grid
- * (OpenCV pads otherwise; not implemented), tiles_x <= 16, tile height >= 8. level0_out (optional, may be NULL): the
- * equalised images back on the host (n * h * w bytes). */
+ * (OpenCV pads otherwise; not implemented), tiles_x <= 16, tile height >= 8, n <= DSDTM_MAX_BATCH_FRAMES. level0_out (optional,
+ * may be NULL): the equalised images back on the host (n * h * w bytes). */
 int dsdtm_frames_upload_clahe_pyramid(dsdtm_ctx* ctx, int first_slot, int n, const uint8_t* imgs, double clip_limit,
                                       int tiles_x, int tiles_y, uint8_t* level0_out);
 
@@ -479,7 +486,7 @@ int dsdtm_track_frame_store(dsdtm_ctx* ctx, const dsdtm_track_store_in* in, dsdt
  * replayed), fetch() copies results back. patches: n_pairs * patches_per_pair entries, patch_level < 0 = unused.
  * flags bit0: rebuild the cur pyramids from their level 0 inside run(); bit1: the refinement chain (dsdtm_batch_stage_map);
  * bit2 (with bit1): selection + pose optimization behind it (dsdtm_batch_stage_track); bit3 (with bit2): the key frame behind the
- * tracked pose (dsdtm_batch_stage_keyframe). */
+ * tracked pose (dsdtm_batch_stage_keyframe). n_pairs <= max_batch and <= DSDTM_MAX_BATCH_FRAMES (DSDTM_E_ARG, nothing staged). */
 int dsdtm_batch_stage(dsdtm_ctx* ctx, int n_pairs, const int* ref_slots, const int* cur_slots,
                       const dsdtm_ref_feat* feats, int feat_stride, const int* n_feats, const double* ref_centers,
                       const double* poses_in, int max_level, int min_level, int max_iters,
@@ -549,7 +556,8 @@ int dsdtm_batch_stage_keyframe(dsdtm_ctx* ctx, const int32_t* depth_slots /* n_p
 int dsdtm_batch_fetch_keyframe(dsdtm_ctx* ctx, int32_t* n_new, dsdtm_corner* corners, dsdtm_lifted* lifted, uint8_t* exact_path);
 int dsdtm_batch_fetch(dsdtm_ctx* ctx, double* poses_out, int* n_tracked, double* patch_px_out, uint8_t* patch_conv);
 /* end-to-end step with HOST buffers: uploads the n_pairs cur images (dense, pinned recommended) into their cur slots,
- * stages the per-pair inputs, runs, and fetches -- copies overlapped with compute in chunks on internal streams. */
+ * stages the per-pair inputs, runs, and fetches -- copies overlapped with compute in chunks on internal streams. Both e2e entries
+ * take n_pairs <= max_batch and <= DSDTM_MAX_BATCH_FRAMES (DSDTM_E_ARG before any copy). */
 /* the same with the refinement chain of dsdtm_batch_stage_map instead of host patches: per pair only the current image, the
  * reference features and three small arrays go up, the poses / counts / per-candidate records come back */
 int dsdtm_track_batch_e2e(dsdtm_ctx* ctx, int n_pairs, const uint8_t* cur_imgs, const int* ref_slots, const int* cur_slots,
