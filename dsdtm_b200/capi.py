@@ -40,6 +40,13 @@ assert MATCH_DT.itemsize == 16
 TRACK_MAX_MATCHES = 200
 CIRCLE_DT = np.dtype([("px", "<f4", 2), ("radius", "<i4"), ("reserved", "<i4")])
 assert CIRCLE_DT.itemsize == 16
+# device-resident map store (dsdtm_store_*)
+STORE_KF_DT = np.dtype([("slot", "<i4"), ("feat_begin", "<i4"), ("feat_count", "<i4"), ("reserved", "<i4"), ("pose_c2w", "<f8", 7),
+                        ("center", "<f8", 3)])
+STORE_FEAT_DT = np.dtype([("mp", "<i4"), ("level", "<i4"), ("px", "<f4", 2), ("normal", "<f8", 3), ("is_obs", "<i4"), ("next_obs", "<i4")])
+STORE_POINT_DT = np.dtype([("point_w", "<f8", 3), ("bad", "<i4"), ("last_obs", "<i4")])
+STORE_CAND_DT = np.dtype([("mp", "<i4"), ("order", "<i4"), ("r", REPROJ_DT)])
+assert STORE_KF_DT.itemsize == 96 and STORE_FEAT_DT.itemsize == 48 and STORE_POINT_DT.itemsize == 32 and STORE_CAND_DT.itemsize == 56
 # dsdtm_batch_run flags: 1 = rebuild the cur pyramids, 2 = the refinement chain (batch_stage_map), 4 (with 2) = SearchLocalPoints'
 # selection + PoseOptimization behind it (batch_stage_track): flags 7 ends in the tracked pose of every pair; 8 (with 4) = the key frame
 # behind the tracked pose (batch_stage_keyframe): flags 15 ends in the new corners and their lifted records
@@ -88,7 +95,7 @@ SYMBOLS = [
     "dsdtm_frame_upload_pyramid_host", "dsdtm_frames_upload_clahe_pyramid", "dsdtm_track_frame",
     "dsdtm_pose_optimize", "dsdtm_pose_optimize_batch", "dsdtm_map_table_upload", "dsdtm_close_keyframes", "dsdtm_probe_fp64", "dsdtm_frame_upload_pyramid_async", "dsdtm_track_frame_store", "dsdtm_store_set_points", "dsdtm_store_update_points", "dsdtm_store_append_keyframe", "dsdtm_store_set_keyframe", "dsdtm_store_clear", "dsdtm_store_track", "dsdtm_frame_upload_level", "dsdtm_batch_stage_map", "dsdtm_batch_fetch_map", "dsdtm_track_batch_e2e",
     "dsdtm_batch_stage_track", "dsdtm_batch_fetch_track", "dsdtm_detect", "dsdtm_detect_batch",
-    "dsdtm_batch_stage_keyframe", "dsdtm_batch_fetch_keyframe",
+    "dsdtm_batch_stage_keyframe", "dsdtm_batch_fetch_keyframe", "dsdtm_batch_stage_store", "dsdtm_batch_fetch_store",
 ]
 
 
@@ -166,6 +173,7 @@ class Context:
         self.grid_rows, self.grid_cols = r.value, c_.value
         self.n_cells = r.value * c_.value
         self.width, self.height = cam["width"], cam["height"]
+        self.store_points = self.store_keyframes = 0       # rows of the map store, as the store_* calls below leave them
 
     def _ck(self, rc):
         if rc != 0:
@@ -445,13 +453,55 @@ class Context:
         return dict(pose_c2r=np.array(to.pose_c2r[:]), pose_cur_c2w=np.array(to.pose_cur_c2w[:]), cur_center=np.array(to.cur_center[:]),
                     n_tracked=int(to.n_tracked)), rep
 
+    # ---- device-resident map store
+    def store_clear(self):
+        self._ck(self.L.dsdtm_store_clear(self.hp))
+        self.store_points = self.store_keyframes = 0
+
+    def store_set_points(self, first, points_w, bad=None):
+        """dsdtm_store_set_points: append (first == current size) or rewrite point rows [first, first + n)"""
+        pw = np.ascontiguousarray(points_w, np.float64).reshape(-1, 3)
+        b = None if bad is None else np.ascontiguousarray(bad, np.int32).reshape(len(pw))
+        self._ck(self.L.dsdtm_store_set_points(self.hp, int(first), len(pw), _p(pw), _p(b)))
+        self.store_points = max(self.store_points, int(first) + len(pw))
+
+    def store_update_points(self, ids, points_w=None, bad=None):
+        """dsdtm_store_update_points: scattered positions (None = keep) and bad flags (None = keep)"""
+        ids = np.ascontiguousarray(ids, np.int32).reshape(-1)
+        pw = None if points_w is None else np.ascontiguousarray(points_w, np.float64).reshape(len(ids), 3)
+        b = None if bad is None else np.ascontiguousarray(bad, np.int32).reshape(len(ids))
+        self._ck(self.L.dsdtm_store_update_points(self.hp, _p(ids), len(ids), _p(pw), _p(b)))
+
+    def store_append_keyframe(self, slot, pose_c2w, center, feats):
+        """dsdtm_store_append_keyframe: feats = STORE_FEAT_DT rows (mp, level, px, normal, is_obs). Returns the key frame's row."""
+        kf = np.zeros(1, STORE_KF_DT)
+        kf["slot"] = slot; kf["pose_c2w"] = pose_c2w; kf["center"] = center
+        fs = np.ascontiguousarray(feats, STORE_FEAT_DT).reshape(-1)
+        row = C.c_int32(0)
+        self._ck(self.L.dsdtm_store_append_keyframe(self.hp, _p(kf), _p(fs), len(fs), C.byref(row)))
+        self.store_keyframes = row.value + 1
+        return row.value
+
+    def store_set_keyframe(self, row, slot, pose_c2w, center):
+        self._ck(self.L.dsdtm_store_set_keyframe(self.hp, int(row), int(slot), _p(np.ascontiguousarray(pose_c2w, np.float64)),
+                                                  _p(np.ascontiguousarray(center, np.float64))))
+
+    def store_track(self, cur_slot, pose_cur_c2w, cur_center, max_local=10, max_search_level=2, align_iters=10, cap=4096):
+        """dsdtm_store_track -> (local key-frame rows in rank order, STORE_CAND_DT records in arrival order). More than cap candidates
+        raises."""
+        local = np.zeros(16, np.int32); nl = C.c_int32(0); out = np.zeros(cap, STORE_CAND_DT); n = C.c_int32(0)
+        self._ck(self.L.dsdtm_store_track(self.hp, int(cur_slot), _p(np.ascontiguousarray(pose_cur_c2w, np.float64)),
+                                          _p(np.ascontiguousarray(cur_center, np.float64)), int(max_local), int(max_search_level),
+                                          int(align_iters), _p(local), C.byref(nl), _p(out), int(cap), C.byref(n)))
+        return local[:nl.value].copy(), out[:n.value].copy()
+
     # ---- batched front end
     def batch_stage(self, ref_slots, cur_slots, feats, n_feats, ref_centers, poses_in, max_level, min_level, max_iters,
                     patches10=None, patch_px=None, patch_level=None, align_iters=10):
         n = len(ref_slots)
         feats = np.ascontiguousarray(feats, REF_FEAT_DT).reshape(n, -1)
         ppp = 0 if patch_level is None else np.asarray(patch_level).reshape(n, -1).shape[1]
-        self._n = n; self._ppp = ppp
+        self._n = n; self._ppp = ppp; self._store_cpf = None
         self._ck(self.L.dsdtm_batch_stage(
             self.hp, n, _p(np.ascontiguousarray(ref_slots, np.int32)), _p(np.ascontiguousarray(cur_slots, np.int32)), _p(feats),
             feats.shape[1], _p(np.ascontiguousarray(n_feats, np.int32)), _p(np.ascontiguousarray(ref_centers, np.float64)),
@@ -463,8 +513,24 @@ class Context:
     def batch_stage_map(self, poses_ref_c2w, points_per_pair, max_search_level, align_iters=10):
         """after batch_stage: the refinement chain's inputs (reference poses); batch_run(flags | 2) then runs the chain"""
         pr = np.ascontiguousarray(poses_ref_c2w, np.float64).reshape(self._n, 7)
-        self._map_ppp = int(points_per_pair)
+        self._map_ppp = int(points_per_pair); self._store_cpf = None
         self._ck(self.L.dsdtm_batch_stage_map(self.hp, _p(pr), int(points_per_pair), int(max_search_level), int(align_iters)))
+
+    def batch_stage_store(self, poses_ref_c2w, kf_range=None, max_local=10, max_search_level=2, align_iters=10, cands_per_frame=1024):
+        """after batch_stage: the store-backed local map (dsdtm_batch_stage_store); kf_range = (n_pairs, 2) key-frame rows [begin, end)
+        or None (every row); batch_run(flags | 2) then runs UpdateLocalMap per frame on the map store"""
+        pr = np.ascontiguousarray(poses_ref_c2w, np.float64).reshape(self._n, 7)
+        kr = None if kf_range is None else np.ascontiguousarray(kf_range, np.int32).reshape(self._n, 2)
+        self._ck(self.L.dsdtm_batch_stage_store(self.hp, _p(pr), _p(kr), int(max_local), int(max_search_level), int(align_iters),
+                                                int(cands_per_frame)))
+        self._store_cpf = int(cands_per_frame)
+
+    def batch_fetch_store(self):
+        """-> (local rows (n, 16), n_local (n,), records (n, cands_per_frame) STORE_CAND_DT in order, n_cand (n,) true counts)"""
+        n, F = self._n, self._store_cpf
+        loc = np.empty((n, 16), np.int32); nl = np.empty(n, np.int32); rec = np.empty((n, F), STORE_CAND_DT); nc = np.empty(n, np.int32)
+        self._ck(self.L.dsdtm_batch_fetch_store(self.hp, _p(loc), _p(nl), _p(rec), _p(nc)))
+        return loc, nl, rec, nc
 
     def batch_fetch_map(self):
         out = np.zeros((self._n, self._map_ppp), REPROJ_DT)
@@ -474,7 +540,11 @@ class Context:
     def batch_stage_track(self, found=None, max_iters=100):
         """after batch_stage_map: found = (n_pairs, points_per_pair) MapPoint::mnFound counts (None = all 1), max_iters = PoseOptimization's
         cap; batch_run(7) then ends in the tracked poses"""
-        f = None if found is None else np.ascontiguousarray(found, np.int32).reshape(self._n, self._map_ppp)
+        f = None if found is None else np.ascontiguousarray(found, np.int32).reshape(-1)
+        if f is not None and getattr(self, "_store_cpf", None) is None:
+            f = f.reshape(self._n, self._map_ppp)
+        elif f is not None and len(f) != self.store_points:     # store mode: one count per store point row
+            raise DsdtmError("batch_stage_track: found has %d entries, the map store %d points" % (len(f), self.store_points))
         self._ck(self.L.dsdtm_batch_stage_track(self.hp, _p(f), int(max_iters)))
 
     def batch_fetch_track(self):

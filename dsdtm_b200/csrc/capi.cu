@@ -196,6 +196,13 @@ static void drop_graphs(dsdtm_ctx* c)
         if (g) { cudaGraphExecDestroy(g); g = nullptr; }
 }
 
+// a map-store change: a captured store-backed step has the tables, their sizes and the grids derived from them baked in (the tables may
+// have been reallocated); steps of the other modes never read the store and stay captured
+static void drop_store_graphs(dsdtm_ctx* c)
+{
+    if (c->batch.store_staged) drop_graphs(c);
+}
+
 static int check_slot(dsdtm_ctx* c, int slot, int n = 1)
 {
     if (slot < 0 || n < 0 || slot + n > c->prm.max_frames) return fail(c, DSDTM_E_ARG, "frame slot out of range");
@@ -328,7 +335,8 @@ void dsdtm_destroy(dsdtm_ctx* c)
                      c->st_kfs_d, c->st_feats_d, c->st_pts_d, c->st_claim_d, c->st_vis_d, c->st_dist_d, c->st_sel_d, c->st_out_d,
                      c->trk_found_d, c->trk_match_d, c->trk_obs_d, c->trk_nobs_d, c->trk_pose_in_d, c->trk_pose_out_d, c->trk_res_d, c->trk_sum_d,
                      c->det_mask_d, c->det_buf_d, c->kf_circ_d, c->kf_ncirc_d, c->kf_max_new_d, c->kf_corner_d, c->kf_lifted_d, c->kf_nnew_d,
-                     c->kf_exact_d, c->kf_depth_slot_d, c->kf_want_d, c->kf_rows_d };
+                     c->kf_exact_d, c->kf_depth_slot_d, c->kf_want_d, c->kf_rows_d,
+                     c->sb_rec_d, c->sb_ncand_d, c->sb_local_d, c->sb_pose10_d, c->sb_range_d, c->sb_found_d };
     for (void* p : bufs) if (p) cudaFree(p);
     if (c->pinned) cudaFreeHost(c->pinned);
     if (c->stage_pin) cudaFreeHost(c->stage_pin);
@@ -1239,6 +1247,7 @@ int dsdtm_store_clear(dsdtm_ctx* c)
     if (!c) return DSDTM_E_ARG;
     c->st_kfs_n = c->st_feats_n = c->st_pts_n = 0;
     c->st_max_feats = 0;
+    drop_store_graphs(c);
     return 0;
 }
 
@@ -1248,6 +1257,7 @@ int dsdtm_store_set_points(dsdtm_ctx* c, int first, int n, const double* point_w
     if (first < 0 || n < 0 || (n && !point_w)) return fail(c, DSDTM_E_ARG, "dsdtm_store_set_points: bad range / null positions");
     if ((size_t)first > c->st_pts_n) return fail(c, DSDTM_E_ARG, "dsdtm_store_set_points: range starts past the end (points are appended or rewritten)");
     if (n == 0) return 0;
+    drop_store_graphs(c);
     const size_t end = (size_t)first + n, old_n = c->st_pts_n;
     const size_t old_claim_cap = c->st_claim_cap;
     if (grow_keep(c, &c->st_pts_d, &c->st_pts_cap, end, old_n) || grow_keep(c, &c->st_claim_d, &c->st_claim_cap, end, old_n)) return DSDTM_E_NOMEM;
@@ -1291,6 +1301,7 @@ int dsdtm_store_update_points(dsdtm_ctx* c, const int32_t* ids, int n, const dou
     if (n < 0 || (n && !ids)) return fail(c, DSDTM_E_ARG, "dsdtm_store_update_points: null ids");
     if (n == 0 || (!point_w && !bad)) return 0;
     for (int i = 0; i < n; ++i) if (ids[i] < 0 || (size_t)ids[i] >= c->st_pts_n) return fail(c, DSDTM_E_ARG, "dsdtm_store_update_points: id outside the point table");
+    drop_store_graphs(c);
     const int chunk = 16384;                                     // 16384 x 32 B + padding fits the 1 MB staging mirror
     cudaStream_t s = c->stream;
     for (int i0 = 0; i0 < n; i0 += chunk) {
@@ -1322,6 +1333,7 @@ int dsdtm_store_append_keyframe(dsdtm_ctx* c, const dsdtm_store_kf* kf, const ds
     for (int j = 0; j < n_feats; ++j)
         if (feats[j].mp >= (int)c->st_pts_n || feats[j].level < 0 || feats[j].level >= c->geo.levels)
             return fail(c, DSDTM_E_ARG, "dsdtm_store_append_keyframe: feature names a map point outside the point table (append the points first) or a bad level");
+    drop_store_graphs(c);
     const size_t r = c->st_kfs_n, f0 = c->st_feats_n;
     if (grow_keep(c, &c->st_kfs_d, &c->st_kfs_cap, r + 1, r) || grow_keep(c, &c->st_feats_d, &c->st_feats_cap, f0 + n_feats, f0)) return DSDTM_E_NOMEM;
     if (grow(c, &c->st_vis_d, &c->st_vis_cap, r + 1) || grow(c, &c->st_dist_d, &c->st_dist_cap, r + 1)) return DSDTM_E_NOMEM;
@@ -1346,6 +1358,7 @@ int dsdtm_store_set_keyframe(dsdtm_ctx* c, int row, int slot, const double pose_
     if (!c || !pose_c2w || !center) return DSDTM_E_ARG;
     if (row < 0 || (size_t)row >= c->st_kfs_n) return fail(c, DSDTM_E_ARG, "dsdtm_store_set_keyframe: row outside the table");
     if (check_slot(c, slot)) return DSDTM_E_ARG;
+    drop_store_graphs(c);
     cudaStream_t s = c->stream;
     dsdtm_store_kf k;
     DSDTM_CUDA(c, cudaMemcpyAsync(&k, c->st_kfs_d + row, sizeof k, cudaMemcpyDeviceToHost, s));
@@ -1631,7 +1644,7 @@ int dsdtm_batch_stage(dsdtm_ctx* c, int n_pairs, const int* ref_slots, const int
     auto& b = c->batch;
     b.staged = true; b.n_pairs = n_pairs; b.feat_stride = feat_stride; b.max_level = max_level; b.min_level = min_level;
     b.max_iters = max_iters; b.patches_per_pair = ppp; b.align_iters = align_iters;
-    b.map_staged = false; b.track_staged = false; b.kf_staged = false;
+    b.map_staged = false; b.store_staged = false; b.track_staged = false; b.kf_staged = false;
     return 0;
 }
 
@@ -1646,8 +1659,90 @@ int dsdtm_batch_stage_map(dsdtm_ctx* c, const double* poses_ref_c2w, int points_
     DSDTM_CUDA(c, cudaMemcpyAsync(c->poses_ref_d, poses_ref_c2w, (size_t)b.n_pairs * 7 * sizeof(double), cudaMemcpyHostToDevice, c->stream));
     DSDTM_CUDA(c, cudaStreamSynchronize(c->stream));
     b.map_staged = true; b.map_ppp = points_per_pair; b.max_search_level = max_search_level; b.map_align_iters = align_iters;
-    b.track_staged = false; b.kf_staged = false;
+    b.store_staged = false; b.track_staged = false; b.kf_staged = false;
     drop_graphs(c);
+    return 0;
+}
+
+// prelude CTA of the store-backed chain: the longest range and the table for max_local key frames must fit one CTA's shared memory
+static int check_store_batch_smem(dsdtm_ctx* c, int range_len, int max_local, const char* who)
+{
+    int max_smem = 0;
+    DSDTM_CUDA(c, cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, c->device));
+    if (store_batch_smem(c, range_len, max_local) > (size_t)max_smem - 1024) {
+        char buf[160];
+        snprintf(buf, sizeof buf, "%s: key-frame range and local map beyond one CTA's shared memory", who);
+        return fail(c, DSDTM_E_ARG, buf);
+    }
+    return 0;
+}
+
+int dsdtm_batch_stage_store(dsdtm_ctx* c, const double* poses_ref_c2w, const int32_t* kf_range, int max_local, int max_search_level,
+                            int align_iters, int cands_per_frame)
+{
+    if (!c || !poses_ref_c2w) return DSDTM_E_ARG;
+    auto& b = c->batch;
+    if (!b.staged) return fail(c, DSDTM_E_STATE, "dsdtm_batch_stage_store: call dsdtm_batch_stage first");
+    if (c->st_kfs_n == 0) return fail(c, DSDTM_E_ARG, "dsdtm_batch_stage_store: the map store is empty");
+    if (max_local < 1 || max_local > 16) return fail(c, DSDTM_E_ARG, "dsdtm_batch_stage_store: max_local must be 1..16");
+    if (cands_per_frame < 1 || cands_per_frame > c->prm.max_patches)
+        return fail(c, DSDTM_E_ARG, "dsdtm_batch_stage_store: cands_per_frame must be 1..max_patches");
+    if (max_search_level < 0 || max_search_level >= c->geo.levels || align_iters < 0)
+        return fail(c, DSDTM_E_ARG, "dsdtm_batch_stage_store: bad max_search_level / align_iters");
+    const int n = b.n_pairs, n_kfs = (int)c->st_kfs_n;
+    int range_max = n_kfs, range_end = n_kfs;
+    if (kf_range) {
+        range_max = 0; range_end = 0;
+        for (int i = 0; i < n; ++i) {
+            const int k0 = kf_range[2 * i], k1 = kf_range[2 * i + 1];
+            if (k0 < 0 || k1 < k0 || k1 > n_kfs) return fail(c, DSDTM_E_ARG, "dsdtm_batch_stage_store: key-frame range outside the store");
+            range_max = std::max(range_max, k1 - k0); range_end = std::max(range_end, k1);
+        }
+    }
+    if (check_store_batch_smem(c, range_max, max_local, "dsdtm_batch_stage_store")) return DSDTM_E_ARG;
+    const size_t B = c->prm.max_batch;
+    if (!c->sb_rec_d) {
+        // once per context at max_batch size: a captured step keeps pointing at these buffers
+        if (dalloc(c, &c->sb_rec_d, B * std::max(c->prm.max_patches, 1)) || dalloc(c, &c->sb_ncand_d, B) || dalloc(c, &c->sb_local_d, B * 17) ||
+            dalloc(c, &c->sb_pose10_d, B * 10) || dalloc(c, &c->sb_range_d, B))
+            return DSDTM_E_NOMEM;
+        DSDTM_CUDA(c, store_batch_init(c));
+        DSDTM_CUDA(c, track_select_init(c));
+    }
+    cudaStream_t s = c->stream;
+    DSDTM_CUDA(c, cudaMemcpyAsync(c->poses_ref_d, poses_ref_c2w, (size_t)n * 7 * sizeof(double), cudaMemcpyHostToDevice, s));
+    if (kf_range) DSDTM_CUDA(c, cudaMemcpyAsync(c->sb_range_d, kf_range, (size_t)n * sizeof(int2), cudaMemcpyHostToDevice, s));
+    DSDTM_CUDA(c, cudaStreamSynchronize(s));
+    b.store_staged = true; b.store_all_rows = kf_range == nullptr; b.store_max_local = max_local; b.store_cpf = cands_per_frame;
+    b.store_range_max = range_max; b.store_range_end = range_end;
+    b.max_search_level = max_search_level; b.map_align_iters = align_iters;
+    b.map_staged = false; b.track_staged = false; b.kf_staged = false;
+    drop_graphs(c);
+    return 0;
+}
+
+int dsdtm_batch_fetch_store(dsdtm_ctx* c, int32_t* local_rows, int32_t* n_local, dsdtm_store_cand* cands, int32_t* n_cand)
+{
+    if (!c) return DSDTM_E_ARG;
+    auto& b = c->batch;
+    if (!b.staged || !b.store_staged) return fail(c, DSDTM_E_STATE, "dsdtm_batch_fetch_store: no staged store batch");
+    cudaStream_t s = c->stream;
+    const size_t n = (size_t)b.n_pairs, F = (size_t)b.store_cpf;
+    std::vector<int32_t> loc(n * 17), nc(n);
+    DSDTM_CUDA(c, cudaMemcpyAsync(loc.data(), c->sb_local_d, n * 17 * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+    DSDTM_CUDA(c, cudaMemcpyAsync(nc.data(), c->sb_ncand_d, n * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+    if (cands) DSDTM_CUDA(c, cudaMemcpyAsync(cands, c->sb_rec_d, n * F * sizeof(dsdtm_store_cand), cudaMemcpyDeviceToHost, s));
+    DSDTM_CUDA(c, cudaStreamSynchronize(s));
+    for (size_t i = 0; i < n; ++i) {
+        if (local_rows) for (int r = 0; r < 16; ++r) local_rows[16 * i + r] = loc[17 * i + 1 + r];
+        if (n_local) n_local[i] = loc[17 * i];
+        // rows past a frame's count hold what earlier replays left there
+        const size_t k = std::min((size_t)std::max(nc[i], 0), F);
+        if (cands) std::memset(cands + i * F + k, 0, (F - k) * sizeof(dsdtm_store_cand));
+    }
+    if (n_cand) std::memcpy(n_cand, nc.data(), n * sizeof(int32_t));
+    float ms = 0.f;
+    if (cudaEventElapsedTime(&ms, c->ev_a, c->ev_b) == cudaSuccess) c->last_run_ms = ms;
     return 0;
 }
 
@@ -1655,10 +1750,19 @@ int dsdtm_batch_stage_track(dsdtm_ctx* c, const int32_t* found, int max_iters)
 {
     if (!c) return DSDTM_E_ARG;
     auto& b = c->batch;
-    if (!b.staged || !b.map_staged) return fail(c, DSDTM_E_STATE, "dsdtm_batch_stage_track: call dsdtm_batch_stage_map first");
+    if (!b.staged || !(b.map_staged || b.store_staged))
+        return fail(c, DSDTM_E_STATE, "dsdtm_batch_stage_track: call dsdtm_batch_stage_map or dsdtm_batch_stage_store first");
     if (max_iters < 0) return fail(c, DSDTM_E_ARG, "negative max_iters");
     if (c->prm.cell_size > track_select_max_radius()) return fail(c, DSDTM_E_ARG, "dsdtm_batch_stage_track: cell_size above the selection's circle bound");
     if (c->n_cells >= (1 << 22)) return fail(c, DSDTM_E_ARG, "dsdtm_batch_stage_track: too many grid cells");
+    if (b.store_staged && track_select_key_bits(c, b.store_cpf) > 64)
+        return fail(c, DSDTM_E_ARG, "dsdtm_batch_stage_track: grid cells x cands_per_frame beyond the selection's 64-bit keys");
+    if (b.store_staged) {
+        int max_smem = 0;
+        DSDTM_CUDA(c, cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, c->device));
+        if (track_select_smem(b.store_cpf) > (size_t)max_smem - 1024)
+            return fail(c, DSDTM_E_ARG, "dsdtm_batch_stage_track: cands_per_frame beyond the selection's shared memory");
+    }
     const size_t B = c->prm.max_batch, K = DSDTM_TRACK_MAX_MATCHES;
     if (!c->trk_found_d) {
         // once per context at max_batch size: a captured step keeps pointing at these buffers
@@ -1668,10 +1772,17 @@ int dsdtm_batch_stage_track(dsdtm_ctx* c, const int32_t* found, int max_iters)
             return DSDTM_E_NOMEM;
     }
     cudaStream_t s = c->stream;
-    const size_t n = (size_t)b.n_pairs * b.map_ppp;
+    // per pair and record, or in store mode per store point row
+    const size_t n = b.store_staged ? c->st_pts_n : (size_t)b.n_pairs * b.map_ppp;
     std::vector<int32_t> ones;
-    if (!found) { ones.assign(n, 1); found = ones.data(); }                 // MapPoint::mnFound starts at 1
-    DSDTM_CUDA(c, cudaMemcpyAsync(c->trk_found_d, found, n * sizeof(int32_t), cudaMemcpyHostToDevice, s));
+    if (!found) { ones.assign(std::max(n, (size_t)1), 1); found = ones.data(); }   // MapPoint::mnFound starts at 1
+    if (b.store_staged) {
+        if (grow(c, &c->sb_found_d, &c->sb_found_cap, std::max(n, (size_t)1))) return DSDTM_E_NOMEM;
+        if (n) DSDTM_CUDA(c, cudaMemcpyAsync(c->sb_found_d, found, n * sizeof(int32_t), cudaMemcpyHostToDevice, s));
+        b.store_n_found = (int)n;
+    } else {
+        DSDTM_CUDA(c, cudaMemcpyAsync(c->trk_found_d, found, n * sizeof(int32_t), cudaMemcpyHostToDevice, s));
+    }
     // rows past a pair's match count are never written by the step: defined (zero) bytes for the fetch
     DSDTM_CUDA(c, cudaMemsetAsync(c->trk_match_d, 0, B * K * sizeof(dsdtm_match), s));
     DSDTM_CUDA(c, cudaMemsetAsync(c->trk_res_d, 0, B * K * sizeof(double), s));
@@ -1686,7 +1797,8 @@ int dsdtm_batch_stage_keyframe(dsdtm_ctx* c, const int32_t* depth_slots, const u
 {
     if (!c) return DSDTM_E_ARG;
     auto& b = c->batch;
-    if (!b.staged || !b.map_staged || !b.track_staged) return fail(c, DSDTM_E_STATE, "dsdtm_batch_stage_keyframe: call dsdtm_batch_stage_track first");
+    if (!b.staged || !(b.map_staged || b.store_staged) || !b.track_staged)
+        return fail(c, DSDTM_E_STATE, "dsdtm_batch_stage_keyframe: call dsdtm_batch_stage_track first");
     if (!dist || !(detection_threshold >= 0.f)) return fail(c, DSDTM_E_ARG, "dsdtm_batch_stage_keyframe: dist NULL or detection_threshold < 0");
     if (max_fts < 1 || max_fts > DSDTM_MAX_FEATS_LIMIT) return fail(c, DSDTM_E_ARG, "dsdtm_batch_stage_keyframe: max_fts must be 1..DSDTM_MAX_FEATS_LIMIT");
     if (min_dist < 0 || min_dist > detect_select_max_radius() || c->prm.cell_size > detect_select_max_radius())
@@ -1750,12 +1862,14 @@ static int enqueue_keyframe(dsdtm_ctx* c, cudaStream_t s, bool timed)
 static int enqueue_track(dsdtm_ctx* c, cudaStream_t s, bool timed)
 {
     auto& b = c->batch;
+    const int ppp = b.store_staged ? b.store_cpf : b.map_ppp;
     if (timed) stage_begin(c, DSDTM_STAGE_LOCAL_MAP);
-    DSDTM_CUDA(c, launch_track_select(c, b.n_pairs, b.feat_stride, b.map_ppp, s));
+    if (b.store_staged) DSDTM_CUDA(c, launch_track_select_store(c, b.n_pairs, b.store_cpf, b.store_n_found, s));
+    else DSDTM_CUDA(c, launch_track_select(c, b.n_pairs, b.feat_stride, b.map_ppp, s));
     if (timed) stage_end(c, 1);
     const PoseOptIo io = { c->trk_obs_d, c->trk_nobs_d, c->trk_pose_in_d, c->trk_pose_out_d, c->trk_res_d, c->trk_sum_d };
     if (timed) stage_begin(c, DSDTM_STAGE_POSE_OPT);
-    DSDTM_CUDA(c, launch_pose_opt_io(c, io, b.n_pairs, DSDTM_TRACK_MAX_MATCHES, std::min(DSDTM_TRACK_MAX_MATCHES, b.map_ppp), b.track_iters, s));
+    DSDTM_CUDA(c, launch_pose_opt_io(c, io, b.n_pairs, DSDTM_TRACK_MAX_MATCHES, std::min(DSDTM_TRACK_MAX_MATCHES, ppp), b.track_iters, s));
     if (timed) stage_end(c, 1);
     return 0;
 }
@@ -1786,7 +1900,28 @@ static int enqueue_step(dsdtm_ctx* c, int flags, cudaStream_t s, bool timed)
         if (timed) stage_begin(c, DSDTM_STAGE_SPARSE_ALIGN);
         DSDTM_CUDA(c, launch_sparse_align(c, b.n_pairs, b.feat_stride, b.max_level, b.min_level, b.max_iters, false, s));
         if (timed) stage_end(c, 1);
-        if (chain) {
+        if (chain && b.store_staged) {
+            // TrackWithLocalMap right after Run on the map store: per frame UpdateLocalMap over its key-frame rows, then the candidates
+            const int n = b.n_pairs * b.store_cpf;
+            if (timed) stage_begin(c, DSDTM_STAGE_LOCAL_MAP);
+            DSDTM_CUDA(c, launch_store_batch(c, b.n_pairs, b.store_all_rows, b.store_all_rows ? (int)c->st_kfs_n : b.store_range_max,
+                                             b.store_max_local, b.store_cpf, b.max_search_level, s));
+            if (timed) stage_end(c, 2);
+            if (timed) stage_begin(c, DSDTM_STAGE_WARP_AFFINE);
+            DSDTM_CUDA(c, launch_warp_affine(c, n, c->patches_d, s));
+            if (timed) stage_end(c, 1);
+            if (timed) stage_begin(c, DSDTM_STAGE_ALIGN2D);
+            DSDTM_CUDA(c, launch_align2d(c, n, b.map_align_iters, s, 0, nullptr, c->sb_rec_d));
+            if (timed) stage_end(c, 1);
+            if (flags & 4) {
+                int r = enqueue_track(c, s, timed);
+                if (r) return r;
+            }
+            if (flags & 8) {
+                int r = enqueue_keyframe(c, s, timed);
+                if (r) return r;
+            }
+        } else if (chain) {
             // TrackWithLocalMap right after Run: the patches come from the reference frame through the aligned pose, nothing from the host
             if (timed) stage_begin(c, DSDTM_STAGE_LOCAL_MAP);
             DSDTM_CUDA(c, launch_pair_candidates(c, 0, b.n_pairs, b.feat_stride, b.map_ppp, s));
@@ -1840,7 +1975,15 @@ int dsdtm_batch_run(dsdtm_ctx* c, int flags)
     if (!c) return DSDTM_E_ARG;
     auto& b = c->batch;
     if (!b.staged) return fail(c, DSDTM_E_STATE, "dsdtm_batch_run: no staged batch");
-    if ((flags & 2) && !b.map_staged) return fail(c, DSDTM_E_STATE, "dsdtm_batch_run: flags bit 1 needs dsdtm_batch_stage_map");
+    if ((flags & 2) && !(b.map_staged || b.store_staged))
+        return fail(c, DSDTM_E_STATE, "dsdtm_batch_run: flags bit 1 needs dsdtm_batch_stage_map or dsdtm_batch_stage_store");
+    if ((flags & 2) && b.store_staged) {
+        // the store may have changed since staging (every change dropped the captured steps): the ranges and the prelude must still fit
+        if (c->st_kfs_n == 0 || (size_t)b.store_range_end > c->st_kfs_n)
+            return fail(c, DSDTM_E_STATE, "dsdtm_batch_run: the map store no longer holds the staged key-frame ranges");
+        if (check_store_batch_smem(c, b.store_all_rows ? (int)c->st_kfs_n : b.store_range_max, b.store_max_local, "dsdtm_batch_run"))
+            return DSDTM_E_ARG;
+    }
     if ((flags & 4) && !(flags & 2)) return fail(c, DSDTM_E_STATE, "dsdtm_batch_run: flags bit 2 needs bit 1 (the refinement chain)");
     if ((flags & 4) && !b.track_staged) return fail(c, DSDTM_E_STATE, "dsdtm_batch_run: flags bit 2 needs dsdtm_batch_stage_track");
     if ((flags & 8) && !(flags & 4)) return fail(c, DSDTM_E_STATE, "dsdtm_batch_run: flags bit 3 needs bit 2 (the tracked pose)");
@@ -1875,7 +2018,7 @@ int dsdtm_batch_run(dsdtm_ctx* c, int flags)
             // what enqueue_step launched when the graph was captured (the capture's own tally was rolled back)
             const int chunks = (c->step_chunks <= 1 || b.n_pairs < 4 * c->sm_count) ? 1 : std::min(c->step_chunks, kMaxStepStreams);
             const int pyr = (flags & 1) ? pyramid_launches(c) : 0;
-            if (flags & 2) c->launches += pyr + 1 + 5 + ((flags & 4) ? 2 : 0) + ((flags & 8) ? (b.kf_n_wanted ? 4 : 3) : 0);
+            if (flags & 2) c->launches += pyr + 1 + (b.store_staged ? 4 : 5) + ((flags & 4) ? 2 : 0) + ((flags & 8) ? (b.kf_n_wanted ? 4 : 3) : 0);
             else c->launches += pyr + (long long)chunks * (1 + (b.patches_per_pair > 0 ? 1 : 0));
         }
     }
@@ -1915,7 +2058,7 @@ int dsdtm_batch_fetch_track(dsdtm_ctx* c, double* poses_c2w_out, int32_t* n_matc
 {
     if (!c) return DSDTM_E_ARG;
     auto& b = c->batch;
-    if (!b.staged || !b.map_staged || !b.track_staged) return fail(c, DSDTM_E_STATE, "dsdtm_batch_fetch_track: no staged track batch");
+    if (!b.staged || !(b.map_staged || b.store_staged) || !b.track_staged) return fail(c, DSDTM_E_STATE, "dsdtm_batch_fetch_track: no staged track batch");
     cudaStream_t s = c->stream;
     const size_t n = (size_t)b.n_pairs, K = DSDTM_TRACK_MAX_MATCHES;
     if (poses_c2w_out) DSDTM_CUDA(c, cudaMemcpyAsync(poses_c2w_out, c->trk_pose_out_d, n * 7 * sizeof(double), cudaMemcpyDeviceToHost, s));
@@ -1923,7 +2066,21 @@ int dsdtm_batch_fetch_track(dsdtm_ctx* c, double* poses_c2w_out, int32_t* n_matc
     if (matches) DSDTM_CUDA(c, cudaMemcpyAsync(matches, c->trk_match_d, n * K * sizeof(dsdtm_match), cudaMemcpyDeviceToHost, s));
     if (res_norm) DSDTM_CUDA(c, cudaMemcpyAsync(res_norm, c->trk_res_d, n * K * sizeof(double), cudaMemcpyDeviceToHost, s));
     if (summaries) DSDTM_CUDA(c, cudaMemcpyAsync(summaries, c->trk_sum_d, n * sizeof(dsdtm_ba_summary), cudaMemcpyDeviceToHost, s));
+    std::vector<int32_t> nm;
+    std::vector<double> prior;
+    if (b.store_staged) {
+        // match counts change with the store between replays, and an overflowed frame (-1) keeps its prior pose
+        nm.resize(n); prior.resize(n * 7);
+        DSDTM_CUDA(c, cudaMemcpyAsync(nm.data(), c->trk_nobs_d, n * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+        DSDTM_CUDA(c, cudaMemcpyAsync(prior.data(), c->trk_pose_in_d, n * 7 * sizeof(double), cudaMemcpyDeviceToHost, s));
+    }
     DSDTM_CUDA(c, cudaStreamSynchronize(s));
+    for (size_t i = 0; i < nm.size(); ++i) {
+        const size_t k = (size_t)std::max(nm[i], 0);
+        if (matches) std::memset(matches + i * K + k, 0, (K - k) * sizeof(dsdtm_match));
+        if (res_norm) std::memset(res_norm + i * K + k, 0, (K - k) * sizeof(double));
+        if (nm[i] < 0 && poses_c2w_out) std::memcpy(poses_c2w_out + 7 * i, prior.data() + 7 * i, 7 * sizeof(double));
+    }
     float ms = 0.f;
     if (cudaEventElapsedTime(&ms, c->ev_a, c->ev_b) == cudaSuccess) c->last_run_ms = ms;
     return 0;
@@ -1933,7 +2090,8 @@ int dsdtm_batch_fetch_keyframe(dsdtm_ctx* c, int32_t* n_new, dsdtm_corner* corne
 {
     if (!c) return DSDTM_E_ARG;
     auto& b = c->batch;
-    if (!b.staged || !b.map_staged || !b.track_staged || !b.kf_staged) return fail(c, DSDTM_E_STATE, "dsdtm_batch_fetch_keyframe: no staged key-frame batch");
+    if (!b.staged || !(b.map_staged || b.store_staged) || !b.track_staged || !b.kf_staged)
+        return fail(c, DSDTM_E_STATE, "dsdtm_batch_fetch_keyframe: no staged key-frame batch");
     cudaStream_t s = c->stream;
     const size_t n = (size_t)b.n_pairs, F = (size_t)b.kf_max_fts;
     std::vector<int32_t> nn(n);

@@ -158,6 +158,14 @@ struct dsdtm_ctx {
     int* kf_depth_slot_d = nullptr;              // max_batch, -1 = no depth
     uint8_t* kf_want_d = nullptr;                // max_batch
     int* kf_rows_d = nullptr;                    // max_batch: the wanted pairs in index order (the rows of the FAST grid)
+    // store-backed local maps of the batched chain (dsdtm_batch_stage_store): allocated once per context at max_batch size, like trk_*,
+    // except the per-point found counts, which follow the point table (any store change drops the captured steps)
+    dsdtm_store_cand* sb_rec_d = nullptr;        // max_batch * max_patches records (row stride: the staged cands_per_frame)
+    int* sb_ncand_d = nullptr;                   // max_batch: true candidate count per frame
+    int* sb_local_d = nullptr;                   // max_batch * 17: n_local, then the local key-frame rows in rank order
+    double* sb_pose10_d = nullptr;               // max_batch * 10: prior pose {c2w[7], centre[3]} = T_c2r * T_ref
+    int2* sb_range_d = nullptr;                  // max_batch key-frame row ranges [begin, end)
+    int* sb_found_d = nullptr;           size_t sb_found_cap = 0;    // per store point row: MapPoint::mnFound
     // key-frame detection (dsdtm_detect_batch), grown on demand
     uint8_t* det_mask_d = nullptr;       size_t det_mask_cap = 0;    // n * w*h mask images: allocated by the first call that passes masks
     uint8_t* det_buf_d = nullptr;        size_t det_buf_cap = 0;     // small inputs (max_new, n_circles, circles) | outputs, one copy each way
@@ -177,6 +185,9 @@ struct dsdtm_ctx {
         int map_ppp = 0, max_search_level = 0, map_align_iters = 0;
         bool track_staged = false;                         // dsdtm_batch_stage_track: selection + pose optimization buffers are ready
         int track_iters = 0;
+        bool store_staged = false;                         // dsdtm_batch_stage_store: bits 1..3 run on the map store instead
+        bool store_all_rows = false;                       // no ranges staged: every frame reads rows [0, key frames at capture)
+        int store_max_local = 0, store_cpf = 0, store_range_max = 0, store_range_end = 0, store_n_found = 0;
         bool kf_staged = false;                            // dsdtm_batch_stage_keyframe: the key-frame half is ready
         int kf_min_dist = 0, kf_max_fts = 0, kf_n_wanted = 0;
         float kf_thr = 0.f, kf_dist[5] = {}, kf_depth_scale = 1.f;
@@ -245,6 +256,12 @@ struct StoreTrackArgs {
 cudaError_t launch_store_link(dsdtm_ctx* c, int feat_begin, int n_feats, cudaStream_t s);
 cudaError_t launch_store_track(dsdtm_ctx* c, const StoreTrackArgs& a, cudaStream_t s);
 const int* store_count_dev(dsdtm_ctx* c);     // number of candidate records of the last launch_store_track, on the device
+// the batched chain on the map store (dsdtm_batch_stage_store): per frame, one prelude CTA (pose, close test, ranking, first-listing-wins
+// walk into the frame's records in `order`) and the candidate records + SolveAffineMatrix / GetBestSearchLevel of entries
+// [f * cpf, f * cpf + cpf); range_len = the longest staged range, all_end = the range of frames without one
+size_t store_batch_smem(const dsdtm_ctx* c, int range_len, int max_local);
+cudaError_t store_batch_init(dsdtm_ctx* c);
+cudaError_t launch_store_batch(dsdtm_ctx* c, int n_pairs, bool all_rows, int range_len, int max_local, int cpf, int max_search_level, cudaStream_t s);
 cudaError_t launch_compose_pose(dsdtm_ctx* c, const double* t_c2r_d, const double pose_ref_c2w[7], double* out10_d, cudaStream_t s);
 cudaError_t launch_close_keyframes(dsdtm_ctx* c, const double pose_cur[7], int n_kfs, cudaStream_t s);
 cudaError_t pose_opt_init(dsdtm_ctx* c);
@@ -258,6 +275,11 @@ struct PoseOptIo {
 cudaError_t launch_pose_opt_io(dsdtm_ctx* c, const PoseOptIo& io, int n_frames, int obs_stride, int max_obs, int max_iters, cudaStream_t s);
 // SearchLocalPoints' selection over the batched chain's records + the PoseOptimization inputs of every pair (select.cu)
 cudaError_t launch_track_select(dsdtm_ctx* c, int n_pairs, int feat_stride, int ppp, cudaStream_t s);
+// the same over the store-backed records (sb_rec_d, cpf per frame): found counts per point row (n_found of them; later rows count 1)
+cudaError_t launch_track_select_store(dsdtm_ctx* c, int n_pairs, int cpf, int n_found, cudaStream_t s);
+size_t track_select_smem(int ppp);             // dynamic shared memory of one selection CTA for ppp records per frame
+int track_select_key_bits(const dsdtm_ctx* c, int ppp);   // bits of a selection key for this grid and ppp (must be <= 64)
+cudaError_t track_select_init(dsdtm_ctx* c);
 int track_select_max_radius();                 // largest Camera.CellSize the selection's circle table holds
 // Feature_detector::detect's sort + mask-circle selection over the cell keys of the last launch_fast_cells (detect_select.cu)
 cudaError_t launch_detect_select(dsdtm_ctx* c, int n, float seed, const uint8_t* masks_d, const dsdtm_circle* circles_d, int circle_stride,

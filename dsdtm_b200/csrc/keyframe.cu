@@ -7,7 +7,7 @@
 //                                pair's mask circles for detect_select_kernel: SearchLocalPoints' filled circles of radius CellSize
 //                                (ref: src/Feature_alignment.cpp:100-113) and Frame::Set_Mask's of radius Camera.Min_dist (ref:
 //                                src/Frame.cpp:286-298; every match carries a map point), both at the match's float px. max_new =
-//                                Max_fts - n_matches, 0 for a pair that is not wanted. The wanted pairs' rows of the occupancy grid and
+//                                Max_fts - n_matches, 0 for a pair that is not wanted or not tracked (n_matches -1). The wanted pairs' rows of the occupancy grid and
 //                                of the FAST cell keys are zeroed here, so every replay rewrites everything it reads (no memset nodes).
 //   (fast_kernel on the cur slots, detect_select_kernel: Feature_detector::detect, fast.cu / detect_select.cu)
 //   keyframe_lift_batch_kernel : grid (corner blocks, pair). The new corners are not mbInitial: Frame::UndistortFeatures,
@@ -32,7 +32,7 @@ struct SeedArgs {
 __global__ void __launch_bounds__(kSeedThreads) keyframe_seed_kernel(const SeedArgs a)
 {
     const int pair = blockIdx.x, tid = threadIdx.x;
-    if (!a.want[pair]) {
+    if (!a.want[pair] || a.n_match[pair] < 0) {          // n_match -1: the store-backed frame overflowed its rows and was not tracked
         if (tid == 0) { a.n_circ[pair] = 0; a.max_new[pair] = 0; }
         return;
     }

@@ -553,33 +553,23 @@ __global__ void __launch_bounds__(1024) store_prelude_kernel(const StArgs a)
     if (t == 0) { a.sel[0] = n_sel; a.sel[17] = 0; }
 }
 
-// ReprojectPoint for the claimed points; the ones inside the image become candidates: Get_ClosetObs over the observation chain,
-// the IsInImage gate, and the dsdtm_candidate record, handed to candidate_prep_one in the same thread
-// (ref: src/Feature_alignment.cpp:54-69,128-141,160-204)
-__global__ void __launch_bounds__(128) store_candidates_kernel(const StArgs a)
+// Frame::World2Pixel of a map point (ref: src/Frame.cpp:318-323), as every kernel of this file computes it
+__device__ __forceinline__ void store_project(const StArgs& a, const double* pose, double P0, double P1, double P2, double& u, double& v)
 {
-    const int j = blockIdx.x * blockDim.x + threadIdx.x, r = blockIdx.y;
-    if (r >= a.sel[0]) return;
-    const dsdtm_store_kf& kfr = a.kfs[a.sel[1 + r]];
-    if (j >= kfr.feat_count) return;
-    const int mp = a.feats[kfr.feat_begin + j].mp;
-    if (mp < 0 || a.pts[mp].bad) return;
-    const unsigned order = (unsigned)((r << 16) | j);
-    if (a.claim[mp] != (((unsigned long long)a.epoch_inv << 32) | order)) return;
-    const double P0 = a.pts[mp].point_w[0], P1 = a.pts[mp].point_w[1], P2 = a.pts[mp].point_w[2];
-    double pose[7], cc[3];
-#pragma unroll
-    for (int q = 0; q < 7; ++q) pose[q] = a.pose_dev ? a.pose_dev[q] : a.pose[q];
-#pragma unroll
-    for (int q = 0; q < 3; ++q) cc[q] = a.pose_dev ? a.pose_dev[7 + q] : a.center[q];
     double q0, q1, q2;
     qrot_exact(pose, P0, P1, P2, q0, q1, q2);
     q0 = __dadd_rn(q0, pose[4]); q1 = __dadd_rn(q1, pose[5]); q2 = __dadd_rn(q2, pose[6]);
-    const double u = __dadd_rn(__ddiv_rn(__dmul_rn((double)a.fx, q0), q2), (double)a.cx);
-    const double v = __dadd_rn(__ddiv_rn(__dmul_rn((double)a.fy, q1), q2), (double)a.cy);
-    if (!in_image(__double2float_rn(u), __double2float_rn(v), 8, 0, a.width, a.height)) return;      // ref: :58
-    const int slot_out = atomicAdd(a.sel + 17, 1);
-    if (slot_out >= a.cap) return;
+    u = __dadd_rn(__ddiv_rn(__dmul_rn((double)a.fx, q0), q2), (double)a.cx);
+    v = __dadd_rn(__ddiv_rn(__dmul_rn((double)a.fy, q1), q2), (double)a.cy);
+}
+
+// A map point that landed in the image at (u, v) (ReprojectPoint returned true): its cell, Get_ClosetObs over its observation chain,
+// the IsInImage gate, and the dsdtm_candidate record, handed to candidate_prep_one as entry i in the same thread
+// (ref: src/Feature_alignment.cpp:54-69,128-141,160-204). Returns the record's reprojection fields.
+__device__ __forceinline__ dsdtm_reproj store_candidate_one(const StArgs& a, int mp, const double* pose, const double* cc, double u, double v,
+                                                            int i, int cur_slot)
+{
+    const double P0 = a.pts[mp].point_w[0], P1 = a.pts[mp].point_w[1], P2 = a.pts[mp].point_w[2];
     int flags = DSDTM_LM_IN_IMAGE;
     const int cell = (int)__ddiv_rn(v, (double)a.cell_size) * a.grid_cols + (int)__ddiv_rn(u, (double)a.cell_size);
     double f0 = __dsub_rn(cc[0], P0), f1 = __dsub_rn(cc[1], P1), f2 = __dsub_rn(cc[2], P2);
@@ -622,12 +612,230 @@ __global__ void __launch_bounds__(128) store_candidates_kernel(const StArgs a)
             for (int k = 0; k < 7; ++k) cd.pose_c2r[k] = T[k];
         }
     }
-    candidate_prep_one(a.cp, slot_out, cd, a.cur_slot);
+    candidate_prep_one(a.cp, i, cd, cur_slot);
+    dsdtm_reproj r;
+    r.px_proj[0] = u; r.px_proj[1] = v; r.px[0] = u; r.px[1] = v;
+    r.cell = cell; r.obs = best; r.flags = flags; r.level = -1;
+    return r;
+}
+
+// ReprojectPoint for the claimed points; the ones inside the image become candidates (store_candidate_one)
+__global__ void __launch_bounds__(128) store_candidates_kernel(const StArgs a)
+{
+    const int j = blockIdx.x * blockDim.x + threadIdx.x, r = blockIdx.y;
+    if (r >= a.sel[0]) return;
+    const dsdtm_store_kf& kfr = a.kfs[a.sel[1 + r]];
+    if (j >= kfr.feat_count) return;
+    const int mp = a.feats[kfr.feat_begin + j].mp;
+    if (mp < 0 || a.pts[mp].bad) return;
+    const unsigned order = (unsigned)((r << 16) | j);
+    if (a.claim[mp] != (((unsigned long long)a.epoch_inv << 32) | order)) return;
+    double pose[7], cc[3];
+#pragma unroll
+    for (int q = 0; q < 7; ++q) pose[q] = a.pose_dev ? a.pose_dev[q] : a.pose[q];
+#pragma unroll
+    for (int q = 0; q < 3; ++q) cc[q] = a.pose_dev ? a.pose_dev[7 + q] : a.center[q];
+    double u, v;
+    store_project(a, pose, a.pts[mp].point_w[0], a.pts[mp].point_w[1], a.pts[mp].point_w[2], u, v);
+    if (!in_image(__double2float_rn(u), __double2float_rn(v), 8, 0, a.width, a.height)) return;      // ref: :58
+    const int slot_out = atomicAdd(a.sel + 17, 1);
+    if (slot_out >= a.cap) return;
     dsdtm_store_cand o;
     o.mp = mp; o.order = (int)order;
-    o.r.px_proj[0] = u; o.r.px_proj[1] = v; o.r.px[0] = u; o.r.px[1] = v;
-    o.r.cell = cell; o.r.obs = best; o.r.flags = flags; o.r.level = -1;
+    o.r = store_candidate_one(a, mp, pose, cc, u, v, slot_out, a.cur_slot);
     a.out[slot_out] = o;
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// The batched chain on the map store (dsdtm_batch_stage_store): every frame of the batch runs UpdateLocalMap + SearchLocalPoints'
+// arithmetic on the key-frame rows [begin, end) of the one store, with the prior pose T_c2r * T_ref of its sparse alignment.
+//   store_batch_prelude_kernel    : one CTA per frame. Pose composition (as store_prelude_kernel), GetCloseKeyFrames over the range
+//                                   (one warp per key frame), the counting rank (ties in row order), then the first-listing-wins walk:
+//                                   every non-bad map point of the local key frames goes into a shared-memory open-addressing table
+//                                   with the smallest order = (rank << 16) | feature index that lists it (atomicMin), and a second
+//                                   pass in order emits the winners that ReprojectPoint puts in the image, compacted block-wide, so
+//                                   record k of a frame is its k-th ReprojectPoint call. No global per-frame state, no epoch, no memset.
+//   store_batch_candidates_kernel : grid (record blocks, frame): store_candidate_one for every emitted record; entries past the
+//                                   frame's count are marked unused for warp_affine / Align2D.
+// Shared memory of the prelude: 9 bytes per key frame of the longest range + 8 bytes per table slot, the table holding at least 4/3 of
+// max_local * the largest feature count of a key frame (store_batch_smem).
+static const int kSbThreads = 256, kSbWarps = kSbThreads / 32;
+
+struct SbArgs {
+    StArgs st;                                           // tables, camera, SolveAffineMatrix inputs (st.cp)
+    const int2* range; int all_end, range_cap;           // per-frame [begin, end); null: [0, all_end)
+    int n_pairs, max_local, cpf, tbits;
+    const double* poses_c2r; const double* poses_ref;    // sparse alignment's T_c2r, reference Frame::Get_Pose
+    const int* cur_slots;
+    double* pose10; int* local; int* n_cand;
+    dsdtm_store_cand* rec;
+};
+
+__global__ void __launch_bounds__(kSbThreads) store_batch_prelude_kernel(const SbArgs b)
+{
+    extern __shared__ __align__(16) unsigned char sb_smem[];
+    __shared__ double s_pose[10];
+    __shared__ int s_sel[16];
+    __shared__ int s_wcnt[kSbWarps];
+    const StArgs& a = b.st;
+    const int f = blockIdx.x, t = threadIdx.x, lane = t & 31, warp = t >> 5;
+    int k0 = 0, k1 = b.all_end;
+    if (b.range) { const int2 r = b.range[f]; k0 = r.x; k1 = r.y; }
+    const int nk = k1 - k0, T = 1 << b.tbits;
+    double* s_dist = reinterpret_cast<double*>(sb_smem);
+    int* s_key = reinterpret_cast<int*>(s_dist + b.range_cap);
+    unsigned* s_val = reinterpret_cast<unsigned*>(s_key + T);
+    uint8_t* s_vis = reinterpret_cast<uint8_t*>(s_val + T);
+    if (t == 0) {
+        double T1[7], Tr[7], Tc[7], inv[7];
+#pragma unroll
+        for (int j = 0; j < 7; ++j) { T1[j] = b.poses_c2r[7 * (size_t)f + j]; Tr[j] = b.poses_ref[7 * (size_t)f + j]; }
+        se3_mul_exact(T1, Tr, Tc);                                                 // ref: src/Sprase_ImageAlign.cpp:57
+        se3_inv_exact(Tc, inv);
+#pragma unroll
+        for (int j = 0; j < 7; ++j) { s_pose[j] = Tc[j]; b.pose10[10 * (size_t)f + j] = Tc[j]; }
+#pragma unroll
+        for (int j = 0; j < 3; ++j) { s_pose[7 + j] = inv[4 + j]; b.pose10[10 * (size_t)f + 7 + j] = inv[4 + j]; }
+    }
+    if (t < 16) s_sel[t] = -1;
+    for (int h = t; h < T; h += kSbThreads) { s_key[h] = -1; s_val[h] = 0xFFFFFFFFu; }
+    __syncthreads();
+    double pose[7];
+#pragma unroll
+    for (int q = 0; q < 7; ++q) pose[q] = s_pose[q];
+    // GetCloseKeyFrames (ref: src/Tracking.cpp:315-345), as store_close_kf_kernel
+    for (int q = warp; q < nk; q += kSbWarps) {
+        const dsdtm_store_kf& kf = a.kfs[k0 + q];
+        bool found = false;
+        for (int base = 0; base < kf.feat_count && !found; base += 32) {
+            const int j = base + lane;
+            bool vis = false;
+            if (j < kf.feat_count) {
+                const int mp = a.feats[kf.feat_begin + j].mp;
+                if (mp >= 0) {
+                    const double P0 = a.pts[mp].point_w[0], P1 = a.pts[mp].point_w[1], P2 = a.pts[mp].point_w[2];
+                    if (!(P0 == 0.0 && P1 == 0.0 && P2 == 0.0)) {
+                        double q0, q1, q2;
+                        qrot_exact(pose, P0, P1, P2, q0, q1, q2);
+                        q0 = __dadd_rn(q0, pose[4]); q1 = __dadd_rn(q1, pose[5]); q2 = __dadd_rn(q2, pose[6]);
+                        if (!(q2 < 0.0)) {
+                            const double u = __dadd_rn(__ddiv_rn(__dmul_rn((double)a.fx, q0), q2), (double)a.cx);
+                            const double v = __dadd_rn(__ddiv_rn(__dmul_rn((double)a.fy, q1), q2), (double)a.cy);
+                            vis = in_image(__double2float_rn(u), __double2float_rn(v), 0, 0, a.width, a.height);
+                        }
+                    }
+                }
+            }
+            found = __any_sync(0xffffffffu, vis);
+        }
+        if (lane == 0) {
+            const double d0 = __dsub_rn(pose[4], kf.pose_c2w[4]), d1 = __dsub_rn(pose[5], kf.pose_c2w[5]), d2 = __dsub_rn(pose[6], kf.pose_c2w[6]);
+            s_vis[q] = found ? 1 : 0;
+            s_dist[q] = found ? sqrt(__dadd_rn(__dadd_rn(__dmul_rn(d0, d0), __dmul_rn(d1, d1)), __dmul_rn(d2, d2))) : 0.0;
+        }
+    }
+    __syncthreads();
+    // UpdateLocalMap's ranking (ref: :266-277): rank = visible (distance, row) pairs below this one's
+    for (int q = t; q < nk; q += kSbThreads) {
+        if (!s_vis[q]) continue;
+        const double d = s_dist[q];
+        int rank = 0;
+        for (int j = 0; j < nk; ++j)
+            if (s_vis[j] && (s_dist[j] < d || (s_dist[j] == d && j < q))) ++rank;
+        if (rank < b.max_local) s_sel[rank] = k0 + q;
+    }
+    __syncthreads();
+    int n_sel = 0;                                       // the ranks of the visible key frames are 0 .. n_visible - 1
+    while (n_sel < b.max_local && s_sel[n_sel] >= 0) ++n_sel;
+    if (t < 17) b.local[17 * (size_t)f + t] = t == 0 ? n_sel : (t - 1 < n_sel ? s_sel[t - 1] : -1);
+    // every map point of the local key frames once: the smallest order that lists it (ref: :283-297, mLastProjectedFrameId)
+    const unsigned hshift = 32u - (unsigned)b.tbits;
+    for (int r = 0; r < n_sel; ++r) {
+        const dsdtm_store_kf& kf = a.kfs[s_sel[r]];
+        for (int j = t; j < kf.feat_count; j += kSbThreads) {
+            const int mp = a.feats[kf.feat_begin + j].mp;
+            if (mp < 0 || a.pts[mp].bad) continue;                                  // ref: :287-291
+            unsigned h = ((unsigned)mp * 0x9E3779B1u) >> hshift;
+            for (;;) {
+                const int prev = atomicCAS(s_key + h, -1, mp);
+                if (prev == -1 || prev == mp) { atomicMin(s_val + h, (unsigned)((r << 16) | j)); break; }
+                h = (h + 1) & (unsigned)(T - 1);
+            }
+        }
+    }
+    __syncthreads();
+    // the winners in order; ReprojectPoint (ref: :54-69) keeps those inside the image
+    int base = 0;
+    dsdtm_store_cand* R = b.rec + (size_t)f * b.cpf;
+    for (int r = 0; r < n_sel; ++r) {
+        const dsdtm_store_kf& kf = a.kfs[s_sel[r]];
+        for (int j0 = 0; j0 < kf.feat_count; j0 += kSbThreads) {
+            const int j = j0 + t;
+            const unsigned order = (unsigned)((r << 16) | j);
+            int mp = -1;
+            bool win = false;
+            if (j < kf.feat_count) {
+                mp = a.feats[kf.feat_begin + j].mp;
+                if (mp >= 0 && !a.pts[mp].bad) {
+                    unsigned h = ((unsigned)mp * 0x9E3779B1u) >> hshift;
+                    while (s_key[h] != mp) h = (h + 1) & (unsigned)(T - 1);
+                    if (s_val[h] == order) {
+                        double u, v;
+                        store_project(a, pose, a.pts[mp].point_w[0], a.pts[mp].point_w[1], a.pts[mp].point_w[2], u, v);
+                        win = in_image(__double2float_rn(u), __double2float_rn(v), 8, 0, a.width, a.height);
+                    }
+                }
+            }
+            const unsigned bal = __ballot_sync(0xffffffffu, win);
+            if (lane == 0) s_wcnt[warp] = __popc(bal);
+            __syncthreads();
+            int off = 0, tot = 0;
+#pragma unroll
+            for (int w = 0; w < kSbWarps; ++w) { const int c = s_wcnt[w]; off += w < warp ? c : 0; tot += c; }
+            if (win) {
+                const int pos = base + off + __popc(bal & ((1u << lane) - 1u));
+                if (pos < b.cpf) { R[pos].mp = mp; R[pos].order = (int)order; }
+            }
+            base += tot;
+            __syncthreads();
+        }
+    }
+    if (t == 0) b.n_cand[f] = base;
+}
+
+__global__ void __launch_bounds__(128) store_batch_candidates_kernel(const SbArgs b)
+{
+    const int f = blockIdx.y, k = blockIdx.x * blockDim.x + threadIdx.x;
+    if (k >= b.cpf) return;
+    const StArgs& a = b.st;
+    const int n = min(b.n_cand[f], b.cpf);
+    const int i = f * b.cpf + k;
+    const int cur_slot = b.cur_slots[f];
+    if (k >= n) {                                        // unused entry: warp_affine and Align2D skip it
+        dsdtm_candidate cd;
+        cd.ref_slot = -1; cd.ref_level = 0; cd.px[0] = 0.0; cd.px[1] = 0.0;
+        candidate_prep_one(a.cp, i, cd, cur_slot);
+        return;
+    }
+    double pose[7], cc[3];
+#pragma unroll
+    for (int q = 0; q < 7; ++q) pose[q] = b.pose10[10 * (size_t)f + q];
+#pragma unroll
+    for (int q = 0; q < 3; ++q) cc[q] = b.pose10[10 * (size_t)f + 7 + q];
+    dsdtm_store_cand o = b.rec[i];
+    double u, v;
+    store_project(a, pose, a.pts[o.mp].point_w[0], a.pts[o.mp].point_w[1], a.pts[o.mp].point_w[2], u, v);
+    o.r = store_candidate_one(a, o.mp, pose, cc, u, v, i, cur_slot);
+    b.rec[i] = o;
+}
+
+// slots of the prelude's table for max_local key frames of the store's widest feature count
+int store_batch_tbits(const dsdtm_ctx* c, int max_local)
+{
+    const long long n = (long long)max_local * std::max(c->st_max_feats, 1);
+    int bits = 6;
+    while ((1ll << bits) * 3 < n * 4) ++bits;
+    return bits;
 }
 
 StArgs store_args(dsdtm_ctx* c)
@@ -697,5 +905,35 @@ cudaError_t launch_store_track(dsdtm_ctx* c, const StoreTrackArgs& t, cudaStream
 }
 
 const int* store_count_dev(dsdtm_ctx* c) { return c->st_sel_d + 17; }
+
+size_t store_batch_smem(const dsdtm_ctx* c, int range_len, int max_local)
+{
+    const size_t cap = (size_t)((std::max(range_len, 1) + 1) & ~1);          // keeps the int table 8-byte aligned after the doubles
+    return cap * sizeof(double) + ((size_t)8 << store_batch_tbits(c, max_local)) + cap;
+}
+
+cudaError_t store_batch_init(dsdtm_ctx* c)
+{
+    int max_smem = 0;
+    cudaError_t e = cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, c->device);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(store_batch_prelude_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem - 1024);
+    return e;
+}
+
+cudaError_t launch_store_batch(dsdtm_ctx* c, int n_pairs, bool all_rows, int range_len, int max_local, int cpf, int max_search_level, cudaStream_t s)
+{
+    SbArgs b;
+    b.st = store_args(c);
+    b.st.cp.n = n_pairs * cpf; b.st.cp.max_search_level = max_search_level;
+    b.range = all_rows ? nullptr : c->sb_range_d; b.all_end = (int)c->st_kfs_n;
+    b.range_cap = (std::max(range_len, 1) + 1) & ~1;
+    b.n_pairs = n_pairs; b.max_local = max_local; b.cpf = cpf; b.tbits = store_batch_tbits(c, max_local);
+    b.poses_c2r = c->poses_out_d; b.poses_ref = c->poses_ref_d; b.cur_slots = c->cur_slots_d;
+    b.pose10 = c->sb_pose10_d; b.local = c->sb_local_d; b.n_cand = c->sb_ncand_d; b.rec = c->sb_rec_d;
+    store_batch_prelude_kernel<<<n_pairs, kSbThreads, store_batch_smem(c, range_len, max_local), s>>>(b);
+    store_batch_candidates_kernel<<<dim3((unsigned)((cpf + 127) / 128), (unsigned)n_pairs), 128, 0, s>>>(b);
+    c->launches += 2;
+    return cudaGetLastError();
+}
 
 }  // namespace dsdtm

@@ -32,6 +32,8 @@ struct SelArgs {
     const dsdtm_reproj* rec; const int* found; const dsdtm_ref_feat* feats; int feat_stride;
     const double* poses_c2r; const double* poses_ref;
     int n_pairs, ppp, per_warp;                   // per_warp = 8-byte words of shared memory per warp
+    // store mode: records sb_rec (ppp per frame, the first n_cand valid, in order), found per store point row, points from the store
+    const dsdtm_store_cand* srec; const int* n_cand; const dsdtm_store_point* pts; int n_found; const double* pose10; int jbits;
     float fx, fy, cx, cy;
     int radius; int span[kMaxRadius + 1];
     dsdtm_match* match; dsdtm_ba_obs* obs; int* n_match; double* pose_in;
@@ -43,6 +45,9 @@ __device__ __forceinline__ bool in_circle(int x, int y, int cx, int cy, int r, c
     return dy <= r && dx <= span[dy];
 }
 
+// kStore: the records are the store-backed chain's (dsdtm_batch_stage_store): j is the record index, which is the order of ReprojectPoint;
+// found comes from the point's row, the match names the store point, and a frame whose candidates overflowed its rows gets n_match -1
+template <bool kStore>
 __global__ void __launch_bounds__(kSelWarps * 32) track_select_kernel(const SelArgs a)
 {
     extern __shared__ unsigned long long sel_smem[];
@@ -56,20 +61,29 @@ __global__ void __launch_bounds__(kSelWarps * 32) track_select_kernel(const SelA
     int2* circ = reinterpret_cast<int2*>(key + a.ppp);
     int* order = reinterpret_cast<int*>(circ + kCap);
     const dsdtm_reproj* R = a.rec + (size_t)pair * a.ppp;
+    const dsdtm_store_cand* SR = a.srec + (size_t)pair * a.ppp;
     const int* F = a.found + (size_t)pair * a.ppp;
+    const int jb = kStore ? a.jbits : 10;
+    int n_rec = a.ppp;
+    bool overflow = false;
+    if (kStore) { const int nc = a.n_cand[pair]; overflow = nc > a.ppp; n_rec = overflow ? 0 : nc; }
 
     // 1. compaction in j order
     int n = 0;
-    for (int j0 = 0; j0 < a.ppp; j0 += 32) {
+    for (int j0 = 0; j0 < n_rec; j0 += 32) {
         const int j = j0 + lane;
         bool ok = false;
         unsigned long long k = 0;
-        if (j < a.ppp) {
+        if (j < n_rec) {
+            const dsdtm_reproj& rj = kStore ? SR[j].r : R[j];
             const int need = DSDTM_LM_OBS_OK | DSDTM_LM_REF_OK | DSDTM_LM_CONVERGED;
-            const int cell = R[j].cell;
-            ok = cell >= 0 && (R[j].flags & need) == need && R[j].level >= 0;
-            const unsigned fdesc = ~((unsigned)F[j] ^ 0x80000000u);          // found descending as an unsigned ascending key
-            k = ((unsigned long long)(unsigned)cell << 42) | ((unsigned long long)fdesc << 10) | (unsigned)j;
+            const int cell = rj.cell;
+            ok = cell >= 0 && (rj.flags & need) == need && rj.level >= 0;
+            int fc = 1;                                                     // a point appended after staging: MapPoint::mnFound starts at 1
+            if (!kStore) fc = F[j];
+            else if (SR[j].mp < a.n_found) fc = a.found[SR[j].mp];
+            const unsigned fdesc = ~((unsigned)fc ^ 0x80000000u);           // found descending as an unsigned ascending key
+            k = ((unsigned long long)(unsigned)cell << (32 + jb)) | ((unsigned long long)fdesc << jb) | (unsigned)j;
         }
         const unsigned b = __ballot_sync(0xffffffffu, ok);
         if (ok) key[n + __popc(b & ((1u << lane) - 1u))] = k;
@@ -81,7 +95,7 @@ __global__ void __launch_bounds__(kSelWarps * 32) track_select_kernel(const SelA
         const unsigned long long k = key[e];
         int rank = 0;
         for (int q = 0; q < n; ++q) rank += key[q] < k ? 1 : 0;
-        order[rank] = (int)(k & 1023u);
+        order[rank] = (int)(k & ((1u << jb) - 1u));
     }
     __syncwarp();
     // 3. the greedy walk
@@ -94,7 +108,7 @@ __global__ void __launch_bounds__(kSelWarps * 32) track_select_kernel(const SelA
         float p0 = 0.f, p1 = 0.f;
         if (alive) {
             j = order[e];
-            const dsdtm_reproj& r = R[j];
+            const dsdtm_reproj& r = kStore ? SR[j].r : R[j];
             cell = r.cell; level = r.level;
             x = __float2int_rn(__double2float_rn(r.px_proj[0])); y = __float2int_rn(__double2float_rn(r.px_proj[1]));   // Mat::at(cvRound)
             p0 = __double2float_rn(r.px[0]); p1 = __double2float_rn(r.px[1]);                                             // Point2f(px)
@@ -109,7 +123,7 @@ __global__ void __launch_bounds__(kSelWarps * 32) track_select_kernel(const SelA
             const int wcell = __shfl_sync(0xffffffffu, cell, w), wx = __shfl_sync(0xffffffffu, mx, w), wy = __shfl_sync(0xffffffffu, my, w);
             if (lane == w) {
                 circ[n_match] = make_int2(mx, my);
-                dsdtm_match m; m.point = j; m.px[0] = p0; m.px[1] = p1; m.level = level;
+                dsdtm_match m; m.point = kStore ? SR[j].mp : j; m.px[0] = p0; m.px[1] = p1; m.level = level;
                 M[n_match] = m;
             }
             ++n_match; won_cell = wcell;
@@ -126,11 +140,15 @@ __global__ void __launch_bounds__(kSelWarps * 32) track_select_kernel(const SelA
         dsdtm_ba_obs o;
         feature_normal_exact(mt.px[0], mt.px[1], a.fx, a.fy, a.cx, a.cy, o.normal);                   // ref: src/Frame.cpp:83-92
 #pragma unroll
-        for (int k = 0; k < 3; ++k) o.point_w[k] = Fe[mt.point].point_w[k];
+        for (int k = 0; k < 3; ++k) o.point_w[k] = kStore ? a.pts[mt.point].point_w[k] : Fe[mt.point].point_w[k];
         o.level = mt.level; o.reserved = 0;
         O[m] = o;
     }
-    if (lane == 0) {
+    if (kStore && lane == 0) {
+        a.n_match[pair] = overflow ? -1 : n_match;
+#pragma unroll
+        for (int k = 0; k < 7; ++k) a.pose_in[7 * (size_t)pair + k] = a.pose10[10 * (size_t)pair + k];   // composed by the prelude
+    } else if (lane == 0) {
         a.n_match[pair] = n_match;
         double Tc2r[7], Tr[7], pc[7];
 #pragma unroll
@@ -141,20 +159,27 @@ __global__ void __launch_bounds__(kSelWarps * 32) track_select_kernel(const SelA
     }
 }
 
-}  // namespace
+// bits of an index below n (at least 1)
+int index_bits(int n)
+{
+    int b = 1;
+    while ((1 << b) < n) ++b;
+    return b;
+}
 
-cudaError_t launch_track_select(dsdtm_ctx* c, int n_pairs, int feat_stride, int ppp, cudaStream_t s)
+SelArgs select_args(dsdtm_ctx* c, int n_pairs, int ppp)
 {
     SelArgs a;
-    a.rec = c->pair_reproj_d; a.found = c->trk_found_d; a.feats = c->feats_d; a.feat_stride = feat_stride;
+    a.rec = c->pair_reproj_d; a.found = c->trk_found_d; a.feats = c->feats_d; a.feat_stride = 0;
     a.poses_c2r = c->poses_out_d; a.poses_ref = c->poses_ref_d;
+    a.srec = nullptr; a.n_cand = nullptr; a.pts = nullptr; a.n_found = 0; a.pose10 = nullptr; a.jbits = 10;
     a.n_pairs = n_pairs; a.ppp = ppp;
     a.per_warp = ppp + kCap + (ppp + 1) / 2;      // keys, circle centres, order
     a.fx = c->cam.fx; a.fy = c->cam.fy; a.cx = c->cam.cx; a.cy = c->cam.cy;
     // row half-widths of cv::circle(img, c, r, color, -1) (OpenCV drawing.cpp, the filled midpoint circle)
     const int r = c->prm.cell_size;
-    if (r < 0 || r > kMaxRadius) return cudaErrorInvalidValue;
-    a.radius = r;
+    a.radius = (r < 0 || r > kMaxRadius) ? -1 : r;       // refused by the launchers
+    if (a.radius < 0) return a;
     for (int k = 0; k <= kMaxRadius; ++k) a.span[k] = -1;
     {
         int err = 0, dx = r, dy = 0, plus = 1, minus = (r << 1) - 1;
@@ -171,10 +196,43 @@ cudaError_t launch_track_select(dsdtm_ctx* c, int n_pairs, int feat_stride, int 
         }
     }
     a.match = c->trk_match_d; a.obs = c->trk_obs_d; a.n_match = c->trk_nobs_d; a.pose_in = c->trk_pose_in_d;
-    const size_t smem = (size_t)kSelWarps * a.per_warp * sizeof(unsigned long long);
-    track_select_kernel<<<(n_pairs + kSelWarps - 1) / kSelWarps, kSelWarps * 32, smem, s>>>(a);
+    return a;
+}
+
+}  // namespace
+
+size_t track_select_smem(int ppp) { return (size_t)kSelWarps * (ppp + kCap + (ppp + 1) / 2) * sizeof(unsigned long long); }
+
+cudaError_t launch_track_select(dsdtm_ctx* c, int n_pairs, int feat_stride, int ppp, cudaStream_t s)
+{
+    SelArgs a = select_args(c, n_pairs, ppp);
+    a.feat_stride = feat_stride;
+    if (a.radius < 0) return cudaErrorInvalidValue;
+    track_select_kernel<false><<<(n_pairs + kSelWarps - 1) / kSelWarps, kSelWarps * 32, track_select_smem(ppp), s>>>(a);
     c->launches++;
     return cudaGetLastError();
+}
+
+cudaError_t launch_track_select_store(dsdtm_ctx* c, int n_pairs, int cpf, int n_found, cudaStream_t s)
+{
+    SelArgs a = select_args(c, n_pairs, cpf);
+    if (a.radius < 0) return cudaErrorInvalidValue;
+    a.srec = c->sb_rec_d; a.n_cand = c->sb_ncand_d; a.pts = c->st_pts_d; a.pose10 = c->sb_pose10_d;
+    a.found = c->sb_found_d; a.n_found = n_found;
+    a.jbits = index_bits(cpf);
+    track_select_kernel<true><<<(n_pairs + kSelWarps - 1) / kSelWarps, kSelWarps * 32, track_select_smem(cpf), s>>>(a);
+    c->launches++;
+    return cudaGetLastError();
+}
+
+int track_select_key_bits(const dsdtm_ctx* c, int ppp) { return index_bits(c->n_cells) + 32 + index_bits(ppp); }
+
+cudaError_t track_select_init(dsdtm_ctx* c)
+{
+    int max_smem = 0;
+    cudaError_t e = cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, c->device);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(track_select_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, max_smem - 1024);
+    return e;
 }
 
 int track_select_max_radius() { return kMaxRadius; }

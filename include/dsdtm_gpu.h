@@ -554,6 +554,36 @@ int dsdtm_batch_stage_keyframe(dsdtm_ctx* ctx, const int32_t* depth_slots /* n_p
 /* after dsdtm_batch_run(flags | 8): n_new = n_pairs corner counts; corners and lifted = n_pairs x max_fts (Add_Feature order, rows past
  * n_new[i] zero); exact_path = n_pairs flags as in dsdtm_detect_batch. Every pointer may be NULL. */
 int dsdtm_batch_fetch_keyframe(dsdtm_ctx* ctx, int32_t* n_new, dsdtm_corner* corners, dsdtm_lifted* lifted, uint8_t* exact_path);
+/* The store-backed local map of the batched chain: instead of dsdtm_batch_stage_map's one-key-frame stand-in, every frame of the batch
+ * runs Tracking::UpdateLocalMap on the context's map store (dsdtm_store_*), as dsdtm_store_track does for one frame (ref:
+ * src/Tracking.cpp:219-345). After dsdtm_batch_stage, stage either dsdtm_batch_stage_map or this; flags bits 1, 2 and 3 then run on
+ * whichever is staged, and staging one drops the other (dsdtm_batch_stage drops both). Per frame i, with the prior pose T_c2r * T_ref
+ * (the sparse alignment's result times poses_ref_c2w[i], ref: src/Sprase_ImageAlign.cpp:57), on the key-frame rows [kf_range[2i],
+ * kf_range[2i+1]) (kf_range NULL: every row of the store at the time of the run):
+ *   GetCloseKeyFrames and UpdateLocalMap's ranking: the max_local nearest, stable in row order;
+ *   every map point of those key frames once, the first key frame in rank order that lists it winning, bad points skipped;
+ *   ReprojectPoint, Get_ClosetObs over the point's whole observation chain, the IsInImage gate, SolveAffineMatrix, GetBestSearchLevel,
+ *   WarpAffine and Align2DGaussNewton
+ * -- each with the semantics dsdtm_store_track documents. Frame i's records fill rows [i * cands_per_frame, ..) IN `order` (UpdateLocalMap's
+ * ReprojectPoint order). A frame with more candidates than cands_per_frame keeps its first cands_per_frame records, gets n_matches -1 and
+ * its prior pose from dsdtm_batch_fetch_track, and no key frame (flags bit 3); the other frames are unaffected.
+ * Behind the chain (flags | 4), dsdtm_batch_stage_track's `found` has one entry per store point row at its call, shared by all frames
+ * (NULL = all 1; rows appended later count 1); a dsdtm_match's `point` is the store point row and its dsdtm_ba_obs point is that
+ * row's point_w; the selection sorts a cell's records by found count, descending, then by `order`. dsdtm_batch_stage_keyframe works on
+ * top unchanged. Any store change (dsdtm_store_set_points / _update_points / _append_keyframe / _set_keyframe / _clear) drops the
+ * captured steps, so the next dsdtm_batch_run runs on the changed map; the run returns DSDTM_E_STATE when the store no longer holds the
+ * staged ranges. DSDTM_E_ARG, with nothing enqueued, for a range outside the store, max_local outside 1..16, cands_per_frame outside
+ * 1..max_patches, an empty store, or a range length and local map whose prelude does not fit one CTA's shared memory (9 bytes per key
+ * frame of the longest range + 32 bytes per 3 features of max_local * the largest key frame, rounded up to a power of two; about 20 k
+ * key frames of 300 features). LIMIT: a range longer than that is refused, not split over CTAs; with kf_range NULL a store that grows
+ * past it makes the next dsdtm_batch_run return DSDTM_E_ARG. DSDTM_E_STATE without dsdtm_batch_stage. Device time: the prelude and the candidates under
+ * DSDTM_STAGE_LOCAL_MAP. */
+int dsdtm_batch_stage_store(dsdtm_ctx* ctx, const double* poses_ref_c2w /* n_pairs x 7 */, const int32_t* kf_range /* n_pairs x 2 or NULL */,
+                            int max_local, int max_search_level, int align_iters, int cands_per_frame);
+/* after dsdtm_batch_run(flags | 2) in store mode: local_rows = n_pairs x 16 (the local key frames' store rows in rank order, -1 past
+ * n_local[i]); cands = n_pairs x cands_per_frame records in `order` (rows past min(n_cand[i], cands_per_frame) zero); n_cand = the true
+ * candidate count, which may exceed cands_per_frame. Every pointer may be NULL. */
+int dsdtm_batch_fetch_store(dsdtm_ctx* ctx, int32_t* local_rows, int32_t* n_local, dsdtm_store_cand* cands, int32_t* n_cand);
 int dsdtm_batch_fetch(dsdtm_ctx* ctx, double* poses_out, int* n_tracked, double* patch_px_out, uint8_t* patch_conv);
 /* end-to-end step with HOST buffers: uploads the n_pairs cur images (dense, pinned recommended) into their cur slots,
  * stages the per-pair inputs, runs, and fetches -- copies overlapped with compute in chunks on internal streams. Both e2e entries
