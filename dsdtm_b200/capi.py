@@ -96,6 +96,7 @@ SYMBOLS = [
     "dsdtm_pose_optimize", "dsdtm_pose_optimize_batch", "dsdtm_map_table_upload", "dsdtm_close_keyframes", "dsdtm_probe_fp64", "dsdtm_frame_upload_pyramid_async", "dsdtm_track_frame_store", "dsdtm_store_set_points", "dsdtm_store_update_points", "dsdtm_store_append_keyframe", "dsdtm_store_set_keyframe", "dsdtm_store_clear", "dsdtm_store_track", "dsdtm_frame_upload_level", "dsdtm_batch_stage_map", "dsdtm_batch_fetch_map", "dsdtm_track_batch_e2e",
     "dsdtm_batch_stage_track", "dsdtm_batch_fetch_track", "dsdtm_detect", "dsdtm_detect_batch",
     "dsdtm_batch_stage_keyframe", "dsdtm_batch_fetch_keyframe", "dsdtm_batch_stage_store", "dsdtm_batch_fetch_store",
+    "dsdtm_store_set_found", "dsdtm_store_size", "dsdtm_store_fetch", "dsdtm_batch_stage_track_live", "dsdtm_batch_commit_store",
 ]
 
 
@@ -486,6 +487,27 @@ class Context:
         self._ck(self.L.dsdtm_store_set_keyframe(self.hp, int(row), int(slot), _p(np.ascontiguousarray(pose_c2w, np.float64)),
                                                   _p(np.ascontiguousarray(center, np.float64))))
 
+    def store_set_found(self, ids, found):
+        """dsdtm_store_set_found: MapPoint::mnFound of the point rows ids (appended points start at 1)"""
+        ids = np.ascontiguousarray(ids, np.int32).reshape(-1)
+        f = np.ascontiguousarray(found, np.int32).reshape(len(ids))
+        self._ck(self.L.dsdtm_store_set_found(self.hp, _p(ids), len(ids), _p(f)))
+
+    def store_size(self):
+        """-> (key frames, features, points): the rows of the store's tables"""
+        k, f, p = C.c_int32(0), C.c_int32(0), C.c_int32(0)
+        self._ck(self.L.dsdtm_store_size(self.hp, C.byref(k), C.byref(f), C.byref(p)))
+        return k.value, f.value, p.value
+
+    def store_fetch(self, kfs=None, feats=None, points=None):
+        """dsdtm_store_fetch: kfs / feats / points = (first, n) row ranges, None = the whole table. Returns (STORE_KF_DT, STORE_FEAT_DT,
+        STORE_POINT_DT, found int32) as the library holds them: is_obs = observing key-frame row + 1, next_obs / last_obs the chains."""
+        nk, nf, npt = self.store_size()
+        (k0, kn), (f0, fn), (p0, pn) = kfs or (0, nk), feats or (0, nf), points or (0, npt)
+        K = np.zeros(kn, STORE_KF_DT); F = np.zeros(fn, STORE_FEAT_DT); P = np.zeros(pn, STORE_POINT_DT); fd = np.zeros(pn, np.int32)
+        self._ck(self.L.dsdtm_store_fetch(self.hp, int(k0), int(kn), _p(K), int(f0), int(fn), _p(F), int(p0), int(pn), _p(P), _p(fd)))
+        return K, F, P, fd
+
     def store_track(self, cur_slot, pose_cur_c2w, cur_center, max_local=10, max_search_level=2, align_iters=10, cap=4096):
         """dsdtm_store_track -> (local key-frame rows in rank order, STORE_CAND_DT records in arrival order). More than cap candidates
         raises."""
@@ -546,6 +568,21 @@ class Context:
         elif f is not None and len(f) != self.store_points:     # store mode: one count per store point row
             raise DsdtmError("batch_stage_track: found has %d entries, the map store %d points" % (len(f), self.store_points))
         self._ck(self.L.dsdtm_batch_stage_track(self.hp, _p(f), int(max_iters)))
+
+    def batch_stage_track_live(self, max_iters=100):
+        """after batch_stage_store: as batch_stage_track, but the selection reads the store's own found counts at every run"""
+        self._ck(self.L.dsdtm_batch_stage_track_live(self.hp, int(max_iters)))
+
+    def batch_commit_store(self, outlier_threshold, kf_rows=None):
+        """dsdtm_batch_commit_store after a store-mode batch_run(7 or 15): found counts, bad flags and (flags 15) the key frames of the
+        wanted frames into the store. kf_rows = (n_pairs,) reserved empty key-frame rows or None (append). Returns (kf_row, point_first,
+        n_points) per frame and updates store_points / store_keyframes."""
+        n = self._n
+        kr = None if kf_rows is None else np.ascontiguousarray(kf_rows, np.int32).reshape(n)
+        row = np.empty(n, np.int32); pf = np.empty(n, np.int32); npt = np.empty(n, np.int32)
+        self._ck(self.L.dsdtm_batch_commit_store(self.hp, C.c_float(outlier_threshold), _p(kr), _p(row), _p(pf), _p(npt)))
+        self.store_keyframes, _, self.store_points = self.store_size()
+        return row, pf, npt
 
     def batch_fetch_track(self):
         """-> (poses c2w after PoseOptimization (n, 7), n_matches (n,), matches (n, 200) MATCH_DT, res_norm (n, 200), summaries (n,)

@@ -1,6 +1,7 @@
 // capi.cu -- the extern "C" boundary (include/dsdtm_gpu.h): context, HBM pools, staging, launches, CUDA-graph replay.
 // No compute happens on the host here; if the CUDA device / kernels are unavailable every entry point fails loudly.
 #include <algorithm>
+#include <cmath>
 #include <cstring>
 #include <vector>
 
@@ -336,7 +337,8 @@ void dsdtm_destroy(dsdtm_ctx* c)
                      c->trk_found_d, c->trk_match_d, c->trk_obs_d, c->trk_nobs_d, c->trk_pose_in_d, c->trk_pose_out_d, c->trk_res_d, c->trk_sum_d,
                      c->det_mask_d, c->det_buf_d, c->kf_circ_d, c->kf_ncirc_d, c->kf_max_new_d, c->kf_corner_d, c->kf_lifted_d, c->kf_nnew_d,
                      c->kf_exact_d, c->kf_depth_slot_d, c->kf_want_d, c->kf_rows_d,
-                     c->sb_rec_d, c->sb_ncand_d, c->sb_local_d, c->sb_pose10_d, c->sb_range_d, c->sb_found_d };
+                     c->sb_rec_d, c->sb_ncand_d, c->sb_local_d, c->sb_pose10_d, c->sb_range_d, c->sb_found_d,
+                     c->st_found_d, c->cm_d, c->cm_push_d };
     for (void* p : bufs) if (p) cudaFree(p);
     if (c->pinned) cudaFreeHost(c->pinned);
     if (c->stage_pin) cudaFreeHost(c->stage_pin);
@@ -1247,6 +1249,8 @@ int dsdtm_store_clear(dsdtm_ctx* c)
     if (!c) return DSDTM_E_ARG;
     c->st_kfs_n = c->st_feats_n = c->st_pts_n = 0;
     c->st_max_feats = 0;
+    c->st_kf_nfeat.clear();
+    c->batch.commit_flags = 0;                   // the step's matches name rows that are gone
     drop_store_graphs(c);
     return 0;
 }
@@ -1260,7 +1264,8 @@ int dsdtm_store_set_points(dsdtm_ctx* c, int first, int n, const double* point_w
     drop_store_graphs(c);
     const size_t end = (size_t)first + n, old_n = c->st_pts_n;
     const size_t old_claim_cap = c->st_claim_cap;
-    if (grow_keep(c, &c->st_pts_d, &c->st_pts_cap, end, old_n) || grow_keep(c, &c->st_claim_d, &c->st_claim_cap, end, old_n)) return DSDTM_E_NOMEM;
+    if (grow_keep(c, &c->st_pts_d, &c->st_pts_cap, end, old_n) || grow_keep(c, &c->st_claim_d, &c->st_claim_cap, end, old_n) ||
+        grow_keep(c, &c->st_found_d, &c->st_found_cap, end, old_n)) return DSDTM_E_NOMEM;
     cudaStream_t s = c->stream;
     if (c->st_claim_cap != old_claim_cap)     // fresh part of the claim array: "never claimed"
         DSDTM_CUDA(c, cudaMemsetAsync(c->st_claim_d + old_n, 0xFF, (c->st_claim_cap - old_n) * sizeof(unsigned long long), s));
@@ -1279,6 +1284,8 @@ int dsdtm_store_set_points(dsdtm_ctx* c, int first, int n, const double* point_w
         rows[(size_t)i].last_obs = last[(size_t)i];
     }
     DSDTM_CUDA(c, cudaMemcpyAsync(c->st_pts_d + first, rows.data(), (size_t)n * sizeof(dsdtm_store_point), cudaMemcpyHostToDevice, s));
+    const std::vector<int32_t> ones(end > old_n ? end - old_n : 0, 1);                            // MapPoint::mnFound starts at 1
+    if (!ones.empty()) DSDTM_CUDA(c, cudaMemcpyAsync(c->st_found_d + old_n, ones.data(), ones.size() * sizeof(int32_t), cudaMemcpyHostToDevice, s));
     DSDTM_CUDA(c, cudaStreamSynchronize(s));
     c->st_pts_n = std::max(old_n, end);
     return 0;
@@ -1347,6 +1354,7 @@ int dsdtm_store_append_keyframe(dsdtm_ctx* c, const dsdtm_store_kf* kf, const ds
     if (n_feats) DSDTM_CUDA(c, cudaMemcpyAsync(c->st_feats_d + f0, fs.data(), (size_t)n_feats * sizeof(dsdtm_store_feat), cudaMemcpyHostToDevice, s));
     c->st_kfs_n = r + 1; c->st_feats_n = f0 + n_feats;
     c->st_max_feats = std::max(c->st_max_feats, n_feats);
+    c->st_kf_nfeat.push_back(n_feats);
     DSDTM_CUDA(c, launch_store_link(c, (int)f0, n_feats, s));
     DSDTM_CUDA(c, cudaStreamSynchronize(s));
     if (row) *row = (int32_t)r;
@@ -1367,6 +1375,63 @@ int dsdtm_store_set_keyframe(dsdtm_ctx* c, int row, int slot, const double pose_
     for (int i = 0; i < 7; ++i) k.pose_c2w[i] = pose_c2w[i];
     for (int i = 0; i < 3; ++i) k.center[i] = center[i];
     DSDTM_CUDA(c, cudaMemcpyAsync(c->st_kfs_d + row, &k, sizeof k, cudaMemcpyHostToDevice, s));
+    DSDTM_CUDA(c, cudaStreamSynchronize(s));
+    return 0;
+}
+
+namespace {
+__global__ void store_set_found_kernel(int* found, const int32_t* ids, int n, const int32_t* v)
+{
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) found[ids[i]] = v[i];
+}
+}  // namespace
+
+int dsdtm_store_set_found(dsdtm_ctx* c, const int32_t* ids, int n, const int32_t* found)
+{
+    if (!c) return DSDTM_E_ARG;
+    if (n < 0 || (n && (!ids || !found))) return fail(c, DSDTM_E_ARG, "dsdtm_store_set_found: null ids / counts");
+    if (n == 0) return 0;
+    for (int i = 0; i < n; ++i) if (ids[i] < 0 || (size_t)ids[i] >= c->st_pts_n) return fail(c, DSDTM_E_ARG, "dsdtm_store_set_found: id outside the point table");
+    drop_store_graphs(c);
+    const int chunk = 65536;                                     // 2 x 256 KB fits the 1 MB staging mirror
+    cudaStream_t s = c->stream;
+    for (int i0 = 0; i0 < n; i0 += chunk) {
+        const int m = std::min(chunk, n - i0);
+        const size_t nb = (size_t)m * sizeof(int32_t);
+        std::memcpy(c->stage_pin, ids + i0, nb);
+        std::memcpy(c->stage_pin + nb, found + i0, nb);
+        DSDTM_CUDA(c, cudaMemcpyAsync(c->stage_dev, c->stage_pin, 2 * nb, cudaMemcpyHostToDevice, s));
+        const int32_t* ids_d = reinterpret_cast<const int32_t*>(c->stage_dev);
+        store_set_found_kernel<<<(m + 127) / 128, 128, 0, s>>>(c->st_found_d, ids_d, m, ids_d + m);
+        c->launches++;
+        DSDTM_CUDA(c, cudaGetLastError());
+        DSDTM_CUDA(c, cudaStreamSynchronize(s));                 // the staging arena is reused by the next chunk / call
+    }
+    return 0;
+}
+
+int dsdtm_store_size(const dsdtm_ctx* c, int32_t* n_kfs, int32_t* n_feats, int32_t* n_points)
+{
+    if (!c) return DSDTM_E_ARG;
+    if (n_kfs) *n_kfs = (int32_t)c->st_kfs_n;
+    if (n_feats) *n_feats = (int32_t)c->st_feats_n;
+    if (n_points) *n_points = (int32_t)c->st_pts_n;
+    return 0;
+}
+
+int dsdtm_store_fetch(dsdtm_ctx* c, int kf_first, int n_kfs, dsdtm_store_kf* kfs, int feat_first, int n_feats, dsdtm_store_feat* feats,
+                      int point_first, int n_points, dsdtm_store_point* points, int32_t* found)
+{
+    if (!c) return DSDTM_E_ARG;
+    auto bad_range = [](int first, int n, size_t size) { return first < 0 || n < 0 || (size_t)first + (size_t)n > size; };
+    if (bad_range(kf_first, n_kfs, c->st_kfs_n) || bad_range(feat_first, n_feats, c->st_feats_n) || bad_range(point_first, n_points, c->st_pts_n))
+        return fail(c, DSDTM_E_ARG, "dsdtm_store_fetch: range outside the store");
+    cudaStream_t s = c->stream;
+    if (kfs && n_kfs) DSDTM_CUDA(c, cudaMemcpyAsync(kfs, c->st_kfs_d + kf_first, (size_t)n_kfs * sizeof(dsdtm_store_kf), cudaMemcpyDeviceToHost, s));
+    if (feats && n_feats) DSDTM_CUDA(c, cudaMemcpyAsync(feats, c->st_feats_d + feat_first, (size_t)n_feats * sizeof(dsdtm_store_feat), cudaMemcpyDeviceToHost, s));
+    if (points && n_points) DSDTM_CUDA(c, cudaMemcpyAsync(points, c->st_pts_d + point_first, (size_t)n_points * sizeof(dsdtm_store_point), cudaMemcpyDeviceToHost, s));
+    if (found && n_points) DSDTM_CUDA(c, cudaMemcpyAsync(found, c->st_found_d + point_first, (size_t)n_points * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
     DSDTM_CUDA(c, cudaStreamSynchronize(s));
     return 0;
 }
@@ -1644,7 +1709,7 @@ int dsdtm_batch_stage(dsdtm_ctx* c, int n_pairs, const int* ref_slots, const int
     auto& b = c->batch;
     b.staged = true; b.n_pairs = n_pairs; b.feat_stride = feat_stride; b.max_level = max_level; b.min_level = min_level;
     b.max_iters = max_iters; b.patches_per_pair = ppp; b.align_iters = align_iters;
-    b.map_staged = false; b.store_staged = false; b.track_staged = false; b.kf_staged = false;
+    b.map_staged = false; b.store_staged = false; b.track_staged = false; b.kf_staged = false; b.commit_flags = 0;
     return 0;
 }
 
@@ -1659,7 +1724,7 @@ int dsdtm_batch_stage_map(dsdtm_ctx* c, const double* poses_ref_c2w, int points_
     DSDTM_CUDA(c, cudaMemcpyAsync(c->poses_ref_d, poses_ref_c2w, (size_t)b.n_pairs * 7 * sizeof(double), cudaMemcpyHostToDevice, c->stream));
     DSDTM_CUDA(c, cudaStreamSynchronize(c->stream));
     b.map_staged = true; b.map_ppp = points_per_pair; b.max_search_level = max_search_level; b.map_align_iters = align_iters;
-    b.store_staged = false; b.track_staged = false; b.kf_staged = false;
+    b.store_staged = false; b.track_staged = false; b.kf_staged = false; b.commit_flags = 0;
     drop_graphs(c);
     return 0;
 }
@@ -1716,7 +1781,7 @@ int dsdtm_batch_stage_store(dsdtm_ctx* c, const double* poses_ref_c2w, const int
     b.store_staged = true; b.store_all_rows = kf_range == nullptr; b.store_max_local = max_local; b.store_cpf = cands_per_frame;
     b.store_range_max = range_max; b.store_range_end = range_end;
     b.max_search_level = max_search_level; b.map_align_iters = align_iters;
-    b.map_staged = false; b.track_staged = false; b.kf_staged = false;
+    b.map_staged = false; b.track_staged = false; b.kf_staged = false; b.commit_flags = 0;
     drop_graphs(c);
     return 0;
 }
@@ -1746,10 +1811,11 @@ int dsdtm_batch_fetch_store(dsdtm_ctx* c, int32_t* local_rows, int32_t* n_local,
     return 0;
 }
 
-int dsdtm_batch_stage_track(dsdtm_ctx* c, const int32_t* found, int max_iters)
+static int stage_track(dsdtm_ctx* c, const int32_t* found, int max_iters, bool live)
 {
-    if (!c) return DSDTM_E_ARG;
     auto& b = c->batch;
+    if (live && (!b.staged || !b.store_staged))
+        return fail(c, DSDTM_E_STATE, "dsdtm_batch_stage_track_live: call dsdtm_batch_stage_store first");
     if (!b.staged || !(b.map_staged || b.store_staged))
         return fail(c, DSDTM_E_STATE, "dsdtm_batch_stage_track: call dsdtm_batch_stage_map or dsdtm_batch_stage_store first");
     if (max_iters < 0) return fail(c, DSDTM_E_ARG, "negative max_iters");
@@ -1775,8 +1841,10 @@ int dsdtm_batch_stage_track(dsdtm_ctx* c, const int32_t* found, int max_iters)
     // per pair and record, or in store mode per store point row
     const size_t n = b.store_staged ? c->st_pts_n : (size_t)b.n_pairs * b.map_ppp;
     std::vector<int32_t> ones;
-    if (!found) { ones.assign(std::max(n, (size_t)1), 1); found = ones.data(); }   // MapPoint::mnFound starts at 1
-    if (b.store_staged) {
+    if (!found && !live) { ones.assign(std::max(n, (size_t)1), 1); found = ones.data(); }   // MapPoint::mnFound starts at 1
+    if (live) {
+        b.store_n_found = 0;                                   // the selection reads the store's own counts (enqueue_track)
+    } else if (b.store_staged) {
         if (grow(c, &c->sb_found_d, &c->sb_found_cap, std::max(n, (size_t)1))) return DSDTM_E_NOMEM;
         if (n) DSDTM_CUDA(c, cudaMemcpyAsync(c->sb_found_d, found, n * sizeof(int32_t), cudaMemcpyHostToDevice, s));
         b.store_n_found = (int)n;
@@ -1787,9 +1855,21 @@ int dsdtm_batch_stage_track(dsdtm_ctx* c, const int32_t* found, int max_iters)
     DSDTM_CUDA(c, cudaMemsetAsync(c->trk_match_d, 0, B * K * sizeof(dsdtm_match), s));
     DSDTM_CUDA(c, cudaMemsetAsync(c->trk_res_d, 0, B * K * sizeof(double), s));
     DSDTM_CUDA(c, cudaStreamSynchronize(s));
-    b.track_staged = true; b.track_iters = max_iters; b.kf_staged = false;
+    b.track_staged = true; b.track_iters = max_iters; b.kf_staged = false; b.store_found_live = live; b.commit_flags = 0;
     drop_graphs(c);
     return 0;
+}
+
+int dsdtm_batch_stage_track(dsdtm_ctx* c, const int32_t* found, int max_iters)
+{
+    if (!c) return DSDTM_E_ARG;
+    return stage_track(c, found, max_iters, false);
+}
+
+int dsdtm_batch_stage_track_live(dsdtm_ctx* c, int max_iters)
+{
+    if (!c) return DSDTM_E_ARG;
+    return stage_track(c, nullptr, max_iters, true);
 }
 
 int dsdtm_batch_stage_keyframe(dsdtm_ctx* c, const int32_t* depth_slots, const uint8_t* want, float detection_threshold, int min_dist, int max_fts,
@@ -1835,6 +1915,7 @@ int dsdtm_batch_stage_keyframe(dsdtm_ctx* c, const int32_t* depth_slots, const u
     if (!rows.empty()) DSDTM_CUDA(c, cudaMemcpyAsync(c->kf_rows_d, rows.data(), rows.size() * sizeof(int32_t), cudaMemcpyHostToDevice, s));
     DSDTM_CUDA(c, cudaStreamSynchronize(s));
     b.kf_staged = true; b.kf_min_dist = min_dist; b.kf_max_fts = max_fts; b.kf_thr = detection_threshold; b.kf_n_wanted = (int)rows.size();
+    b.kf_want = wt; b.commit_flags = 0;
     for (int k = 0; k < 5; ++k) b.kf_dist[k] = dist[k];
     b.kf_depth_scale = any_depth ? depth_scale : 1.0f;
     drop_graphs(c);
@@ -1864,7 +1945,8 @@ static int enqueue_track(dsdtm_ctx* c, cudaStream_t s, bool timed)
     auto& b = c->batch;
     const int ppp = b.store_staged ? b.store_cpf : b.map_ppp;
     if (timed) stage_begin(c, DSDTM_STAGE_LOCAL_MAP);
-    if (b.store_staged) DSDTM_CUDA(c, launch_track_select_store(c, b.n_pairs, b.store_cpf, b.store_n_found, s));
+    if (b.store_staged && b.store_found_live) DSDTM_CUDA(c, launch_track_select_store(c, b.n_pairs, b.store_cpf, c->st_found_d, (int)c->st_pts_n, s));
+    else if (b.store_staged) DSDTM_CUDA(c, launch_track_select_store(c, b.n_pairs, b.store_cpf, c->sb_found_d, b.store_n_found, s));
     else DSDTM_CUDA(c, launch_track_select(c, b.n_pairs, b.feat_stride, b.map_ppp, s));
     if (timed) stage_end(c, 1);
     const PoseOptIo io = { c->trk_obs_d, c->trk_nobs_d, c->trk_pose_in_d, c->trk_pose_out_d, c->trk_res_d, c->trk_sum_d };
@@ -1989,6 +2071,7 @@ int dsdtm_batch_run(dsdtm_ctx* c, int flags)
     if ((flags & 8) && !(flags & 4)) return fail(c, DSDTM_E_STATE, "dsdtm_batch_run: flags bit 3 needs bit 2 (the tracked pose)");
     if ((flags & 8) && !b.kf_staged) return fail(c, DSDTM_E_STATE, "dsdtm_batch_run: flags bit 3 needs dsdtm_batch_stage_keyframe");
     const int gi = flags & 15;
+    b.commit_flags = 0;
     DSDTM_CUDA(c, cudaEventRecord(c->ev_a, c->stream));
     if (c->profiling) {
         // per-stage events cannot be recorded inside a captured graph: launch directly
@@ -2023,6 +2106,7 @@ int dsdtm_batch_run(dsdtm_ctx* c, int flags)
         }
     }
     DSDTM_CUDA(c, cudaEventRecord(c->ev_b, c->stream));
+    b.commit_flags = (b.store_staged && (flags & 4)) ? flags : 0;   // what dsdtm_batch_commit_store may apply
     return 0;
 }
 
@@ -2112,6 +2196,74 @@ int dsdtm_batch_fetch_keyframe(dsdtm_ctx* c, int32_t* n_new, dsdtm_corner* corne
     return 0;
 }
 
+int dsdtm_batch_commit_store(dsdtm_ctx* c, float outlier_threshold, const int32_t* kf_rows, int32_t* kf_row_out, int32_t* point_first_out,
+                             int32_t* n_points_out)
+{
+    if (!c) return DSDTM_E_ARG;
+    auto& b = c->batch;
+    if (!b.staged || !b.store_staged || !b.track_staged || !b.commit_flags)
+        return fail(c, DSDTM_E_STATE, "dsdtm_batch_commit_store: no store-mode run with flags bit 2 since the last staging or commit");
+    if (std::isnan(outlier_threshold)) return fail(c, DSDTM_E_ARG, "dsdtm_batch_commit_store: outlier_threshold is NaN");
+    const int n = b.n_pairs;
+    const bool kf = (b.commit_flags & 8) != 0 && b.kf_staged;
+    int n_w = 0;
+    if (kf) for (int i = 0; i < n; ++i) n_w += b.kf_want[(size_t)i] ? 1 : 0;
+    if (kf && kf_rows) {
+        // every wanted frame names its own empty key frame (dsdtm_store_append_keyframe with no features)
+        std::vector<uint8_t> named(c->st_kfs_n, 0);
+        for (int i = 0; i < n; ++i) {
+            if (!b.kf_want[(size_t)i]) continue;
+            const int r = kf_rows[i];
+            if (r < 0 || (size_t)r >= c->st_kfs_n) return fail(c, DSDTM_E_ARG, "dsdtm_batch_commit_store: reserved key-frame row outside the table");
+            if (c->st_kf_nfeat[(size_t)r] != 0) return fail(c, DSDTM_E_ARG, "dsdtm_batch_commit_store: reserved key-frame row is not empty");
+            if (named[(size_t)r]) return fail(c, DSDTM_E_ARG, "dsdtm_batch_commit_store: two frames name the same key-frame row");
+            named[(size_t)r] = 1;
+        }
+    }
+    // the worst case, reserved before anything is enqueued: every wanted frame a key frame of max(Max_fts, 200) features, all new corners
+    // with a point
+    const size_t F0 = c->st_feats_n, P0 = c->st_pts_n, K0 = c->st_kfs_n;
+    const size_t max_f = (size_t)n_w * (size_t)std::max(b.kf_max_fts, DSDTM_TRACK_MAX_MATCHES), max_p = (size_t)n_w * (size_t)b.kf_max_fts;
+    const size_t max_k = kf_rows ? 0 : (size_t)n_w;
+    if (F0 + max_f > (size_t)INT32_MAX || P0 + max_p > (size_t)INT32_MAX) return fail(c, DSDTM_E_ARG, "dsdtm_batch_commit_store: tables beyond 32-bit rows");
+    const size_t old_claim_cap = c->st_claim_cap;
+    if (grow_keep(c, &c->st_feats_d, &c->st_feats_cap, F0 + max_f, F0) || grow_keep(c, &c->st_pts_d, &c->st_pts_cap, P0 + max_p, P0) ||
+        grow_keep(c, &c->st_found_d, &c->st_found_cap, P0 + max_p, P0) || grow_keep(c, &c->st_claim_d, &c->st_claim_cap, P0 + max_p, P0) ||
+        grow_keep(c, &c->st_kfs_d, &c->st_kfs_cap, K0 + max_k, K0) || grow(c, &c->st_vis_d, &c->st_vis_cap, K0 + max_k) ||
+        grow(c, &c->st_dist_d, &c->st_dist_cap, K0 + max_k) || grow(c, &c->cm_d, &c->cm_cap, (size_t)9 * n + 4) ||
+        grow(c, &c->cm_push_d, &c->cm_push_cap, std::max(max_f, (size_t)1)))
+        return DSDTM_E_NOMEM;
+    if (!c->st_sel_d && dalloc(c, &c->st_sel_d, 32)) return DSDTM_E_NOMEM;
+    if (ensure_pinned(c, ((size_t)5 * n + 4) * sizeof(int32_t))) return DSDTM_E_NOMEM;
+    c->st_kf_nfeat.reserve(K0 + max_k);
+    drop_store_graphs(c);
+    cudaStream_t s = c->stream;
+    if (c->st_claim_cap != old_claim_cap)     // fresh part of the claim array: "never claimed" (as dsdtm_store_set_points)
+        DSDTM_CUDA(c, cudaMemsetAsync(c->st_claim_d + P0, 0xFF, (c->st_claim_cap - P0) * sizeof(unsigned long long), s));
+    int* rows_d = c->cm_d + 8 * (size_t)n + 4;
+    if (kf && kf_rows) DSDTM_CUDA(c, cudaMemcpyAsync(rows_d, kf_rows, (size_t)n * sizeof(int32_t), cudaMemcpyHostToDevice, s));
+    StoreCommitArgs a;
+    a.threshold = outlier_threshold; a.keyframes = kf; a.kf_rows_d = (kf && kf_rows) ? rows_d : nullptr;
+    a.cnt_d = c->cm_d; a.out_d = c->cm_d + 3 * (size_t)n; a.push_d = c->cm_push_d;
+    DSDTM_CUDA(c, launch_store_commit(c, a, s));
+    b.commit_flags = 0;                       // enqueued: a second commit of this run is a state error whatever happens below
+    int32_t* out_h = reinterpret_cast<int32_t*>(c->pinned);
+    DSDTM_CUDA(c, cudaMemcpyAsync(out_h, a.out_d, ((size_t)5 * n + 4) * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+    DSDTM_CUDA(c, cudaStreamSynchronize(s));
+    const int32_t* tot = out_h + 5 * (size_t)n;
+    c->st_feats_n = F0 + (size_t)tot[0];
+    c->st_pts_n = P0 + (size_t)tot[1];
+    if (!kf_rows) c->st_kfs_n = K0 + (size_t)tot[2];
+    c->st_kf_nfeat.resize(c->st_kfs_n, 0);
+    for (int i = 0; i < n; ++i)
+        if (out_h[i] >= 0) c->st_kf_nfeat[(size_t)out_h[i]] = out_h[4 * (size_t)n + i];
+    c->st_max_feats = std::max(c->st_max_feats, (int)tot[3]);
+    if (kf_row_out) std::memcpy(kf_row_out, out_h, (size_t)n * sizeof(int32_t));
+    if (point_first_out) std::memcpy(point_first_out, out_h + n, (size_t)n * sizeof(int32_t));
+    if (n_points_out) std::memcpy(n_points_out, out_h + 2 * (size_t)n, (size_t)n * sizeof(int32_t));
+    return 0;
+}
+
 float dsdtm_last_run_ms(const dsdtm_ctx* c) { return c ? c->last_run_ms : 0.f; }
 
 int dsdtm_timer_start(dsdtm_ctx* c)
@@ -2147,7 +2299,7 @@ static int pair_batch_e2e_impl(dsdtm_ctx* c, int n_pairs, const uint8_t* cur_img
         return DSDTM_E_ARG;
     if (ppp < 0 || ppp > c->prm.max_patches || align_iters < 0) return fail(c, DSDTM_E_ARG, "patches_per_pair > max_patches");
     if (ppp > 0 && (!patches10 || !patch_px || !patch_level || !patch_px_out || !patch_conv)) return fail(c, DSDTM_E_ARG, "null patch arrays");
-    c->batch.staged = false;
+    c->batch.staged = false; c->batch.commit_flags = 0;
     const LevelGeom& g = c->geo;
     const size_t img_bytes = (size_t)g.w[0] * g.h[0];
     // chunked pipeline: H2D of chunk k+1 (copy stream) overlaps the kernels of chunk k (compute stream) and the D2H of chunk k-1.

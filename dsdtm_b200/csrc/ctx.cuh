@@ -12,6 +12,7 @@
 #include <stdint.h>
 #include <stdio.h>
 #include <string>
+#include <vector>
 
 #include "../../include/dsdtm_gpu.h"
 
@@ -120,6 +121,8 @@ struct dsdtm_ctx {
     dsdtm_store_kf* st_kfs_d = nullptr;      size_t st_kfs_cap = 0, st_kfs_n = 0;
     dsdtm_store_feat* st_feats_d = nullptr;  size_t st_feats_cap = 0, st_feats_n = 0;
     dsdtm_store_point* st_pts_d = nullptr;   size_t st_pts_cap = 0, st_pts_n = 0;
+    int* st_found_d = nullptr;               size_t st_found_cap = 0;      // per point: MapPoint::mnFound (appended points start at 1)
+    std::vector<int32_t> st_kf_nfeat;        // host mirror of every key-frame row's feat_count (reserved rows of dsdtm_batch_commit_store)
     unsigned long long* st_claim_d = nullptr; size_t st_claim_cap = 0;     // per point: (~epoch << 32 | order) of the first local key frame that lists it
     uint8_t* st_vis_d = nullptr;             size_t st_vis_cap = 0;
     double* st_dist_d = nullptr;             size_t st_dist_cap = 0;
@@ -166,6 +169,9 @@ struct dsdtm_ctx {
     double* sb_pose10_d = nullptr;               // max_batch * 10: prior pose {c2w[7], centre[3]} = T_c2r * T_ref
     int2* sb_range_d = nullptr;                  // max_batch key-frame row ranges [begin, end)
     int* sb_found_d = nullptr;           size_t sb_found_cap = 0;    // per store point row: MapPoint::mnFound
+    // dsdtm_batch_commit_store's scratch, grown on demand (never captured): per-frame counts / outputs and one push link per new feature
+    int* cm_d = nullptr;                 size_t cm_cap = 0;
+    int* cm_push_d = nullptr;            size_t cm_push_cap = 0;
     // key-frame detection (dsdtm_detect_batch), grown on demand
     uint8_t* det_mask_d = nullptr;       size_t det_mask_cap = 0;    // n * w*h mask images: allocated by the first call that passes masks
     uint8_t* det_buf_d = nullptr;        size_t det_buf_cap = 0;     // small inputs (max_new, n_circles, circles) | outputs, one copy each way
@@ -188,9 +194,12 @@ struct dsdtm_ctx {
         bool store_staged = false;                         // dsdtm_batch_stage_store: bits 1..3 run on the map store instead
         bool store_all_rows = false;                       // no ranges staged: every frame reads rows [0, key frames at capture)
         int store_max_local = 0, store_cpf = 0, store_range_max = 0, store_range_end = 0, store_n_found = 0;
+        bool store_found_live = false;                     // dsdtm_batch_stage_track_live: the selection reads st_found_d
+        int commit_flags = 0;                              // flags of the last store-mode run with bit 2 not yet committed, 0 = none
         bool kf_staged = false;                            // dsdtm_batch_stage_keyframe: the key-frame half is ready
         int kf_min_dist = 0, kf_max_fts = 0, kf_n_wanted = 0;
         float kf_thr = 0.f, kf_dist[5] = {}, kf_depth_scale = 1.f;
+        std::vector<uint8_t> kf_want;                      // the staged want mask (host copy)
         cudaGraphExec_t graph[16] = {};                    // [flags & 15]
         int graph_key[16][8];
     } batch;
@@ -276,7 +285,15 @@ cudaError_t launch_pose_opt_io(dsdtm_ctx* c, const PoseOptIo& io, int n_frames, 
 // SearchLocalPoints' selection over the batched chain's records + the PoseOptimization inputs of every pair (select.cu)
 cudaError_t launch_track_select(dsdtm_ctx* c, int n_pairs, int feat_stride, int ppp, cudaStream_t s);
 // the same over the store-backed records (sb_rec_d, cpf per frame): found counts per point row (n_found of them; later rows count 1)
-cudaError_t launch_track_select_store(dsdtm_ctx* c, int n_pairs, int cpf, int n_found, cudaStream_t s);
+cudaError_t launch_track_select_store(dsdtm_ctx* c, int n_pairs, int cpf, const int* found_d, int n_found, cudaStream_t s);
+// dsdtm_batch_commit_store (store_commit.cu): found counts, bad flags, key frames, new points and observation chains of the last
+// store-mode step; four launches on the tables as they are sized now (the caller reserved the worst case)
+struct StoreCommitArgs {
+    float threshold; bool keyframes;
+    const int* kf_rows_d;                       // reserved key-frame row per frame, or null (append)
+    int* cnt_d; int* out_d; int* push_d;        // 3n, 5n + 4, one per new feature row
+};
+cudaError_t launch_store_commit(dsdtm_ctx* c, const StoreCommitArgs& a, cudaStream_t s);
 size_t track_select_smem(int ppp);             // dynamic shared memory of one selection CTA for ppp records per frame
 int track_select_key_bits(const dsdtm_ctx* c, int ppp);   // bits of a selection key for this grid and ppp (must be <= 64)
 cudaError_t track_select_init(dsdtm_ctx* c);

@@ -213,12 +213,12 @@ cudaError_t launch_track_select(dsdtm_ctx* c, int n_pairs, int feat_stride, int 
     return cudaGetLastError();
 }
 
-cudaError_t launch_track_select_store(dsdtm_ctx* c, int n_pairs, int cpf, int n_found, cudaStream_t s)
+cudaError_t launch_track_select_store(dsdtm_ctx* c, int n_pairs, int cpf, const int* found_d, int n_found, cudaStream_t s)
 {
     SelArgs a = select_args(c, n_pairs, cpf);
     if (a.radius < 0) return cudaErrorInvalidValue;
     a.srec = c->sb_rec_d; a.n_cand = c->sb_ncand_d; a.pts = c->st_pts_d; a.pose10 = c->sb_pose10_d;
-    a.found = c->sb_found_d; a.n_found = n_found;
+    a.found = found_d; a.n_found = n_found;
     a.jbits = index_bits(cpf);
     track_select_kernel<true><<<(n_pairs + kSelWarps - 1) / kSelWarps, kSelWarps * 32, track_select_smem(cpf), s>>>(a);
     c->launches++;

@@ -414,7 +414,8 @@ int dsdtm_track_frame(dsdtm_ctx* ctx, const dsdtm_track_in* in, dsdtm_track_out*
  * reference -- a loop over every map point of the ten local key frames, a mutex-guarded Get_Pose per point, a std::map copy per
  * candidate -- becomes table maintenance at key-frame rate: a key frame appends its row and its features' rows once
  * (dsdtm_store_append_keyframe), map points are appended / updated when they are created, moved by a bundle adjustment or flagged bad
- * (dsdtm_store_set_points / dsdtm_store_update_points), and every frame makes one call (dsdtm_store_track). */
+ * (dsdtm_store_set_points / dsdtm_store_update_points), and every frame makes one call (dsdtm_store_track). The batched chain writes back
+ * into the store itself with dsdtm_batch_commit_store (found counts, bad flags, key frames and their new points). */
 typedef struct {
     int32_t slot;           /* frame slot of the key frame's pyramid (KeyFrame::mvImg_Pyr) */
     int32_t feat_begin;     /* first row of this key frame in the feature table (filled by the library on append) */
@@ -451,6 +452,20 @@ int dsdtm_store_append_keyframe(dsdtm_ctx* ctx, const dsdtm_store_kf* kf, const 
 /* pose / slot of an existing key frame (bundle adjustment moved it; its pyramid was re-uploaded into another slot) */
 int dsdtm_store_set_keyframe(dsdtm_ctx* ctx, int row, int slot, const double pose_c2w[7], const double center[3]);
 int dsdtm_store_clear(dsdtm_ctx* ctx);
+/* MapPoint::mnFound: the store keeps one count per point row; a point appended by any path (dsdtm_store_set_points,
+ * dsdtm_batch_commit_store) starts at 1, as MapPoint's constructor does; a rewritten row keeps its count. Scattered setter, as
+ * dsdtm_store_update_points: found[i] becomes the count of point ids[i]. */
+int dsdtm_store_set_found(dsdtm_ctx* ctx, const int32_t* ids, int n, const int32_t* found);
+/* rows of the key-frame, feature and point tables (any pointer may be NULL) */
+int dsdtm_store_size(const dsdtm_ctx* ctx, int32_t* n_kfs, int32_t* n_feats, int32_t* n_points);
+/* Reads ranges of the tables as the library holds them (any output pointer may be NULL; found follows the point range): key frames
+ * [kf_first, +n_kfs), features [feat_first, +n_feats), points and their found counts [point_first, +n_points). DSDTM_E_ARG for a range
+ * past a table's end. Library fields: a feature's is_obs is the row of the key frame that observes its point + 1 (0 = no observation;
+ * dsdtm_store_append_keyframe turns the caller's flag into this), next_obs the next older observing feature row of the same point (-1 =
+ * end), a point's last_obs its newest observing feature row (-1 = none): walking last_obs -> next_obs lists MapPoint::mObservations
+ * newest first. */
+int dsdtm_store_fetch(dsdtm_ctx* ctx, int kf_first, int n_kfs, dsdtm_store_kf* kfs, int feat_first, int n_feats, dsdtm_store_feat* feats,
+                      int point_first, int n_points, dsdtm_store_point* points, int32_t* found);
 /* One frame: GetCloseKeyFrames over all key frames (a point of the key frame visible in the current frame), the max_local nearest by
  * |t_cur - t_kf| (stable in row order), every map point of those key frames once (first key frame in rank order wins, bad points
  * skipped), ReprojectPoint, and for the points inside the image Get_ClosetObs + the IsInImage gate + SolveAffineMatrix +
@@ -528,7 +543,8 @@ int dsdtm_batch_stage_track(dsdtm_ctx* ctx, const int32_t* found, int max_iters)
  * n_matches = n_pairs; matches = n_pairs x DSDTM_TRACK_MAX_MATCHES (mvFeatures order, the first n_matches[i] valid);
  * res_norm = n_pairs x DSDTM_TRACK_MAX_MATCHES, GetReprojectReidual() at the final pose per match (ref: src/Optimizer.cpp:298-318):
  * the caller compares it with LocalBAthreshhold / Camera.f to call MapPoint::EraseFound (ref: :81-94) and keeps the found counts
- * itself; summaries = n_pairs. Every pointer may be NULL. */
+ * itself, or, in store mode, dsdtm_batch_commit_store applies them to the store on the device; summaries = n_pairs. Every pointer may
+ * be NULL. */
 int dsdtm_batch_fetch_track(dsdtm_ctx* ctx, double* poses_c2w_out, int32_t* n_matches, dsdtm_match* matches, double* res_norm,
                             dsdtm_ba_summary* summaries);
 /* Tracking::CraeteKeyframe behind the tracked pose (ref: src/Tracking.cpp:412-464), so that dsdtm_batch_run(flags | 2 | 4 | 8) ends in the
@@ -584,6 +600,43 @@ int dsdtm_batch_stage_store(dsdtm_ctx* ctx, const double* poses_ref_c2w /* n_pai
  * n_local[i]); cands = n_pairs x cands_per_frame records in `order` (rows past min(n_cand[i], cands_per_frame) zero); n_cand = the true
  * candidate count, which may exceed cands_per_frame. Every pointer may be NULL. */
 int dsdtm_batch_fetch_store(dsdtm_ctx* ctx, int32_t* local_rows, int32_t* n_local, dsdtm_store_cand* cands, int32_t* n_cand);
+/* dsdtm_batch_stage_track in store mode with live found counts: the selection reads the store's own counts (dsdtm_store_set_found,
+ * dsdtm_batch_commit_store) at every run instead of a host snapshot. DSDTM_E_STATE without dsdtm_batch_stage_store; otherwise as
+ * dsdtm_batch_stage_track, which keeps its snapshot semantics (NULL = all 1). */
+int dsdtm_batch_stage_track_live(dsdtm_ctx* ctx, int max_iters);
+/* Commits what the frames of the last dsdtm_batch_run with flags 7 or 15 in store mode did to the map store, in frame order, on the device
+ * (ref: src/Feature_alignment.cpp:106, src/Optimizer.cpp:81-94, src/Tracking.cpp:412-464):
+ *   found : for every frame with n_matches >= 0, +1 for each match's point (IncreaseFound); then -1 for each match i with
+ *           res_norm[i] > outlier_threshold (strict; pass LocalBAthreshhold / Camera.f, compared in double) unless its point was bad when
+ *           the commit started (EraseFound); every matched point whose count ends <= 0 gets bad = 1. The bad flags and counts are read
+ *           when the commit starts, not when the step ran, on purpose: the walk never lists a bad point, so for the tracker the two are
+ *           the same, and a caller that changes the store between the run and the commit (dsdtm_store_set_found, a point flagged bad by
+ *           LocalMapping) gets what the reference's EraseFound loop, running after that change, would do. Residual block i is match i: a new
+ *           frame's features are exactly its matches and the walk never lists a bad point, so the block / feature index shift of the
+ *           per-frame EraseFound loop (features without a point or with a bad one) cannot arise. A frame with n_matches -1 changes nothing.
+ *   key frames (flags 15 only): every wanted frame with n_matches >= 0 becomes a key frame. Features in mvFeatures order: the matches
+ *           (mp = the store point row, the match level and px, normal = the bearing PoseOptimization's observation used, observing), then
+ *           the new corners (px and normal of the lifted record, the corner level; a DSDTM_LIFT_OK corner gets a new point at point_w,
+ *           found 1, not bad, and observes it; a corner without depth has mp -1). Row: slot = the pair's cur slot (the store now names
+ *           it: do not reuse it for a later cur frame while the key frame lives), pose_c2w = the pose after PoseOptimization, center =
+ *           Get_CameraCnt() of that pose.
+ *   rows  : features and new points are appended frame by frame in frame order; key frames are appended in frame order (kf_rows NULL) or
+ *           fill the row kf_rows[i] that the caller reserved for wanted frame i as an EMPTY key frame (dsdtm_store_append_keyframe with no
+ *           features: never close, never in a local map), e.g. inside the scene's own range of a tiled store. Entries of frames that are
+ *           not wanted are ignored; a wanted frame that overflowed leaves its row empty.
+ *   chains: the store equals, bit for bit, the one sequential calls build in frame order: dsdtm_store_set_points for the new points,
+ *           dsdtm_store_append_keyframe per key frame (or the same rewrite of the reserved row), dsdtm_store_update_points for the bad
+ *           flags; a point observed by several key frames of one commit is linked newest first above its older chain.
+ * Per frame i: kf_row_out[i] = its key-frame row (-1 if none), point_first_out[i] = its first new point row (-1 without a key frame),
+ * n_points_out[i] = its new points; any of them may be NULL. Frames of one step that share a map all read the counts the step started
+ * with and their increments add up; the result equals the sequential tracker when each map has at most one frame per step (a later frame
+ * of the same map would have seen the earlier frame's counts, bad flags and key frame). Cost: a point that k key frames of one commit
+ * observe is linked by one thread in O(k log k) dependent loads (k = 1 in that layout, k = frames per map otherwise). The commit drops the captured store-mode steps,
+ * reserves the worst case before enqueuing (DSDTM_E_NOMEM: the store is unchanged) and synchronises once to read the new table sizes.
+ * DSDTM_E_ARG, nothing enqueued, for a NaN threshold or, for a wanted frame, a reserved row outside the table, not empty or named twice.
+ * DSDTM_E_STATE without a store-mode run with flags bit 2 since the last staging, after dsdtm_store_clear, or for a second commit. */
+int dsdtm_batch_commit_store(dsdtm_ctx* ctx, float outlier_threshold, const int32_t* kf_rows /* n_pairs or NULL */, int32_t* kf_row_out,
+                             int32_t* point_first_out, int32_t* n_points_out);
 int dsdtm_batch_fetch(dsdtm_ctx* ctx, double* poses_out, int* n_tracked, double* patch_px_out, uint8_t* patch_conv);
 /* end-to-end step with HOST buffers: uploads the n_pairs cur images (dense, pinned recommended) into their cur slots,
  * stages the per-pair inputs, runs, and fetches -- copies overlapped with compute in chunks on internal streams. Both e2e entries
