@@ -13,7 +13,7 @@ CSRC = os.path.join(HERE, "csrc")
 LIBDIR = os.path.join(HERE, "lib")
 # DSDTM_GPU_LIB: measurement scripts load a prebuilt experiment library (scripts/sa_build_variants.py) instead of the default build
 LIB = os.environ.get("DSDTM_GPU_LIB") or os.path.join(LIBDIR, "libdsdtm_gpu.so")
-SOURCES = ["capi.cu", "pyramid.cu", "fast.cu", "sparse_align.cu", "align2d.cu", "local_map.cu", "ingest.cu", "clahe.cu", "pose_opt.cu", "select.cu", "detect_select.cu", "keyframe.cu", "store_commit.cu", "probe.cu"]
+SOURCES = ["capi.cu", "pyramid.cu", "fast.cu", "sparse_align.cu", "align2d.cu", "local_map.cu", "ingest.cu", "clahe.cu", "pose_opt.cu", "select.cu", "detect_select.cu", "keyframe.cu", "store_commit.cu", "sequence_advance.cu", "probe.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "--fmad=true", "-Xptxas", "-v"]
 

@@ -38,6 +38,7 @@ BA_MAX_OBS = 4096
 MATCH_DT = np.dtype([("point", "<i4"), ("px", "<f4", 2), ("level", "<i4")])
 assert MATCH_DT.itemsize == 16
 TRACK_MAX_MATCHES = 200
+ADV_ADVANCED, ADV_KEYFRAME, ADV_HELD_OVERFLOW, ADV_HELD_CALLER = 0, 1, 2, 3   # dsdtm_batch_advance's per-frame status
 CIRCLE_DT = np.dtype([("px", "<f4", 2), ("radius", "<i4"), ("reserved", "<i4")])
 assert CIRCLE_DT.itemsize == 16
 # device-resident map store (dsdtm_store_*)
@@ -96,6 +97,7 @@ SYMBOLS = [
     "dsdtm_pose_optimize", "dsdtm_pose_optimize_batch", "dsdtm_map_table_upload", "dsdtm_close_keyframes", "dsdtm_probe_fp64", "dsdtm_frame_upload_pyramid_async", "dsdtm_track_frame_store", "dsdtm_store_set_points", "dsdtm_store_update_points", "dsdtm_store_append_keyframe", "dsdtm_store_set_keyframe", "dsdtm_store_clear", "dsdtm_store_track", "dsdtm_frame_upload_level", "dsdtm_batch_stage_map", "dsdtm_batch_fetch_map", "dsdtm_track_batch_e2e",
     "dsdtm_batch_stage_track", "dsdtm_batch_fetch_track", "dsdtm_detect", "dsdtm_detect_batch",
     "dsdtm_batch_stage_keyframe", "dsdtm_batch_fetch_keyframe", "dsdtm_batch_stage_store", "dsdtm_batch_fetch_store",
+    "dsdtm_batch_advance", "dsdtm_batch_upload_step", "dsdtm_batch_fetch_ref", "dsdtm_graph_captures",
     "dsdtm_store_set_found", "dsdtm_store_size", "dsdtm_store_fetch", "dsdtm_batch_stage_track_live", "dsdtm_batch_commit_store",
 ]
 
@@ -124,6 +126,8 @@ def load():
     L.dsdtm_host_free.argtypes = [C.c_void_p]
     L.dsdtm_launch_count.restype = C.c_longlong
     L.dsdtm_launch_count.argtypes = [C.c_void_p]
+    L.dsdtm_graph_captures.restype = C.c_longlong
+    L.dsdtm_graph_captures.argtypes = [C.c_void_p]
     L.dsdtm_last_run_ms.restype = C.c_float
     L.dsdtm_last_run_ms.argtypes = [C.c_void_p]
     L.dsdtm_timer_stop.restype = C.c_float
@@ -200,6 +204,10 @@ class Context:
 
     def launch_count(self):
         return int(self.L.dsdtm_launch_count(self.hp))
+
+    def graph_captures(self):
+        """CUDA graphs batch_run has captured on this context: a run that replays a captured step adds nothing"""
+        return int(self.L.dsdtm_graph_captures(self.hp))
 
     def set_option(self, key, value):
         self._ck(self.L.dsdtm_set_option(self.hp, key.encode(), int(value)))
@@ -523,7 +531,7 @@ class Context:
         n = len(ref_slots)
         feats = np.ascontiguousarray(feats, REF_FEAT_DT).reshape(n, -1)
         ppp = 0 if patch_level is None else np.asarray(patch_level).reshape(n, -1).shape[1]
-        self._n = n; self._ppp = ppp; self._store_cpf = None
+        self._n = n; self._ppp = ppp; self._store_cpf = None; self._feat_stride = feats.shape[1]
         self._ck(self.L.dsdtm_batch_stage(
             self.hp, n, _p(np.ascontiguousarray(ref_slots, np.int32)), _p(np.ascontiguousarray(cur_slots, np.int32)), _p(feats),
             feats.shape[1], _p(np.ascontiguousarray(n_feats, np.int32)), _p(np.ascontiguousarray(ref_centers, np.float64)),
@@ -583,6 +591,35 @@ class Context:
         self._ck(self.L.dsdtm_batch_commit_store(self.hp, C.c_float(outlier_threshold), _p(kr), _p(row), _p(pf), _p(npt)))
         self.store_keyframes, _, self.store_points = self.store_size()
         return row, pf, npt
+
+    def batch_advance(self, next_cur_slots, hold=None, want_next=None):
+        """dsdtm_batch_advance after batch_commit_store: every frame that is not held becomes its own next reference frame on the device,
+        every frame's cur slot moves to next_cur_slots. hold / want_next = (n_pairs,) bools or None. Returns the (n_pairs,) ADV_* status."""
+        n = self._n
+        nc = np.ascontiguousarray(next_cur_slots, np.int32).reshape(n)
+        hd = None if hold is None else np.ascontiguousarray(hold, np.uint8).reshape(n)
+        wt = None if want_next is None else np.ascontiguousarray(want_next, np.uint8).reshape(n)
+        st = np.empty(n, np.uint8)
+        self._ck(self.L.dsdtm_batch_advance(self.hp, _p(nc), _p(hd), _p(wt), _p(st)))
+        return st
+
+    def batch_upload_step(self, imgs, depth=None):
+        """dsdtm_batch_upload_step: (n_pairs, height, width) uint8 images into the staged cur slots and, optionally, (n_pairs, height, width)
+        uint16 depth images into the staged depth slots; batch_run(flags | 1) builds the pyramids"""
+        n = self._n
+        im = np.ascontiguousarray(imgs, np.uint8).reshape(n, self.height, self.width)
+        d = None if depth is None else np.ascontiguousarray(depth, np.uint16).reshape(n, self.height, self.width)
+        self._ck(self.L.dsdtm_batch_upload_step(self.hp, _p(im), _p(d)))
+
+    def batch_fetch_ref(self):
+        """-> dict(ref_slots, cur_slots, feats (n, feat_stride) REF_FEAT_DT, n_feats, centers (n, 3), poses_ref (n, 7), poses_in (n, 7)):
+        the staged per-frame inputs as the next batch_run reads them"""
+        n, fs = self._n, self._feat_stride
+        r = dict(ref_slots=np.empty(n, np.int32), cur_slots=np.empty(n, np.int32), feats=np.empty((n, fs), REF_FEAT_DT),
+                 n_feats=np.empty(n, np.int32), centers=np.empty((n, 3)), poses_ref=np.empty((n, 7)), poses_in=np.empty((n, 7)))
+        self._ck(self.L.dsdtm_batch_fetch_ref(self.hp, *(_p(r[k]) for k in ("ref_slots", "cur_slots", "feats", "n_feats", "centers",
+                                                                            "poses_ref", "poses_in"))))
+        return r
 
     def batch_fetch_track(self):
         """-> (poses c2w after PoseOptimization (n, 7), n_matches (n,), matches (n, 200) MATCH_DT, res_norm (n, 200), summaries (n,)

@@ -338,7 +338,7 @@ void dsdtm_destroy(dsdtm_ctx* c)
                      c->det_mask_d, c->det_buf_d, c->kf_circ_d, c->kf_ncirc_d, c->kf_max_new_d, c->kf_corner_d, c->kf_lifted_d, c->kf_nnew_d,
                      c->kf_exact_d, c->kf_depth_slot_d, c->kf_want_d, c->kf_rows_d,
                      c->sb_rec_d, c->sb_ncand_d, c->sb_local_d, c->sb_pose10_d, c->sb_range_d, c->sb_found_d,
-                     c->st_found_d, c->cm_d, c->cm_push_d };
+                     c->st_found_d, c->cm_d, c->cm_push_d, c->adv_d };
     for (void* p : bufs) if (p) cudaFree(p);
     if (c->pinned) cudaFreeHost(c->pinned);
     if (c->stage_pin) cudaFreeHost(c->stage_pin);
@@ -389,6 +389,7 @@ void* dsdtm_host_alloc(size_t bytes)
 void dsdtm_host_free(void* p) { if (p) cudaFreeHost(p); }
 
 long long dsdtm_launch_count(const dsdtm_ctx* c) { return c ? c->launches : 0; }
+long long dsdtm_graph_captures(const dsdtm_ctx* c) { return c ? c->captures : 0; }
 
 int dsdtm_set_option(dsdtm_ctx* c, const char* key, int value)
 {
@@ -1250,7 +1251,8 @@ int dsdtm_store_clear(dsdtm_ctx* c)
     c->st_kfs_n = c->st_feats_n = c->st_pts_n = 0;
     c->st_max_feats = 0;
     c->st_kf_nfeat.clear();
-    c->batch.commit_flags = 0;                   // the step's matches name rows that are gone
+    c->st_kf_slot.clear();
+    c->batch.commit_flags = 0; c->batch.advance_flags = 0;                   // the step's matches name rows that are gone
     drop_store_graphs(c);
     return 0;
 }
@@ -1355,6 +1357,7 @@ int dsdtm_store_append_keyframe(dsdtm_ctx* c, const dsdtm_store_kf* kf, const ds
     c->st_kfs_n = r + 1; c->st_feats_n = f0 + n_feats;
     c->st_max_feats = std::max(c->st_max_feats, n_feats);
     c->st_kf_nfeat.push_back(n_feats);
+    c->st_kf_slot.push_back(kf->slot);
     DSDTM_CUDA(c, launch_store_link(c, (int)f0, n_feats, s));
     DSDTM_CUDA(c, cudaStreamSynchronize(s));
     if (row) *row = (int32_t)r;
@@ -1376,6 +1379,7 @@ int dsdtm_store_set_keyframe(dsdtm_ctx* c, int row, int slot, const double pose_
     for (int i = 0; i < 3; ++i) k.center[i] = center[i];
     DSDTM_CUDA(c, cudaMemcpyAsync(c->st_kfs_d + row, &k, sizeof k, cudaMemcpyHostToDevice, s));
     DSDTM_CUDA(c, cudaStreamSynchronize(s));
+    c->st_kf_slot[(size_t)row] = slot;
     return 0;
 }
 
@@ -1709,7 +1713,8 @@ int dsdtm_batch_stage(dsdtm_ctx* c, int n_pairs, const int* ref_slots, const int
     auto& b = c->batch;
     b.staged = true; b.n_pairs = n_pairs; b.feat_stride = feat_stride; b.max_level = max_level; b.min_level = min_level;
     b.max_iters = max_iters; b.patches_per_pair = ppp; b.align_iters = align_iters;
-    b.map_staged = false; b.store_staged = false; b.track_staged = false; b.kf_staged = false; b.commit_flags = 0;
+    b.ref_h.assign(ref_slots, ref_slots + n_pairs); b.cur_h.assign(cur_slots, cur_slots + n_pairs);
+    b.map_staged = false; b.store_staged = false; b.track_staged = false; b.kf_staged = false; b.commit_flags = 0; b.advance_flags = 0;
     return 0;
 }
 
@@ -1724,7 +1729,7 @@ int dsdtm_batch_stage_map(dsdtm_ctx* c, const double* poses_ref_c2w, int points_
     DSDTM_CUDA(c, cudaMemcpyAsync(c->poses_ref_d, poses_ref_c2w, (size_t)b.n_pairs * 7 * sizeof(double), cudaMemcpyHostToDevice, c->stream));
     DSDTM_CUDA(c, cudaStreamSynchronize(c->stream));
     b.map_staged = true; b.map_ppp = points_per_pair; b.max_search_level = max_search_level; b.map_align_iters = align_iters;
-    b.store_staged = false; b.track_staged = false; b.kf_staged = false; b.commit_flags = 0;
+    b.store_staged = false; b.track_staged = false; b.kf_staged = false; b.commit_flags = 0; b.advance_flags = 0;
     drop_graphs(c);
     return 0;
 }
@@ -1781,7 +1786,7 @@ int dsdtm_batch_stage_store(dsdtm_ctx* c, const double* poses_ref_c2w, const int
     b.store_staged = true; b.store_all_rows = kf_range == nullptr; b.store_max_local = max_local; b.store_cpf = cands_per_frame;
     b.store_range_max = range_max; b.store_range_end = range_end;
     b.max_search_level = max_search_level; b.map_align_iters = align_iters;
-    b.map_staged = false; b.track_staged = false; b.kf_staged = false; b.commit_flags = 0;
+    b.map_staged = false; b.track_staged = false; b.kf_staged = false; b.commit_flags = 0; b.advance_flags = 0;
     drop_graphs(c);
     return 0;
 }
@@ -1855,7 +1860,7 @@ static int stage_track(dsdtm_ctx* c, const int32_t* found, int max_iters, bool l
     DSDTM_CUDA(c, cudaMemsetAsync(c->trk_match_d, 0, B * K * sizeof(dsdtm_match), s));
     DSDTM_CUDA(c, cudaMemsetAsync(c->trk_res_d, 0, B * K * sizeof(double), s));
     DSDTM_CUDA(c, cudaStreamSynchronize(s));
-    b.track_staged = true; b.track_iters = max_iters; b.kf_staged = false; b.store_found_live = live; b.commit_flags = 0;
+    b.track_staged = true; b.track_iters = max_iters; b.kf_staged = false; b.store_found_live = live; b.commit_flags = 0; b.advance_flags = 0;
     drop_graphs(c);
     return 0;
 }
@@ -1915,7 +1920,7 @@ int dsdtm_batch_stage_keyframe(dsdtm_ctx* c, const int32_t* depth_slots, const u
     if (!rows.empty()) DSDTM_CUDA(c, cudaMemcpyAsync(c->kf_rows_d, rows.data(), rows.size() * sizeof(int32_t), cudaMemcpyHostToDevice, s));
     DSDTM_CUDA(c, cudaStreamSynchronize(s));
     b.kf_staged = true; b.kf_min_dist = min_dist; b.kf_max_fts = max_fts; b.kf_thr = detection_threshold; b.kf_n_wanted = (int)rows.size();
-    b.kf_want = wt; b.commit_flags = 0;
+    b.kf_want = wt; b.kf_depth_h = ds; b.commit_flags = 0; b.advance_flags = 0;
     for (int k = 0; k < 5; ++k) b.kf_dist[k] = dist[k];
     b.kf_depth_scale = any_depth ? depth_scale : 1.0f;
     drop_graphs(c);
@@ -2071,7 +2076,7 @@ int dsdtm_batch_run(dsdtm_ctx* c, int flags)
     if ((flags & 8) && !(flags & 4)) return fail(c, DSDTM_E_STATE, "dsdtm_batch_run: flags bit 3 needs bit 2 (the tracked pose)");
     if ((flags & 8) && !b.kf_staged) return fail(c, DSDTM_E_STATE, "dsdtm_batch_run: flags bit 3 needs dsdtm_batch_stage_keyframe");
     const int gi = flags & 15;
-    b.commit_flags = 0;
+    b.commit_flags = 0; b.advance_flags = 0;
     DSDTM_CUDA(c, cudaEventRecord(c->ev_a, c->stream));
     if (c->profiling) {
         // per-stage events cannot be recorded inside a captured graph: launch directly
@@ -2093,6 +2098,7 @@ int dsdtm_batch_run(dsdtm_ctx* c, int flags)
             cudaGraphDestroy(g);
             if (e != cudaSuccess) return fail(c, DSDTM_E_CUDA, "cudaGraphInstantiate", e);
             std::memcpy(b.graph_key[gi], key, sizeof key);
+            ++c->captures;
             // re-record the start event after the (untimed) capture work
             DSDTM_CUDA(c, cudaEventRecord(c->ev_a, c->stream));
         }
@@ -2227,6 +2233,8 @@ int dsdtm_batch_commit_store(dsdtm_ctx* c, float outlier_threshold, const int32_
     const size_t max_k = kf_rows ? 0 : (size_t)n_w;
     if (F0 + max_f > (size_t)INT32_MAX || P0 + max_p > (size_t)INT32_MAX) return fail(c, DSDTM_E_ARG, "dsdtm_batch_commit_store: tables beyond 32-bit rows");
     const size_t old_claim_cap = c->st_claim_cap;
+    // what a captured store-mode step points at: a commit that moves none of these tables and writes no key frame keeps the captures
+    const void* tables0[] = { c->st_feats_d, c->st_pts_d, c->st_found_d, c->st_claim_d, c->st_kfs_d, c->st_vis_d, c->st_dist_d };
     if (grow_keep(c, &c->st_feats_d, &c->st_feats_cap, F0 + max_f, F0) || grow_keep(c, &c->st_pts_d, &c->st_pts_cap, P0 + max_p, P0) ||
         grow_keep(c, &c->st_found_d, &c->st_found_cap, P0 + max_p, P0) || grow_keep(c, &c->st_claim_d, &c->st_claim_cap, P0 + max_p, P0) ||
         grow_keep(c, &c->st_kfs_d, &c->st_kfs_cap, K0 + max_k, K0) || grow(c, &c->st_vis_d, &c->st_vis_cap, K0 + max_k) ||
@@ -2234,9 +2242,11 @@ int dsdtm_batch_commit_store(dsdtm_ctx* c, float outlier_threshold, const int32_
         grow(c, &c->cm_push_d, &c->cm_push_cap, std::max(max_f, (size_t)1)))
         return DSDTM_E_NOMEM;
     if (!c->st_sel_d && dalloc(c, &c->st_sel_d, 32)) return DSDTM_E_NOMEM;
-    if (ensure_pinned(c, ((size_t)5 * n + 4) * sizeof(int32_t))) return DSDTM_E_NOMEM;
+    if (ensure_pinned(c, ((size_t)6 * n + 4) * sizeof(int32_t))) return DSDTM_E_NOMEM;
     c->st_kf_nfeat.reserve(K0 + max_k);
-    drop_store_graphs(c);
+    c->st_kf_slot.reserve(K0 + max_k);
+    const void* tables1[] = { c->st_feats_d, c->st_pts_d, c->st_found_d, c->st_claim_d, c->st_kfs_d, c->st_vis_d, c->st_dist_d };
+    if (std::memcmp(tables0, tables1, sizeof tables0) != 0) drop_store_graphs(c);
     cudaStream_t s = c->stream;
     if (c->st_claim_cap != old_claim_cap)     // fresh part of the claim array: "never claimed" (as dsdtm_store_set_points)
         DSDTM_CUDA(c, cudaMemsetAsync(c->st_claim_d + P0, 0xFF, (c->st_claim_cap - P0) * sizeof(unsigned long long), s));
@@ -2246,21 +2256,154 @@ int dsdtm_batch_commit_store(dsdtm_ctx* c, float outlier_threshold, const int32_
     a.threshold = outlier_threshold; a.keyframes = kf; a.kf_rows_d = (kf && kf_rows) ? rows_d : nullptr;
     a.cnt_d = c->cm_d; a.out_d = c->cm_d + 3 * (size_t)n; a.push_d = c->cm_push_d;
     DSDTM_CUDA(c, launch_store_commit(c, a, s));
-    b.commit_flags = 0;                       // enqueued: a second commit of this run is a state error whatever happens below
+    const int committed = b.commit_flags;
+    b.commit_flags = 0; b.advance_flags = 0;                       // enqueued: a second commit of this run is a state error whatever happens below
     int32_t* out_h = reinterpret_cast<int32_t*>(c->pinned);
     DSDTM_CUDA(c, cudaMemcpyAsync(out_h, a.out_d, ((size_t)5 * n + 4) * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+    int32_t* nm_h = out_h + 5 * (size_t)n + 4;                // the match counts, for dsdtm_batch_advance's held frames
+    DSDTM_CUDA(c, cudaMemcpyAsync(nm_h, c->trk_nobs_d, (size_t)n * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
     DSDTM_CUDA(c, cudaStreamSynchronize(s));
     const int32_t* tot = out_h + 5 * (size_t)n;
+    if (tot[2] != 0) drop_store_graphs(c);    // a key frame: new rows, a reserved row filled, maybe a wider st_max_feats
     c->st_feats_n = F0 + (size_t)tot[0];
     c->st_pts_n = P0 + (size_t)tot[1];
     if (!kf_rows) c->st_kfs_n = K0 + (size_t)tot[2];
     c->st_kf_nfeat.resize(c->st_kfs_n, 0);
+    c->st_kf_slot.resize(c->st_kfs_n, 0);
     for (int i = 0; i < n; ++i)
-        if (out_h[i] >= 0) c->st_kf_nfeat[(size_t)out_h[i]] = out_h[4 * (size_t)n + i];
+        if (out_h[i] >= 0) {
+            c->st_kf_nfeat[(size_t)out_h[i]] = out_h[4 * (size_t)n + i];
+            c->st_kf_slot[(size_t)out_h[i]] = b.cur_h[(size_t)i];
+        }
     c->st_max_feats = std::max(c->st_max_feats, (int)tot[3]);
+    b.nm_h.assign(nm_h, nm_h + n);
+    b.advance_flags = committed;
     if (kf_row_out) std::memcpy(kf_row_out, out_h, (size_t)n * sizeof(int32_t));
     if (point_first_out) std::memcpy(point_first_out, out_h + n, (size_t)n * sizeof(int32_t));
     if (n_points_out) std::memcpy(n_points_out, out_h + 2 * (size_t)n, (size_t)n * sizeof(int32_t));
+    return 0;
+}
+
+int dsdtm_batch_advance(dsdtm_ctx* c, const int32_t* next_cur_slots, const uint8_t* hold, const uint8_t* want_next, uint8_t* status_out)
+{
+    if (!c) return DSDTM_E_ARG;
+    auto& b = c->batch;
+    if (!b.staged || !b.store_staged || !b.track_staged || !b.advance_flags)
+        return fail(c, DSDTM_E_STATE, "dsdtm_batch_advance: no committed store-mode run with flags 7 or 15 since the last staging or advance");
+    if (want_next && !b.kf_staged) return fail(c, DSDTM_E_STATE, "dsdtm_batch_advance: want_next needs dsdtm_batch_stage_keyframe");
+    if (!next_cur_slots) return fail(c, DSDTM_E_ARG, "dsdtm_batch_advance: next_cur_slots is NULL");
+    const int n = b.n_pairs;
+    const bool kf = (b.advance_flags & 8) != 0 && b.kf_staged;
+    if (b.feat_stride < std::max(DSDTM_TRACK_MAX_MATCHES, b.kf_staged ? b.kf_max_fts : 0))
+        return fail(c, DSDTM_E_ARG, "dsdtm_batch_advance: feat_stride below max(DSDTM_TRACK_MAX_MATCHES, max_fts): a frame's features would not fit");
+    // the decisions, on the host: which frames advance (as key frames), and their reference slots afterwards
+    std::vector<int32_t> adv((size_t)2 * n);
+    std::vector<int32_t> ref_next(b.ref_h);
+    for (int i = 0; i < n; ++i) {
+        const int mode = b.nm_h[(size_t)i] < 0 ? DSDTM_ADV_HELD_OVERFLOW : (hold && hold[i]) ? DSDTM_ADV_HELD_CALLER
+                       : (kf && b.kf_want[(size_t)i]) ? DSDTM_ADV_KEYFRAME : DSDTM_ADV_ADVANCED;
+        adv[(size_t)i] = next_cur_slots[i];
+        adv[(size_t)n + i] = mode;
+        if (mode <= DSDTM_ADV_KEYFRAME) ref_next[(size_t)i] = b.cur_h[(size_t)i];
+    }
+    std::vector<uint8_t> named((size_t)c->prm.max_frames, 0);
+    // a key frame's pyramid must stay; an empty reserved row (no features: never close, never local) reads no slot and is skipped
+    for (size_t r = 0; r < c->st_kf_slot.size(); ++r) {
+        const int32_t sl = c->st_kf_slot[r];
+        if (c->st_kf_nfeat[r] != 0 && sl >= 0 && sl < c->prm.max_frames) named[(size_t)sl] = 1;
+    }
+    for (int32_t s : ref_next) named[(size_t)s] |= 2;
+    for (int i = 0; i < n; ++i) {
+        const int s = next_cur_slots[i];
+        if (s < 0 || s >= c->prm.max_frames) return fail(c, DSDTM_E_ARG, "dsdtm_batch_advance: next cur slot out of range");
+        if (named[(size_t)s] & 1) return fail(c, DSDTM_E_ARG, "dsdtm_batch_advance: next cur slot holds a key frame of the store");
+        if (named[(size_t)s] & 2) return fail(c, DSDTM_E_ARG, "dsdtm_batch_advance: next cur slot is a reference slot after the advance");
+        if (named[(size_t)s] & 4) return fail(c, DSDTM_E_ARG, "dsdtm_batch_advance: next cur slot named twice");
+        named[(size_t)s] |= 4;
+    }
+    std::vector<uint8_t> wt;
+    std::vector<int32_t> rows;
+    if (want_next) {
+        wt.resize((size_t)n);
+        for (int i = 0; i < n; ++i) if ((wt[(size_t)i] = want_next[i] ? 1 : 0)) rows.push_back(i);
+    }
+    if (!c->adv_d && dalloc(c, &c->adv_d, (size_t)2 * c->prm.max_batch)) return DSDTM_E_NOMEM;
+    if (ensure_pinned(c, adv.size() * sizeof(int32_t) + 2 * (size_t)n * sizeof(int32_t))) return DSDTM_E_NOMEM;
+    cudaStream_t s = c->stream;
+    int32_t* pin = reinterpret_cast<int32_t*>(c->pinned);
+    std::memcpy(pin, adv.data(), adv.size() * sizeof(int32_t));
+    DSDTM_CUDA(c, cudaMemcpyAsync(c->adv_d, pin, adv.size() * sizeof(int32_t), cudaMemcpyHostToDevice, s));
+    DSDTM_CUDA(c, launch_sequence_advance(c, c->adv_d, kf, s));
+    // enqueued: the host mirrors follow the device from here, and a second advance of this commit is a state error whatever happens below
+    b.advance_flags = 0;
+    for (int i = 0; i < n; ++i) b.cur_h[(size_t)i] = next_cur_slots[i];
+    b.ref_h = ref_next;
+    if (want_next) {
+        // after the advance, so that a launch that fails leaves the want mask as it was on the device and on the host alike
+        int32_t* rp = pin + adv.size();
+        uint8_t* wp = reinterpret_cast<uint8_t*>(rp + n);
+        if (!rows.empty()) std::memcpy(rp, rows.data(), rows.size() * sizeof(int32_t));
+        std::memcpy(wp, wt.data(), (size_t)n);
+        DSDTM_CUDA(c, cudaMemcpyAsync(c->kf_want_d, wp, (size_t)n, cudaMemcpyHostToDevice, s));
+        if (!rows.empty()) DSDTM_CUDA(c, cudaMemcpyAsync(c->kf_rows_d, rp, rows.size() * sizeof(int32_t), cudaMemcpyHostToDevice, s));
+        // the wanted count sizes the FAST grid of the captured flags-8 steps; the mask and the rows are read from device memory
+        if ((int)rows.size() != b.kf_n_wanted)
+            for (int gi = 8; gi < 16; ++gi)
+                if (b.graph[gi]) { cudaGraphExecDestroy(b.graph[gi]); b.graph[gi] = nullptr; }
+        b.kf_want = wt; b.kf_n_wanted = (int)rows.size();
+    }
+    DSDTM_CUDA(c, cudaStreamSynchronize(s));
+    if (status_out)
+        for (int i = 0; i < n; ++i) status_out[i] = (uint8_t)adv[(size_t)n + i];
+    return 0;
+}
+
+int dsdtm_batch_upload_step(dsdtm_ctx* c, const uint8_t* imgs, const uint16_t* depth)
+{
+    if (!c || !imgs) return DSDTM_E_ARG;
+    auto& b = c->batch;
+    if (!b.staged) return fail(c, DSDTM_E_STATE, "dsdtm_batch_upload_step: no staged batch");
+    if (depth && !b.kf_staged) return fail(c, DSDTM_E_STATE, "dsdtm_batch_upload_step: depth needs dsdtm_batch_stage_keyframe's depth slots");
+    const int n = b.n_pairs;
+    const size_t px = (size_t)c->cam.width * c->cam.height;
+    if (depth && ensure_depth_pool(c)) return DSDTM_E_NOMEM;
+    cudaStream_t s = c->stream;
+    bool contiguous = true;
+    for (int i = 1; i < n; ++i) contiguous &= b.cur_h[(size_t)i] == b.cur_h[0] + i;
+    // level 0 of a slot is dense at offset 0 (stride == width)
+    if (contiguous)
+        DSDTM_CUDA(c, cudaMemcpy2DAsync(c->frames_d + (size_t)b.cur_h[0] * c->geo.frame_stride, c->geo.frame_stride, imgs, px, px, (size_t)n,
+                                        cudaMemcpyHostToDevice, s));
+    else
+        for (int i = 0; i < n; ++i)
+            DSDTM_CUDA(c, cudaMemcpyAsync(c->frames_d + (size_t)b.cur_h[(size_t)i] * c->geo.frame_stride, imgs + (size_t)i * px, px,
+                                          cudaMemcpyHostToDevice, s));
+    if (depth)
+        for (int i = 0; i < n; ++i) {
+            const int ds = b.kf_depth_h[(size_t)i];
+            if (ds >= 0)
+                DSDTM_CUDA(c, cudaMemcpyAsync(c->depth_d + (size_t)ds * px, depth + (size_t)i * px, px * sizeof(uint16_t), cudaMemcpyHostToDevice, s));
+        }
+    DSDTM_CUDA(c, cudaStreamSynchronize(s));
+    return 0;
+}
+
+int dsdtm_batch_fetch_ref(dsdtm_ctx* c, int32_t* ref_slots, int32_t* cur_slots, dsdtm_ref_feat* feats, int32_t* n_feats, double* centers,
+                          double* poses_ref, double* poses_in)
+{
+    if (!c) return DSDTM_E_ARG;
+    auto& b = c->batch;
+    if (!b.staged) return fail(c, DSDTM_E_STATE, "dsdtm_batch_fetch_ref: no staged batch");
+    const size_t n = (size_t)b.n_pairs;
+    cudaStream_t s = c->stream;
+    if (ref_slots) DSDTM_CUDA(c, cudaMemcpyAsync(ref_slots, c->ref_slots_d, n * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+    if (cur_slots) DSDTM_CUDA(c, cudaMemcpyAsync(cur_slots, c->cur_slots_d, n * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+    if (feats) DSDTM_CUDA(c, cudaMemcpyAsync(feats, c->feats_d, n * b.feat_stride * sizeof(dsdtm_ref_feat), cudaMemcpyDeviceToHost, s));
+    if (n_feats) DSDTM_CUDA(c, cudaMemcpyAsync(n_feats, c->n_feats_d, n * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+    if (centers) DSDTM_CUDA(c, cudaMemcpyAsync(centers, c->centers_d, n * 3 * sizeof(double), cudaMemcpyDeviceToHost, s));
+    if (poses_ref) DSDTM_CUDA(c, cudaMemcpyAsync(poses_ref, c->poses_ref_d, n * 7 * sizeof(double), cudaMemcpyDeviceToHost, s));
+    if (poses_in) DSDTM_CUDA(c, cudaMemcpyAsync(poses_in, c->poses_in_d, n * 7 * sizeof(double), cudaMemcpyDeviceToHost, s));
+    DSDTM_CUDA(c, cudaStreamSynchronize(s));
     return 0;
 }
 
@@ -2299,7 +2442,7 @@ static int pair_batch_e2e_impl(dsdtm_ctx* c, int n_pairs, const uint8_t* cur_img
         return DSDTM_E_ARG;
     if (ppp < 0 || ppp > c->prm.max_patches || align_iters < 0) return fail(c, DSDTM_E_ARG, "patches_per_pair > max_patches");
     if (ppp > 0 && (!patches10 || !patch_px || !patch_level || !patch_px_out || !patch_conv)) return fail(c, DSDTM_E_ARG, "null patch arrays");
-    c->batch.staged = false; c->batch.commit_flags = 0;
+    c->batch.staged = false; c->batch.commit_flags = 0; c->batch.advance_flags = 0;
     const LevelGeom& g = c->geo;
     const size_t img_bytes = (size_t)g.w[0] * g.h[0];
     // chunked pipeline: H2D of chunk k+1 (copy stream) overlaps the kernels of chunk k (compute stream) and the D2H of chunk k-1.

@@ -56,6 +56,7 @@ struct dsdtm_ctx {
     int step_chunks = 1;                         // dsdtm_batch_run: pairs split over this many concurrent streams
     std::string err;
     long long launches = 0;
+    long long captures = 0;                      // CUDA graphs captured by dsdtm_batch_run (dsdtm_graph_captures)
     bool profiling = false;
     dsdtm::StageTimer timer;
     float last_run_ms = 0.f;
@@ -123,6 +124,7 @@ struct dsdtm_ctx {
     dsdtm_store_point* st_pts_d = nullptr;   size_t st_pts_cap = 0, st_pts_n = 0;
     int* st_found_d = nullptr;               size_t st_found_cap = 0;      // per point: MapPoint::mnFound (appended points start at 1)
     std::vector<int32_t> st_kf_nfeat;        // host mirror of every key-frame row's feat_count (reserved rows of dsdtm_batch_commit_store)
+    std::vector<int32_t> st_kf_slot;         // host mirror of every key-frame row's slot (dsdtm_batch_advance refuses a cur slot the store names)
     unsigned long long* st_claim_d = nullptr; size_t st_claim_cap = 0;     // per point: (~epoch << 32 | order) of the first local key frame that lists it
     uint8_t* st_vis_d = nullptr;             size_t st_vis_cap = 0;
     double* st_dist_d = nullptr;             size_t st_dist_cap = 0;
@@ -172,6 +174,7 @@ struct dsdtm_ctx {
     // dsdtm_batch_commit_store's scratch, grown on demand (never captured): per-frame counts / outputs and one push link per new feature
     int* cm_d = nullptr;                 size_t cm_cap = 0;
     int* cm_push_d = nullptr;            size_t cm_push_cap = 0;
+    int* adv_d = nullptr;                        // dsdtm_batch_advance: max_batch * 2 (next cur slot, DSDTM_ADV_* per frame), allocated on first use
     // key-frame detection (dsdtm_detect_batch), grown on demand
     uint8_t* det_mask_d = nullptr;       size_t det_mask_cap = 0;    // n * w*h mask images: allocated by the first call that passes masks
     uint8_t* det_buf_d = nullptr;        size_t det_buf_cap = 0;     // small inputs (max_new, n_circles, circles) | outputs, one copy each way
@@ -196,6 +199,10 @@ struct dsdtm_ctx {
         int store_max_local = 0, store_cpf = 0, store_range_max = 0, store_range_end = 0, store_n_found = 0;
         bool store_found_live = false;                     // dsdtm_batch_stage_track_live: the selection reads st_found_d
         int commit_flags = 0;                              // flags of the last store-mode run with bit 2 not yet committed, 0 = none
+        int advance_flags = 0;                             // flags of the last committed run not yet advanced (dsdtm_batch_advance), 0 = none
+        std::vector<int32_t> ref_h, cur_h;                 // host mirrors of ref_slots_d / cur_slots_d (dsdtm_batch_stage, dsdtm_batch_advance)
+        std::vector<int32_t> nm_h;                         // n_matches of the committed run, read back by the commit (frames held on overflow)
+        std::vector<int32_t> kf_depth_h;                   // the staged depth slots (host copy, dsdtm_batch_upload_step)
         bool kf_staged = false;                            // dsdtm_batch_stage_keyframe: the key-frame half is ready
         int kf_min_dist = 0, kf_max_fts = 0, kf_n_wanted = 0;
         float kf_thr = 0.f, kf_dist[5] = {}, kf_depth_scale = 1.f;
@@ -294,6 +301,9 @@ struct StoreCommitArgs {
     int* cnt_d; int* out_d; int* push_d;        // 3n, 5n + 4, one per new feature row
 };
 cudaError_t launch_store_commit(dsdtm_ctx* c, const StoreCommitArgs& a, cudaStream_t s);
+// dsdtm_batch_advance (sequence_advance.cu): every frame's next reference frame from the committed step; adv_d = next cur slot and
+// DSDTM_ADV_* per frame, decided on the host
+cudaError_t launch_sequence_advance(dsdtm_ctx* c, const int* adv_d, bool keyframes, cudaStream_t s);
 size_t track_select_smem(int ppp);             // dynamic shared memory of one selection CTA for ppp records per frame
 int track_select_key_bits(const dsdtm_ctx* c, int ppp);   // bits of a selection key for this grid and ppp (must be <= 64)
 cudaError_t track_select_init(dsdtm_ctx* c);

@@ -102,6 +102,8 @@ void*       dsdtm_host_alloc(size_t bytes);
 void        dsdtm_host_free(void* p);
 /* kernels launched by this context since creation (bench.py's gpu_launches) */
 long long   dsdtm_launch_count(const dsdtm_ctx* ctx);
+/* CUDA graphs dsdtm_batch_run has captured on this context since creation: a run that only replays a captured step adds nothing */
+long long   dsdtm_graph_captures(const dsdtm_ctx* ctx);
 /* measurement aid (no reference counterpart): the DFMA throughput this GPU sustains on dependency-free streams, in TFLOP/s (2 flops
  * per DFMA) and in warp instructions per clock and SM at the nominal maximum clock -- the ceiling bench.py puts the fp64
  * sparse-alignment kernel against. Runs a ~10 ms kernel on the context's stream and synchronises. */
@@ -631,12 +633,51 @@ int dsdtm_batch_stage_track_live(dsdtm_ctx* ctx, int max_iters);
  * n_points_out[i] = its new points; any of them may be NULL. Frames of one step that share a map all read the counts the step started
  * with and their increments add up; the result equals the sequential tracker when each map has at most one frame per step (a later frame
  * of the same map would have seen the earlier frame's counts, bad flags and key frame). Cost: a point that k key frames of one commit
- * observe is linked by one thread in O(k log k) dependent loads (k = 1 in that layout, k = frames per map otherwise). The commit drops the captured store-mode steps,
- * reserves the worst case before enqueuing (DSDTM_E_NOMEM: the store is unchanged) and synchronises once to read the new table sizes.
+ * observe is linked by one thread in O(k log k) dependent loads (k = 1 in that layout, k = frames per map otherwise). A commit that writes a
+ * key frame or reallocates a table drops the captured store-mode steps; one that writes none (every flags-7 commit, flags 15 with nothing
+ * wanted) keeps them: its found counts and bad flags are read from device memory by the replay. It reserves the worst case before enqueuing (DSDTM_E_NOMEM: the store is unchanged) and synchronises once to read the new table sizes.
  * DSDTM_E_ARG, nothing enqueued, for a NaN threshold or, for a wanted frame, a reserved row outside the table, not empty or named twice.
  * DSDTM_E_STATE without a store-mode run with flags bit 2 since the last staging, after dsdtm_store_clear, or for a second commit. */
 int dsdtm_batch_commit_store(dsdtm_ctx* ctx, float outlier_threshold, const int32_t* kf_rows /* n_pairs or NULL */, int32_t* kf_row_out,
                              int32_t* point_first_out, int32_t* n_points_out);
+/* Sequences on the device: after a store-mode dsdtm_batch_run with flags 7 or 15 and its dsdtm_batch_commit_store, every frame that advances
+ * becomes its own next reference frame, as Tracking::Track_RGBDCam's TrackWithLastFrame does (ref: src/Tracking.cpp:199-205: the reference
+ * frame is the last frame, cur.Set_Pose(last.Get_Pose())). One kernel, one CTA per frame, rewrites the staged per-frame inputs the captured
+ * step reads, so the next dsdtm_batch_run replays it on them:
+ *   ref slot   = the frame's cur slot (its pyramid is built);          pose_ref = the pose after PoseOptimization;
+ *   centre     = Get_CameraCnt() of that pose (the arithmetic the commit uses for a key frame's centre);
+ *   prior      = identity (T_c2r of cur.Set_Pose(last.Get_Pose()));   cur slot = next_cur_slots[i];
+ *   features   = the frame's mvFeatures as Sprase_ImgAlign::GetJocabianMat reads them next (ref: src/Sprase_ImageAlign.cpp:84-103): its matches
+ *                in match order (px and level of the match, initial 1, normal = the bearing PoseOptimization used, point_w = the store's
+ *                point_w of the match's point row -- a point the commit flagged bad stays: the reference tests the pointer, not IsBad); after
+ *                flags 15 a frame that became a key frame continues with its new corners in Add_Feature order (px and normal of the lifted
+ *                record, the corner level, initial = DSDTM_LIFT_OK, point_w = the lifted point or zero): the feature list the commit wrote.
+ *                Rows past n_feats[i] are zero.
+ * Held frames keep reference, pose, centre, prior and features; only their cur slot moves to next_cur_slots[i]: frames with n_matches -1
+ * (candidate overflow) and frames with hold[i] != 0 (hold NULL = none). The Lost rule (< 20 tracked points after Run, ref: :208) and
+ * NeedKeyframe stay with the caller, who reads n_tracked with dsdtm_batch_fetch and passes the decisions through hold and want_next.
+ * want_next (NULL = unchanged) replaces dsdtm_batch_stage_keyframe's want mask for the next run; a change of the wanted count drops the
+ * captured flags-8 steps (their FAST grid is sized by it), never the others. status_out[i] (NULL allowed) = DSDTM_ADV_*.
+ * Writes only buffers the captured steps point at: nothing is dropped (except as above) and a steady flags-7 sequence is pure replays.
+ * Every error returns before anything is enqueued, with the staged state unchanged. DSDTM_E_STATE: no store-mode flags 7/15 run, no commit
+ * since it, a second advance, one-key-frame mode, want_next without dsdtm_batch_stage_keyframe. DSDTM_E_ARG: a next cur slot outside
+ * max_frames, named twice, the slot of a key frame of the store (an empty reserved row names no slot: it is never close and never
+ * local) or equal to a frame's reference slot after the advance; a staged
+ * feat_stride below max(DSDTM_TRACK_MAX_MATCHES, max_fts) -- refused rather than truncated. Synchronises once. */
+enum { DSDTM_ADV_ADVANCED = 0, DSDTM_ADV_KEYFRAME = 1, DSDTM_ADV_HELD_OVERFLOW = 2, DSDTM_ADV_HELD_CALLER = 3 };
+int dsdtm_batch_advance(dsdtm_ctx* ctx, const int32_t* next_cur_slots /* n_pairs */, const uint8_t* hold /* n_pairs or NULL */,
+                        const uint8_t* want_next /* n_pairs or NULL */, uint8_t* status_out /* n_pairs or NULL */);
+/* Frame::Frame's image input for the staged step (ref: src/Frame.cpp:48-81) in one call: the n_pairs dense level-0 images (imgs, n_pairs x
+ * height x width bytes) into the staged cur slots, and, when depth is not NULL, the n_pairs 16-bit depth images (dense, n_pairs x height x
+ * width) into the frames' depth slots of dsdtm_batch_stage_keyframe (frames without one skip theirs). The pyramids are built by the run's
+ * flags bit 0. cudaMemcpyAsync on the context's stream, one copy per frame or one for contiguous slots; pinned buffers are faster, pageable
+ * ones work. Returns when the images are on the device. DSDTM_E_STATE without dsdtm_batch_stage (depth: without _stage_keyframe). */
+int dsdtm_batch_upload_step(dsdtm_ctx* ctx, const uint8_t* imgs, const uint16_t* depth);
+/* the staged per-frame inputs exactly as the next dsdtm_batch_run reads them (every pointer may be NULL): ref_slots / cur_slots / n_feats
+ * n_pairs each, feats n_pairs x feat_stride, centers n_pairs x 3, poses_ref (the reference poses of store or map mode) and poses_in (the
+ * sparse alignment's prior T_c2r) n_pairs x 7. DSDTM_E_STATE without dsdtm_batch_stage. */
+int dsdtm_batch_fetch_ref(dsdtm_ctx* ctx, int32_t* ref_slots, int32_t* cur_slots, dsdtm_ref_feat* feats, int32_t* n_feats, double* centers,
+                          double* poses_ref, double* poses_in);
 int dsdtm_batch_fetch(dsdtm_ctx* ctx, double* poses_out, int* n_tracked, double* patch_px_out, uint8_t* patch_conv);
 /* end-to-end step with HOST buffers: uploads the n_pairs cur images (dense, pinned recommended) into their cur slots,
  * stages the per-pair inputs, runs, and fetches -- copies overlapped with compute in chunks on internal streams. Both e2e entries
